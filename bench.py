@@ -9,6 +9,10 @@ copies inside the timed region (`e2e`).
   python bench.py [--gpus N] [--steps K] [--warmup W]          our arm (CUDA, through the C ABI)
   python bench.py --impl reference [...]                       the reference's CPU algorithm (oracle port) on the host cores
   python bench.py --no-configs / --no-cpu                      skip the per-config legs / the cpu_baseline leg
+  python bench.py --dump-outputs DIR [...]                     also write a sample of the headline's last-step output to DIR
+
+--steps is the number of timed steps of every GPU leg (headline, H/V split, e2e, configs); the cpu_baseline leg of our
+arm is a fixed 8-step sample.  Inputs are generated from fixed seeds, so the same arguments give the same inputs on every run.
 
 The JSON line carries, next to the contract keys:
   configs   one entry per BASELINE.json config (c1..c5): device-resident frames/s, algorithmic GB/s and fraction of the
@@ -47,6 +51,23 @@ WORKLOAD = "configs[1]: BoxBlur 13/5/13/5 on 1920x1080 YUV420P16 uniform-noise f
 CONFIG = {"workload": WORKLOAD, "filter": "vszip.BoxBlur", "args": ARGS, "format": FMT, "width": W, "height": H, "content": "uniform noise",
           "parallelism": "frame-parallel (frame n -> GPU n mod k), no collective",
           "l2": "every timed step streams far more than the 126 MB L2 (inputs larger than L2, no flush needed)"}
+
+
+DUMP_FRAMES = 4   # 4 whole frames as float32 = 49.8 MB, under the 64 MB a dump may take
+
+
+def dump_outputs(out_dir, dst, frame_nos):
+    """Writes what the headline's last step left in `dst` (what a caller of run_device receives) for comparing two builds:
+    DUMP_FRAMES frames of the batch picked with a fixed seed, every plane whole, as float32 (exact for 16-bit samples),
+    boxblur_{y,u,v}.npy of shape (DUMP_FRAMES, h, w), and their frame numbers in frame_numbers.npy."""
+    import numpy as np
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    pick = sorted(np.random.default_rng(0).choice(len(frame_nos), DUMP_FRAMES, replace=False).tolist())
+    frames = [dst.download(i) for i in pick]
+    for p, name in enumerate("yuv"):
+        np.save(out / f"boxblur_{name}.npy", np.stack([f[p] for f in frames]).astype(np.float32))
+    np.save(out / "frame_numbers.npy", np.array([frame_nos[i] for i in pick], dtype=np.float64))
 
 
 def frames_of_rank(rank, world, per_rank):
@@ -254,12 +275,14 @@ def run_ours(args):
     launches = (vz.core.kernel_launches - l0) * args.steps // (args.steps + args.warmup)
     clocks = sampler.stop() if sampler else None
     fps = world * n / (ms_step * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, dst, mine)   # before the legs below overwrite dst
 
     # ---- per-kernel durations for the roofline (H passes only / V passes only, same batch)
     fh = vz.BoxBlurFilter(src.info(), hradius=13, hpasses=5, vradius=0, vpasses=0)
     fv = vz.BoxBlurFilter(src.info(), hradius=0, hpasses=0, vradius=13, vpasses=5)
-    ms_h = timed(lambda: fh.run_device(src, dst, 0, n, stream), max(3, args.steps // 2), 3)
-    ms_v = timed(lambda: fv.run_device(src, dst, 0, n, stream), max(3, args.steps // 2), 3)
+    ms_h = timed(lambda: fh.run_device(src, dst, 0, n, stream), args.steps, 3)
+    ms_v = timed(lambda: fv.run_device(src, dst, 0, n, stream), args.steps, 3)
     dom_name, dom_ms = ("hseg_kernel<13> (5 H passes)", ms_h) if ms_h >= ms_v else ("vseg_tile_kernel<13> (5 V passes)", ms_v)
     achieved = ALGO_BYTES * n / (dom_ms * 1e-3) / 1e9
     traffic = None  # DRAM bytes per launch of that kernel, from the committed ncu --set full capture
@@ -270,7 +293,7 @@ def run_ours(args):
     path_gbs = ALGO_BYTES * n / (ms_step * 1e-3) / 1e9
 
     # ---- one entry per BASELINE config, device-resident (c5 also end to end), every rank on its own frames
-    configs = None if args.no_configs else other_configs(vz, lib, torch, np, timed, timed_host, stream, world, peak,
+    configs = None if args.no_configs else other_configs(vz, lib, torch, np, timed, timed_host, stream, world, peak, args.steps,
                                                          {"fps": fps, "ms_per_frame_batch": ms_step, "frames": n}, path_gbs, my_cores)
     src.free(); dst.free()
 
@@ -282,7 +305,6 @@ def run_ours(args):
     in_flight_staged = max(2, min(16, ncores))   # memcpy-bound leg: as many worker threads as VapourSynth would run (<= 16 slots per GPU)
     pools = {n: ThreadPoolExecutor(n) for n in {in_flight, in_flight_staged}}
     rng = np.random.default_rng(rank)
-    e2e_steps = max(3, min(args.steps, 6))
 
     def e2e_leg(frames_in, frames_out, threads):
         pool = pools[threads]
@@ -292,7 +314,7 @@ def run_ours(args):
         def one(i):
             if lib.vszip_boxblur_get_frame(flt.handle, mine[i], C.byref(cin[i]), C.byref(cout[i])):
                 raise RuntimeError(vz._last_error())
-        s = timed_host(lambda: list(pool.map(one, range(ne))), e2e_steps, 3)
+        s = timed_host(lambda: list(pool.map(one, range(ne))), args.steps, 3)
         return world * ne / s
 
     # (a) pageable planes, one allocation per plane (anonymous mappings with malloc's 64-byte offset, which is what the
@@ -349,7 +371,7 @@ def run_ours(args):
                 dbuf[i].copy_(host_in[i], non_blocking=True)
                 host_out[i].copy_(dbuf[i], non_blocking=True)
         torch.cuda.synchronize()
-    ceiling = world * ne / timed_host(copy_step, e2e_steps, 2)
+    ceiling = world * ne / timed_host(copy_step, args.steps, 2)
     torch.cuda.set_stream(tstream)
 
     # ---- CPU baseline (rank 0, N=1 only): bounded sample of the same workload on the host cores
@@ -389,7 +411,7 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
-def other_configs(vz, lib, torch, np, timed, timed_host, stream, world, peak, headline, headline_gbs, my_cores):
+def other_configs(vz, lib, torch, np, timed, timed_host, stream, world, peak, steps, headline, headline_gbs, my_cores):
     """BASELINE.json configs 1..5 at this N (every rank runs the same batch on its own GPU; fps is the whole job's)."""
     out = {}
 
@@ -401,17 +423,17 @@ def other_configs(vz, lib, torch, np, timed, timed_host, stream, world, peak, he
         e.update(more)
         return e
 
-    def pixel(name, fmt, w, h, frames, make, reps=5):
+    def pixel(name, fmt, w, h, frames, make):
         a, b = vz.DeviceClip(fmt, w, h, frames), vz.DeviceClip(fmt, w, h, frames)
         a.fill_noise(1234)
         f = make(a)
-        ms = timed(lambda: f.run_device(a, b, first=0, count=frames, stream=stream), reps, 3)
+        ms = timed(lambda: f.run_device(a, b, first=0, count=frames, stream=stream), steps, 3)
         e = entry(name, fmt, w, h, frames, 2 * a.frame_bytes, ms)
         a.free(); b.free()
         return e
 
     out["c1"] = pixel("configs[0]: BoxBlur 13/1/13/1 (comptime path, one read + one write)", "YUV420P16", 1920, 1080, 256,
-                      lambda s: vz.BoxBlurFilter(s.info(), hradius=13, hpasses=1, vradius=13, vpasses=1), reps=10)
+                      lambda s: vz.BoxBlurFilter(s.info(), hradius=13, hpasses=1, vradius=13, vpasses=1))
     out["c2"] = {"config": "configs[1]: BoxBlur 13/5/13/5 [headline, see value/roofline/path]", "format": "YUV420P16", "size": "1920x1080",
                  "frames_per_launch_per_gpu": headline["frames"], "fps": headline["fps"], "us_per_frame_per_gpu": headline["ms_per_frame_batch"] * 1e3 / headline["frames"],
                  "algorithmic_bytes_per_frame": ALGO_BYTES, "GBps_per_gpu": headline_gbs, "frac_of_hbm_peak": headline_gbs / peak}
@@ -435,10 +457,10 @@ def other_configs(vz, lib, torch, np, timed, timed_host, stream, world, peak, he
         a.fill_noise(1234)
         mmf = vz.PlaneMinMaxFilter(a.info(), minthr=0.1, maxthr=0.1)
         avf = vz.PlaneAverageFilter(a.info(), exclude=excl)
-        ms_mm = timed(lambda: vz._check(lib.vszip_planeminmax_device(mmf.handle, a.handle, None, 0, frames, None, stream)), 5, 3)
-        ms_av = timed(lambda: vz._check(lib.vszip_planeaverage_device(avf.handle, a.handle, None, 0, frames, None, stream)), 5, 3)
+        ms_mm = timed(lambda: vz._check(lib.vszip_planeminmax_device(mmf.handle, a.handle, None, 0, frames, None, stream)), steps, 3)
+        ms_av = timed(lambda: vz._check(lib.vszip_planeaverage_device(avf.handle, a.handle, None, 0, frames, None, stream)), steps, 3)
         _, fused = vz.plane_stats_device(mmf, avf, a, count=frames, stream=stream, fetch=False)
-        ms_both = timed(lambda: vz.plane_stats_device(mmf, avf, a, count=frames, stream=stream, fetch=False), 5, 3)
+        ms_both = timed(lambda: vz.plane_stats_device(mmf, avf, a, count=frames, stream=stream, fetch=False), steps, 3)
         fb = a.frame_bytes
         c4[fmt] = {"PlaneMinMax(minthr=.1,maxthr=.1)": entry("PlaneMinMax thr", fmt, 3840, 2160, frames, fb, ms_mm),
                    f"PlaneAverage(exclude={excl})": entry("PlaneAverage", fmt, 3840, 2160, frames, fb, ms_av),
@@ -453,15 +475,15 @@ def other_configs(vz, lib, torch, np, timed, timed_host, stream, world, peak, he
     blur = vz.BoxBlurFilter(a.info(), hradius=13, hpasses=1, vradius=13, vpasses=1)
     bil = vz.BilateralFilter(a.info(), sigmaS=2, sigmaR=2)
     mm = vz.PlaneMinMaxFilter(a.info(), minthr=0.1, maxthr=0.1, planes=[0])
-    ms_blur = timed(lambda: blur.run_device(a, b, count=frames, stream=stream), 3, 2)
-    ms_bil = timed(lambda: bil.run_device(b, c, count=frames, stream=stream), 3, 2)
-    ms_mm = timed(lambda: vz._check(lib.vszip_planeminmax_device(mm.handle, c.handle, None, 0, frames, None, stream)), 3, 2)
+    ms_blur = timed(lambda: blur.run_device(a, b, count=frames, stream=stream), steps, 2)
+    ms_bil = timed(lambda: bil.run_device(b, c, count=frames, stream=stream), steps, 2)
+    ms_mm = timed(lambda: vz._check(lib.vszip_planeminmax_device(mm.handle, c.handle, None, 0, frames, None, stream)), steps, 2)
 
     def chain_dev():
         blur.run_device(a, b, count=frames, stream=stream)
         bil.run_device(b, c, count=frames, stream=stream)
         vz._check(lib.vszip_planeminmax_device(mm.handle, c.handle, None, 0, frames, None, stream))
-    ms_chain = timed(chain_dev, 3, 2)
+    ms_chain = timed(chain_dev, steps, 2)
     fb = a.frame_bytes
     c5 = {"config": "configs[4]: BoxBlur(13,1,13,1) -> Bilateral(2,2) -> PlaneMinMax(.1,.1,planes=[0]) on 3840x2160 YUV444PS (bounded sample of the 5000-frame clip)",
           "BoxBlur": entry("BoxBlur 13/1/13/1 f32 (comptime float path)", fmt, w, h, frames, 2 * fb, ms_blur),
@@ -497,7 +519,7 @@ def other_configs(vz, lib, torch, np, timed, timed_host, stream, world, peak, he
             raise RuntimeError(vz._last_error())
     threads = max(2, min(4, len(my_cores) if my_cores else 4))
     with ThreadPoolExecutor(threads) as ex:
-        s = timed_host(lambda: list(ex.map(one, range(ne))), 3, 2)
+        s = timed_host(lambda: list(ex.map(one, range(ne))), steps, 2)
     c5["e2e_fused_chain"] = {"fps": world * ne / s, "api": "vszip_chain_get_frame on pinned frames", "in_flight": threads,
                              "h2d_bytes_per_frame": 3 * w * h * 4, "d2h_bytes_per_frame": 3 * w * h * 4, "frames_per_step_per_gpu": ne}
     lib.vszip_chain_free(chain)
@@ -514,7 +536,12 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-configs", action="store_true", help="skip the per-config legs (configs c1..c5)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a seeded sample of the headline's last-step output to DIR/*.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the CUDA arm's output; the reference arm runs on other inputs")
     # The contract is ONE JSON line on stdout.  Libraries (NCCL prints its version banner there) must not add to it:
     # point fd 1 at stderr for the whole run and hand the real stdout to the two print(json.dumps(..)) calls only.
     sys.stdout.flush()
