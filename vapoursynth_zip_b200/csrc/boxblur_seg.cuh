@@ -122,23 +122,20 @@ __device__ __forceinline__ void bulk_wait0() { asm volatile("cp.async.bulk.wait_
 #define VSZ_SEG_ALL_DP false
 #endif
 constexpr bool kAllDp = VSZ_SEG_ALL_DP;
-#ifndef VSZ_SEG_HCHAINS
-#define VSZ_SEG_HCHAINS 2
-#endif
-constexpr int kHChains = VSZ_SEG_HCHAINS;  // independent running sums per thread in the H pass
+constexpr int kCtChains = 2;  // independent running sums per thread in the comptime path's H pass
 
-// One warp-synchronous H pass over the row(s) of a lane group.  `row` = the group's staged row (sample 0 at row + PAD);
-// e[] = the lane's registers with the pass input (own part), o[] receives the results (own part).
-//   first_pass: the input is in the staged row (put there by the TMA engine or by the comptime V phase), else in e[] and is
-//   published to the row here.  Mirrors: when the row ends exactly at a segment end the first and last lane write them from
-//   registers; ragged rows copy them inside the staged row and the last lane reloads its span (which contains mirrored samples).
+// The lane's view ext[] of the staged row(s) of a lane group (sample 0 at row + PAD), halos included.
+//   e[] = the lane's registers: its own samples are loaded from the row here (from_row), or are given (two consecutive samples
+//   per word) and published to the row.  Mirrors: when the row ends exactly at a segment end the first and last lane write them
+//   from registers; ragged rows copy them inside the staged row and the last lane reloads its span (which contains mirrored
+//   samples).  The row may be overwritten after the next __syncwarp.
 template <int R>
-__device__ __forceinline__ void hseg_pass(uint32_t (&e)[HGeom<R>::NW], uint32_t (&o)[HGeom<R>::NW], uint16_t* row, int n, int sg, int G, int S,
-                                          bool first_pass, bool act, int lane, uint32_t inv, uint32_t inv2) {
+__device__ __forceinline__ void hseg_load_row(uint32_t (&e)[HGeom<R>::NW], uint16_t* row, int n, int sg, int G, int S, bool from_row, bool act,
+                                              int lane) {
     using Gm = HGeom<R>;
     uint16_t* own = row + Gm::PAD + L * sg;
     const int lig = lane & (G - 1);
-    if (first_pass) h_load_own<R>(e, own);
+    if (from_row) h_load_own<R>(e, own);
     else if (act) h_store_own<R>(e, own);
     if (L * S == n) {
         if (lig == 0) h_write_left_pad<R>(e, row + Gm::PAD);
@@ -158,11 +155,45 @@ __device__ __forceinline__ void hseg_pass(uint32_t (&e)[HGeom<R>::NW], uint32_t 
         if (lig == S - 1) h_load_own<R>(e, own);
     }
     h_load_halos<R>(e, own);
-    const uint32_t W = h_window<R>(e);
-    uint32_t C = line_const(W, inv, inv2);
-    C = __shfl_sync(0xffffffffu, C, lane & ~(G - 1));  // the group's first lane holds the window at position 0
-    h_slide<R, kHChains, kAllDp>(e, o, W, C, inv2);
-    __syncwarp();  // every lane has read its halos: the staged row may be overwritten
+}
+// ... and the words of the H pass from it; ends with every lane past its reads of the row, so the row may be overwritten
+template <int R>
+__device__ __forceinline__ void hseg_load_pairs(uint32_t (&e)[HGeom<R>::NW], uint32_t (&p)[NP], uint16_t* row, int n, int sg, int G, int S,
+                                                bool from_row, bool act, int lane) {
+    hseg_load_row<R>(e, row, n, sg, G, S, from_row, act, lane);
+    h_pairs<R>(e, p);
+    __syncwarp();
+}
+
+// The words of the next H pass from h_slide_next's q[] and xs[].  Rows that end at a segment end exchange only the edges: every
+// lane publishes its first and last HW words (the first / last lane their mirrors too) and completes its edge words from the
+// neighbours'.  Ragged rows go through hseg_load_pairs with the lane's own samples.
+template <int R>
+__device__ __forceinline__ void hseg_next_pairs(uint32_t (&e)[HGeom<R>::NW], uint32_t (&q)[NP], const uint32_t (&xs)[2 * HGeom<R>::HW],
+                                                uint16_t* row, int n, int sg, int G, int S, bool act, int lane) {
+    using Gm = HGeom<R>;
+    if (L * S == n) {
+        uint16_t* own = row + Gm::PAD + L * sg;
+        const int lig = lane & (G - 1);
+        if (act) h_store_edges<R>(xs, own);
+        if (lig == 0) h_write_left_pad_words<R>(xs, row + Gm::PAD);
+        if (lig == S - 1) h_write_right_pad_words<R>(xs + 2 * Gm::HW, row + Gm::PAD + n);
+        __syncwarp();
+        h_load_halos<R>(e, own);
+        __syncwarp();
+        h_complete_edges<R>(q, e);
+    } else {
+        h_own_words<R>(q, e + Gm::HW);
+        hseg_load_pairs<R>(e, q, row, n, sg, G, S, false, act, lane);
+    }
+}
+
+// window sum at own[0] and the line constant C of the pass (the group's first lane holds the window at position 0)
+template <int R>
+__device__ __forceinline__ uint32_t hseg_window(const uint32_t (&p)[NP], int lane, int G, uint32_t inv, uint32_t inv2, uint32_t& C) {
+    const uint32_t W = pair_window<R>(p);
+    C = __shfl_sync(0xffffffffu, line_const(W, inv, inv2), lane & ~(G - 1));
+    return W;
 }
 
 // --------------------------------------------------------------------------- host side

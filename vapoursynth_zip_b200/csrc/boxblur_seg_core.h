@@ -7,8 +7,9 @@
 // A thread therefore owns a SEGMENT of L = 60 consecutive samples of a line, keeps it in registers across all
 // passes, and only exchanges the r samples either side of the segment with its neighbours per pass.
 //
-// 16-bit samples stay packed two per 32-bit word; `dp2a` (IDP.2A) adds or subtracts one half of a word to
-// a 32-bit sum in one instruction, so samples are never unpacked.
+// 16-bit samples stay packed two per 32-bit word; `dp2a` (IDP.2A) adds or subtracts the halves of a word to a 32-bit sum
+// in one instruction, so samples are never unpacked.  H passes pair each sample with the one 2r+1 further on (see h_pairs),
+// so that one window step is one dp2a.
 //
 // Everything here is __host__ __device__: tests/sim/boxblur_seg_sim.cpp runs the same code lane by lane on the
 // CPU against the oracle (the container that builds this has no GPU).
@@ -88,26 +89,12 @@ VSZ_HD uint32_t line_const(uint32_t w0, uint32_t inv, uint32_t inv2) {
     return s0 - inv2 * w0;
 }
 
-// add / subtract sample `half` (0 = low, 1 = high) of word w.  Low halves go through dp2a (FMA pipe), high halves
-// through a shift + add (ALU pipe): the two pipes issue at the same rate on sm_100, so the split keeps both busy.
-template <bool ALL_DP>
-VSZ_HD uint32_t add_sample(uint32_t W, uint32_t w, int half) {
-    if (half == 0) return dp2a(w, ADD_LO, W);
-    if (ALL_DP) return dp2a(w, ADD_HI, W);
-    return W + (w >> 16);
-}
-template <bool ALL_DP>
-VSZ_HD uint32_t sub_sample(uint32_t W, uint32_t w, int half) {
-    if (half == 0) return dp2a(w, SUB_LO, W);
-    if (ALL_DP) return dp2a(w, SUB_HI, W);
-    return W - (w >> 16);
-}
-
-// =========================================================================== H: a word = two consecutive samples
-// ext[] is the thread's view of its row: [prev halo | own 60 samples | next halo], whole 64-bit units.
+// =========================================================================== H
+// ext[] is the thread's view of its row as staged in shared memory: [prev halo | own 60 samples | next halo], two consecutive
+// samples per word, whole 64-bit units.
 template <int R>
 struct HGeom {
-    static_assert(R >= 1 && R < L, "segment kernels need 1 <= r < 60");
+    static_assert(R >= 1 && 2 * R + 2 <= L, "segment kernels need 1 <= r <= 29");
     static constexpr int HW = 2 * ((R + 3) / 4);   // words of either halo (>= r samples, loaded as 64-bit units)
     static constexpr int NW = HW + LW + HW;
     static constexpr int J0 = 2 * HW;              // sample index of own[0] inside ext[]
@@ -116,6 +103,115 @@ struct HGeom {
     // samples of one staged row: pad, S segments, tail
     static constexpr int row_samples(int S) { return PAD + L * S + PADR; }
 };
+
+// A pass holds one word per window step of the segment [x0, x0 + 60): both samples of that step,
+//     p[k] = (lo16: s[x0 + k + r + 1], hi16: s[x0 + k - r]),   k = 0 .. NP-1,
+// so that a step is one dp2a, W_{k+1} = W_k + lo16(p[k]) - hi16(p[k]), and an output one IMAD, o_k = W_k * inv2 + C (16.16:
+// the sample is hi16(o_k)).  The words of the next pass are two 16.16 outputs 2r+1 apart, pack_hi(o_{k+r+1}, o_{k-r}) (PRMT).
+// The first r words take their high half from the left neighbour's last r outputs, the last r words their low half from the
+// right neighbour's first r outputs; between passes they hold the lane's own 16.16 output alone (h_complete_edges fills in
+// the other half once the neighbours have published theirs).
+constexpr int NP = L - 1;
+constexpr uint32_t STEP = 0xff01u;  // dp2a selector: + low half - high half
+
+// byte permute: bytes 0-3 of x, 4-7 of y, one selector nibble per result byte
+VSZ_HD uint32_t prmt(uint32_t x, uint32_t y, uint32_t sel) {
+#if defined(__CUDA_ARCH__)
+    return __byte_perm(x, y, sel);
+#else
+    const uint64_t v = ((uint64_t)y << 32) | x;
+    uint32_t d = 0;
+    for (int b = 0; b < 4; ++b) d |= (uint32_t)((v >> (8 * ((sel >> (4 * b)) & 7u))) & 0xffu) << (8 * b);
+    return d;
+#endif
+}
+
+// the words of a pass from the staged samples in ext[]
+template <int R>
+VSZ_HD void h_pairs(const uint32_t (&ext)[HGeom<R>::NW], uint32_t (&p)[NP]) {
+    using G = HGeom<R>;
+#pragma unroll
+    for (int k = 0; k < NP; ++k) {
+        const int a = G::J0 + k + R + 1, b = G::J0 + k - R;  // entering / leaving sample (a - b is odd: opposite halves)
+        p[k] = prmt(ext[a >> 1], ext[b >> 1], (a & 1) ? 0x5432u : 0x7610u);
+    }
+}
+
+// the edge words, from the neighbours' samples in the halo part of ext[] (the own part is not read)
+template <int R>
+VSZ_HD void h_complete_edges(uint32_t (&p)[NP], const uint32_t (&ext)[HGeom<R>::NW]) {
+    using G = HGeom<R>;
+#pragma unroll
+    for (int k = 0; k < R; ++k) {
+        const int b = G::J0 + k - R;
+        p[k] = prmt(p[k], ext[b >> 1], (b & 1) ? 0x7632u : 0x5432u);
+    }
+#pragma unroll
+    for (int k = NP - R; k < NP; ++k) {
+        const int a = G::J0 + k + R + 1;
+        p[k] = prmt(ext[a >> 1], p[k], (a & 1) ? 0x7632u : 0x7610u);
+    }
+}
+
+// window sum of the samples [-r, r] around the segment's first sample: the high halves of p[0..2r]
+template <int R, int N>
+VSZ_HD uint32_t pair_window(const uint32_t (&p)[N]) {
+    uint32_t W = 0;
+#pragma unroll
+    for (int k = 0; k <= 2 * R; ++k) W = dp2a(p[k], ADD_HI, W);
+    return W;
+}
+
+// One pass over a segment of N + 1 samples that feeds another: emit(i, o_i) gets the 16.16 outputs, q[] receives the next
+// pass's words (edge words holding the own output only).
+template <int R, int N, class Emit>
+VSZ_HD void pair_slide_next(const uint32_t (&p)[N], uint32_t (&q)[N], uint32_t W, uint32_t C, uint32_t inv2, Emit emit) {
+    uint32_t o[N + 1];
+#pragma unroll
+    for (int i = 0; i <= N; ++i) {
+        o[i] = W * inv2 + C;
+        if (i < N) W = dp2a(p[i], STEP, W);
+        if (i > 2 * R) q[i - R - 1] = pack_hi(o[i], o[i - 2 * R - 1]);
+        else if (i > R) q[i - R - 1] = o[i];                    // first r words: the high half comes from the segment before
+        if (i >= N - 2 * R && i < N - R) q[i + R] = o[i];     // last r words: the low half comes from the segment after
+        emit(i, o[i]);
+    }
+}
+// The last pass: emit(i, o_i) only.
+template <int R, int N, class Emit>
+VSZ_HD void pair_slide_out(const uint32_t (&p)[N], uint32_t W, uint32_t C, uint32_t inv2, Emit emit) {
+#pragma unroll
+    for (int i = 0; i <= N; ++i) {
+        emit(i, W * inv2 + C);
+        if (i < N) W = dp2a(p[i], STEP, W);
+    }
+}
+
+// H, a pass that feeds another: also xs[], the first and the last HW words of the own samples (two consecutive samples per
+// word) that the neighbours need.
+template <int R>
+VSZ_HD void h_slide_next(const uint32_t (&p)[NP], uint32_t (&q)[NP], uint32_t (&xs)[2 * HGeom<R>::HW], uint32_t W, uint32_t C,
+                         uint32_t inv2) {
+    constexpr int HW = HGeom<R>::HW;
+    uint32_t prev = 0;
+    pair_slide_next<R>(p, q, W, C, inv2, [&](int i, uint32_t o) {
+        if (i & 1) {
+            if (i < 2 * HW) xs[i >> 1] = pack_hi(prev, o);
+            if (i >= L - 2 * HW) xs[HW + ((i - (L - 2 * HW)) >> 1)] = pack_hi(prev, o);
+        }
+        prev = o;
+    });
+}
+
+// H, the last pass: the outputs packed two consecutive samples per word.
+template <int R>
+VSZ_HD void h_slide_out(const uint32_t (&p)[NP], uint32_t (&out)[LW], uint32_t W, uint32_t C, uint32_t inv2) {
+    uint32_t prev = 0;
+    pair_slide_out<R>(p, W, C, inv2, [&](int i, uint32_t o) {
+        if (i & 1) out[i >> 1] = pack_hi(prev, o);
+        prev = o;
+    });
+}
 
 // window sum of the samples [-R, R] around own[0]
 template <int R>
@@ -131,6 +227,8 @@ VSZ_HD uint32_t h_window(const uint32_t (&ext)[HGeom<R>::NW]) {
     return W;
 }
 
+// The single H pass of the comptime path (ctfused_kernel) works on ext[] as staged: with no next pass to feed, building the
+// pair words would cost a PRMT per sample that nothing reuses.
 // One pass over the owned segment.  The segment is cut into NCH independent chains (each with its own running window
 // sum, started from a window computed out of registers) so that a thread always has NCH dependency chains in flight.
 // Within a chain two steps are taken together:  W1 = t -/+ hi,  W2 = u + hiA - hiB  with t, u the dp2a (low-half)
@@ -189,6 +287,24 @@ VSZ_HD void h_slide(const uint32_t (&ext)[HGeom<R>::NW], uint32_t (&out)[HGeom<R
     }
 }
 
+// The own samples of h_slide_next's q[] (before h_complete_edges), packed two consecutive samples per word: sample i is hi16 of
+// q[i + r] for i < NP - r, else (i - r - 1 >= r + 1) hi16 of a left edge word or lo16 of a complete word.
+template <int R>
+VSZ_HD void h_own_words(const uint32_t (&q)[NP], uint32_t* own) {
+    auto at = [](int i, int& w, bool& hi) {
+        if (i < NP - R) { w = i + R; hi = true; }
+        else { w = i - R - 1; hi = w < R; }
+    };
+#pragma unroll
+    for (int m = 0; m < LW; ++m) {
+        int wa, wb;
+        bool ha, hb;
+        at(2 * m, wa, ha);
+        at(2 * m + 1, wb, hb);
+        own[m] = prmt(q[wa], q[wb], (ha ? 0x32u : 0x10u) | ((hb ? 0x76u : 0x54u) << 8));
+    }
+}
+
 // Loads.  `own` points at the thread's first sample inside the staged row (8-byte aligned).
 template <int R>
 VSZ_HD void h_load_halos(uint32_t (&ext)[HGeom<R>::NW], const uint16_t* own) {
@@ -207,12 +323,23 @@ VSZ_HD void h_load_own(uint32_t (&ext)[HGeom<R>::NW], const uint16_t* own) {
         ld64(own + 2 * k, ext[G::HW + k], ext[G::HW + k + 1]);
     }
 }
+// w = LW words of own samples
+VSZ_HD void h_store_words(const uint32_t* w, uint16_t* own) {
+#pragma unroll
+    for (int k = 0; k < LW; k += 2) st64(own + 2 * k, w[k], w[k + 1]);
+}
 template <int R>
 VSZ_HD void h_store_own(const uint32_t (&ext)[HGeom<R>::NW], uint16_t* own) {
+    h_store_words(ext + HGeom<R>::HW, own);
+}
+// the neighbours' part of h_slide_next's xs[]: the first and the last HW words of the own samples
+template <int R>
+VSZ_HD void h_store_edges(const uint32_t (&xs)[2 * HGeom<R>::HW], uint16_t* own) {
     using G = HGeom<R>;
 #pragma unroll
-    for (int k = 0; k < LW; k += 2) {
-        st64(own + 2 * k, ext[G::HW + k], ext[G::HW + k + 1]);
+    for (int k = 0; k < G::HW; k += 2) {
+        st64(own + 2 * k, xs[k], xs[k + 1]);
+        st64(own + L - 2 * G::HW + 2 * k, xs[G::HW + k], xs[G::HW + k + 1]);
     }
 }
 
@@ -233,21 +360,30 @@ VSZ_HD void st32(uint16_t* p, uint32_t a) {
     memcpy(p, &a, 4);
 #endif
 }
+// first = the lane's first own words (two consecutive samples each), at least (r + 1) / 2 of them
 template <int R>
-VSZ_HD void h_write_left_pad(const uint32_t (&ext)[HGeom<R>::NW], uint16_t* row0) {  // row0 = sample 0 of the staged row
-    using G = HGeom<R>;
+VSZ_HD void h_write_left_pad_words(const uint32_t* first, uint16_t* row0) {  // row0 = sample 0 of the staged row
     constexpr int NWD = (R + 1) / 2;
 #pragma unroll
-    for (int m = 0; m + 1 < NWD; m += 2) st64(row0 - 4 - 2 * m, halfswap(ext[G::HW + m + 1]), halfswap(ext[G::HW + m]));
-    if (NWD & 1) st32(row0 - 2 * NWD, halfswap(ext[G::HW + NWD - 1]));
+    for (int m = 0; m + 1 < NWD; m += 2) st64(row0 - 4 - 2 * m, halfswap(first[m + 1]), halfswap(first[m]));
+    if (NWD & 1) st32(row0 - 2 * NWD, halfswap(first[NWD - 1]));
+}
+// end = one past the lane's last own word
+template <int R>
+VSZ_HD void h_write_right_pad_words(const uint32_t* end, uint16_t* row_end) {  // row_end = sample n (= end of the lane's segment)
+    constexpr int NWD = (R + 1) / 2;
+#pragma unroll
+    for (int m = 0; m + 1 < NWD; m += 2) st64(row_end + 2 * m, halfswap(end[-1 - m]), halfswap(end[-2 - m]));
+    if (NWD & 1) st32(row_end + 2 * (NWD - 1), halfswap(end[-NWD]));
+}
+
+template <int R>
+VSZ_HD void h_write_left_pad(const uint32_t (&ext)[HGeom<R>::NW], uint16_t* row0) {
+    h_write_left_pad_words<R>(ext + HGeom<R>::HW, row0);
 }
 template <int R>
-VSZ_HD void h_write_right_pad(const uint32_t (&ext)[HGeom<R>::NW], uint16_t* row_end) {  // row_end = sample n (= end of the lane's segment)
-    using G = HGeom<R>;
-    constexpr int NWD = (R + 1) / 2;
-#pragma unroll
-    for (int m = 0; m + 1 < NWD; m += 2) st64(row_end + 2 * m, halfswap(ext[G::HW + LW - 1 - m]), halfswap(ext[G::HW + LW - 2 - m]));
-    if (NWD & 1) st32(row_end + 2 * (NWD - 1), halfswap(ext[G::HW + LW - NWD]));
+VSZ_HD void h_write_right_pad(const uint32_t (&ext)[HGeom<R>::NW], uint16_t* row_end) {
+    h_write_right_pad_words<R>(ext + HGeom<R>::HW + LW, row_end);
 }
 
 // =========================================================================== V: a word = the same row of two columns

@@ -131,7 +131,11 @@ __global__ void __launch_bounds__(NWARPS * 32, NWARPS == 4 ? 4 : 2) ctfused_kern
         // ---- H: each lane group blurs one row of means (SYM closed form), in place in tmpb
         {
             uint16_t* row = reinterpret_cast<uint16_t*>(tmpb + (size_t)(warp * RPW + sub) * pj.rowbuf);
-            hseg_pass<R>(e, eo, row, w, sg, G, pj.S, true, act, lane, job.inv, job.inv2);
+            hseg_load_row<R>(e, row, w, sg, G, pj.S, true, act, lane);
+            const uint32_t W = h_window<R>(e);
+            const uint32_t C = __shfl_sync(0xffffffffu, line_const(W, job.inv, job.inv2), lane & ~(G - 1));
+            h_slide<R, kCtChains, false>(e, eo, W, C, job.inv2);
+            __syncwarp();  // every lane has read its halos: the staged row may be overwritten
             if (act) h_store_own<R>(eo, row + Gm::PAD + L * sg);
             __syncwarp();
             // coalesced copy-out of the warp's rows

@@ -50,7 +50,7 @@ __global__ void __launch_bounds__(HSEG_WARPS * 32, VSZ_HSEG_MINB) hseg_kernel(co
     };
     int g = local * pj.per_cta + warp;
     if (lane == 0 && g < g_end) issue(g, 0);
-    uint32_t ea[Gm::NW], eb[Gm::NW];  // pass input / output, swapping roles every pass (no register copies)
+    uint32_t e[Gm::NW], pa[NP], pb[NP], xs[2 * Gm::HW], out[LW];
     for (int it = 0; g < g_end; g += HSEG_WARPS, ++it) {
         const int b = it & 1;
         uint16_t* row = reinterpret_cast<uint16_t*>(wbase + (size_t)(b * RPW + sub) * pj.rowbuf);
@@ -61,28 +61,45 @@ __global__ void __launch_bounds__(HSEG_WARPS * 32, VSZ_HSEG_MINB) hseg_kernel(co
 #pragma unroll
             for (int j = 0; j < L / 4; ++j) {
                 const uint32_t w4 = bown[j];
-                ea[Gm::HW + 2 * j] = __byte_perm(w4, 0u, 0x4140);
-                ea[Gm::HW + 2 * j + 1] = __byte_perm(w4, 0u, 0x4342);
+                e[Gm::HW + 2 * j] = __byte_perm(w4, 0u, 0x4140);
+                e[Gm::HW + 2 * j + 1] = __byte_perm(w4, 0u, 0x4342);
             }
         }
-        hseg_pass<R>(ea, eb, row, n, sg, G, pj.S, !U8, act, lane, job.inv, job.inv2);
+        hseg_load_pairs<R>(e, pa, row, n, sg, G, pj.S, !U8, act, lane);
         if (lane == 0 && g + HSEG_WARPS < g_end) {
             bulk_wait_read0();  // the other buffer's previous rows have left shared memory
             fence_proxy_async();
             issue(g + HSEG_WARPS, b ^ 1);
         }
-        for (int p = 1; p < job.passes; p += 2) {
-            hseg_pass<R>(eb, ea, row, n, sg, G, pj.S, false, act, lane, job.inv, job.inv2);
-            if (p + 1 < job.passes) hseg_pass<R>(ea, eb, row, n, sg, G, pj.S, false, act, lane, job.inv, job.inv2);
+        // Every call site has fixed roles for pa / pb, so that passes need no register copies.
+        auto mid = [&](uint32_t (&in)[NP], uint32_t (&next)[NP]) {
+            uint32_t C;
+            const uint32_t W = hseg_window<R>(in, lane, G, job.inv, job.inv2, C);
+            h_slide_next<R>(in, next, xs, W, C, job.inv2);
+            hseg_next_pairs<R>(e, next, xs, row, n, sg, G, pj.S, act, lane);
+        };
+        auto last = [&](uint32_t (&in)[NP]) {
+            uint32_t C;
+            const uint32_t W = hseg_window<R>(in, lane, G, job.inv, job.inv2, C);
+            h_slide_out<R>(in, out, W, C, job.inv2);
+        };
+        int left = job.passes;
+        for (; left > 2; left -= 2) {
+            mid(pa, pb);
+            mid(pb, pa);
+        }
+        if (left == 2) {
+            mid(pa, pb);
+            last(pb);
+        } else {
+            last(pa);
         }
         if (act) {
             if constexpr (U8) {
-                const uint32_t(&res)[Gm::NW] = (job.passes & 1) ? eb : ea;
 #pragma unroll
-                for (int j = 0; j < L / 4; ++j) bown[j] = __byte_perm(res[Gm::HW + 2 * j], res[Gm::HW + 2 * j + 1], 0x6420);
+                for (int j = 0; j < L / 4; ++j) bown[j] = __byte_perm(out[2 * j], out[2 * j + 1], 0x6420);
             } else {
-                if (job.passes & 1) h_store_own<R>(eb, own);
-                else h_store_own<R>(ea, own);
+                h_store_words(out, own);
             }
         }
         fence_proxy_async();
