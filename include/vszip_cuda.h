@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define VSZIP_CUDA_ABI_VERSION 5  /* 2: + vszip_chain_*, vszip_limiter_*; 3: + vszip_limitfilter_*, vszip_adaptivebinarize_*, vszip_planestats_device; 4: + vszip_cuda_host_forget, vszip_cuda_host_registered_bytes, vszip_cuda_host_register_limit; 5: + vszip_cuda_reserve */
+#define VSZIP_CUDA_ABI_VERSION 5  /* 2: + vszip_chain_*, vszip_limiter_*; 3: + vszip_limitfilter_*, vszip_adaptivebinarize_*, vszip_planestats_device; 4: + vszip_cuda_host_forget, vszip_cuda_host_registered_bytes, vszip_cuda_host_register_limit; 5: + vszip_cuda_reserve, and additions that leave every earlier entry point unchanged: vszip_chain_create2, vszip_planestats_device_b, vszip_cuda_transfer_bytes (a caller that needs them resolves them by name) */
 
 /* VapourSynth4.h values (VSColorFamily / VSSampleType) so the Zig glue can pass vi.format as is. */
 enum { VSZIP_CF_GRAY = 1, VSZIP_CF_RGB = 2, VSZIP_CF_YUV = 3 };
@@ -64,6 +64,10 @@ const char* vszip_cuda_last_error(void);
 int vszip_cuda_abi_version(void);
 /* Number of kernels this library has launched so far in this process (all threads). */
 uint64_t vszip_cuda_kernel_launches(void);
+/* Sample bytes (width * height * bytes per sample of each plane) of the frames this library has copied between host and GPU so far
+ * in this process: direction 0 = host to device, 1 = device to host (the get_frame / chain staging and vszip_dev_clip_upload /
+ * _download; not the small reduction results).  Any other direction returns 0. */
+uint64_t vszip_cuda_transfer_bytes(int32_t direction);
 
 /* Host frame buffers.  getFrame hands over pageable planes owned by the VapourSynth core (getReadPtr / getWritePtr,
  * src/helper.zig:510-531).  Planes that lie entirely inside memory the application page-locked are DMA'd in place; everything
@@ -276,6 +280,14 @@ int vszip_planeaverage_device(const vszip_filter* f, const vszip_dev_clip* clipa
 int vszip_planestats_device(const vszip_filter* minmax, const vszip_filter* average, const vszip_dev_clip* clipa,
                             int32_t first, int32_t count, vszip_minmax_props* minmax_out, vszip_average_props* average_out,
                             int32_t* fused_out, void* stream);
+/* The same with clipb: clipb is the second clip of every filter of the pair that was created with clipb (and must be NULL when
+ * neither was).  One read of each (clipa, clipb) plane pair when both filters were created with clipb and the pair is otherwise
+ * eligible as above (plus: a float clip with thresholds only when its planes have row padding, so that every float sum is
+ * accumulated in the same order as by the separate calls); Diff is accumulated once and reported to both.  Results are bit-identical
+ * to the two separate calls either way. */
+int vszip_planestats_device_b(const vszip_filter* minmax, const vszip_filter* average, const vszip_dev_clip* clipa,
+                              const vszip_dev_clip* clipb, int32_t first, int32_t count, vszip_minmax_props* minmax_out,
+                              vszip_average_props* average_out, int32_t* fused_out, void* stream);
 int vszip_limiter_device(const vszip_filter* f, const vszip_dev_clip* src, vszip_dev_clip* dst,
                          int32_t first, int32_t count, void* stream);
 int vszip_limitfilter_device(const vszip_filter* f, const vszip_dev_clip* flt, const vszip_dev_clip* src,
@@ -301,6 +313,22 @@ int vszip_cuda_stream_sync(int32_t device, void* stream);
  *    the remaining planes equal the source's.  May be NULL when the chain holds no pixel filter. */
 typedef struct vszip_chain vszip_chain;
 vszip_chain* vszip_chain_create(const vszip_filter* const* filters, int32_t count);
+/* A chain that is a small DAG: elements may read the source or an earlier element's pixel output as their extra clips, so
+ * `m = src.BoxBlur().PlaneMinMax(clipb=src)` or `src.Bilateral(ref=src.BoxBlur())` also run with one upload and one download.
+ * Values are numbered 0 = the chain's source frame, k >= 1 = the pixel output of element k - 1 (which must come before the reader
+ * and be a pixel filter).  For element i:
+ *  - input[i]: the clip it filters (its first clip).  input == NULL: every element reads the latest pixel output before it, or the
+ *    source (the linear chain of vszip_chain_create).
+ *  - second[i] / third[i]: its extra clips, -1 = none: PlaneMinMax / PlaneAverage clipb, Bilateral ref, LimitFilter src (second)
+ *    and ref (third), AdaptiveBinarize clip (second; input is its clip2).  Exactly the clips the filter was created with must be
+ *    given.  second / third == NULL: none anywhere.
+ * The chain returns the last element's pixel output, or, when the last element is a PlaneMinMax / PlaneAverage, the value it reads;
+ * vszip_chain_planes reports the planes in which that value differs from the source.  Intermediates live in HBM as long as a
+ * later element reads them.  vszip_chain_create(f, n) equals vszip_chain_create2 with input == NULL and second[i] = 0 for its
+ * diamond elements.  An adjacent PlaneMinMax + PlaneAverage that read the same value with the same planes and clipb (or none) share
+ * one read when vszip_planestats_device_b would fuse them, with bit-identical results. */
+vszip_chain* vszip_chain_create2(const vszip_filter* const* filters, int32_t count, const int32_t* input, const int32_t* second,
+                                 const int32_t* third);
 void vszip_chain_free(vszip_chain* c);
 int vszip_chain_planes(const vszip_chain* c, int32_t written[3]);
 int vszip_chain_get_frame(const vszip_chain* c, int32_t n, const vszip_frame* src, vszip_frame* dst, void* const* props_out);

@@ -102,6 +102,7 @@ ABI = {
     "vszip_cuda_last_error": (C.c_char_p, []),
     "vszip_cuda_abi_version": (C.c_int, []),
     "vszip_cuda_kernel_launches": (C.c_uint64, []),
+    "vszip_cuda_transfer_bytes": (C.c_uint64, [C.c_int32]),
     "vszip_cuda_stream_sync": (C.c_int, [C.c_int32, _P]),
     "vszip_cuda_host_forget": (None, [_P]),
     "vszip_cuda_host_registered_bytes": (C.c_size_t, []),
@@ -121,6 +122,8 @@ ABI = {
     "vszip_planeaverage_get_frame": (C.c_int, [_P, C.c_int32, C.POINTER(_Frame), C.POINTER(_Frame), C.POINTER(_AverageProps)]),
     "vszip_planeaverage_device": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int32, C.POINTER(_AverageProps), _P]),
     "vszip_planestats_device": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int32, C.POINTER(_MinMaxProps), C.POINTER(_AverageProps), C.POINTER(C.c_int32), _P]),
+    "vszip_planestats_device_b": (C.c_int, [_P, _P, _P, _P, C.c_int32, C.c_int32, C.POINTER(_MinMaxProps), C.POINTER(_AverageProps),
+                                            C.POINTER(C.c_int32), _P]),
     "vszip_filter_free": (None, [_P]),
     "vszip_filter_planes": (C.c_int, [_P, C.POINTER(C.c_int32 * 3)]),
     "vszip_dev_clip_alloc": (_P, [C.POINTER(_VideoInfo), C.c_int32, C.c_int32]),
@@ -141,6 +144,7 @@ ABI = {
     "vszip_adaptivebinarize_get_frame": (C.c_int, [_P, C.c_int32, C.POINTER(_Frame), C.POINTER(_Frame), C.POINTER(_Frame)]),
     "vszip_adaptivebinarize_device": (C.c_int, [_P, _P, _P, _P, C.c_int32, C.c_int32, _P]),
     "vszip_chain_create": (_P, [C.POINTER(_P), C.c_int32]),
+    "vszip_chain_create2": (_P, [C.POINTER(_P), C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "vszip_chain_free": (None, [_P]),
     "vszip_chain_planes": (C.c_int, [_P, C.POINTER(C.c_int32 * 3)]),
     "vszip_chain_get_frame": (C.c_int, [_P, C.c_int32, C.POINTER(_Frame), C.POINTER(_Frame), C.POINTER(_P)]),
@@ -426,14 +430,20 @@ class PlaneAverageFilter(_Filter):
         return [self.to_props(out[i], prop) for i in range(count)]
 
 
-def plane_stats_device(minmax: "PlaneMinMaxFilter", average: "PlaneAverageFilter", clipa, first=0, count=None, stream=None, prop="psm", fetch=True):
-    """PlaneMinMax + PlaneAverage over the same device-resident frames (vszip_planestats_device): one read of each plane when the pair
-    is eligible.  Returns (props per frame - both filters' props merged, like `clip.vszip.PlaneMinMax().vszip.PlaneAverage()` -, fused)."""
+def plane_stats_device(minmax: "PlaneMinMaxFilter", average: "PlaneAverageFilter", clipa, first=0, count=None, stream=None, prop="psm", fetch=True,
+                       clipb=None):
+    """PlaneMinMax + PlaneAverage over the same device-resident frames (vszip_planestats_device, or vszip_planestats_device_b with
+    clipb): one read of each plane (pair) when the pair is eligible.  Returns (props per frame - both filters' props merged, like
+    `clip.vszip.PlaneMinMax().vszip.PlaneAverage()` -, fused)."""
     count = clipa.num_frames - first if count is None else count
     mm = (_MinMaxProps * max(count, 1))() if fetch else None
     av = (_AverageProps * max(count, 1))() if fetch else None
     fused = C.c_int32(0)
-    _check(load_library().vszip_planestats_device(minmax.handle, average.handle, clipa.handle, first, count, mm, av, C.byref(fused), stream))
+    if clipb is None:
+        _check(load_library().vszip_planestats_device(minmax.handle, average.handle, clipa.handle, first, count, mm, av, C.byref(fused), stream))
+    else:
+        _check(load_library().vszip_planestats_device_b(minmax.handle, average.handle, clipa.handle, clipb.handle, first, count, mm, av,
+                                                        C.byref(fused), stream))
     if not fetch:
         return None, bool(fused.value)
     out = []
@@ -541,7 +551,7 @@ class _Namespace:
                 f = LimitFilterFilter(flt._info(), src._info(), ref._info() if ref is not None else None, dark_thr, bright_thr, elast, planes, cr)
         return _multi_node(flt, [src] + ([ref] if ref is not None else []), f, lambda n, a, others, d: load_library().vszip_limitfilter_get_frame(
             f.handle, n, C.byref(a), C.byref(others[0]), C.byref(others[1]) if len(others) > 1 else None, C.byref(d)),
-            through=flt if ref is None else None, needs_source=src)
+            through=flt, extra=(src, ref))
 
     def AdaptiveBinarize(self, *pos, **kw) -> VideoNode:
         clip, clip2, c = self._bind(("clip", "clip2", "c"), pos, kw)
@@ -550,7 +560,7 @@ class _Namespace:
         f = AdaptiveBinarizeFilter(clip._info(), clip2._info(), c)
         return _multi_node(clip, [clip2], f, lambda n, a, others, d: load_library().vszip_adaptivebinarize_get_frame(
             f.handle, n, C.byref(a), C.byref(others[0]), C.byref(d)), {"_ColorRange": 0},  # dst_prop.setColorRange(.FULL)
-            through=clip2, needs_source=clip)
+            through=clip2, extra=(clip, None))
 
     def Bilateral(self, clip=None, ref=None, sigmaS=None, sigmaR=None, planes=None, algorithm=None, PBFICnum=None) -> VideoNode:
         clip = self._c(clip)
@@ -606,10 +616,12 @@ def _pixel_node(clip: VideoNode, ref: VideoNode | None, flt: _Filter, call) -> V
     node = VideoNode(fmt, clip.width, clip.height, clip.num_frames, get)
     node.filter = flt
     node._chain_info = ("pixel", clip, ref, None)
+    node._extra = (ref, None)
+    node._props_of = clip
     return node
 
 
-def _multi_node(first: VideoNode, others, flt: _Filter, call, set_props=None, through=None, needs_source=None) -> VideoNode:
+def _multi_node(first: VideoNode, others, flt: _Filter, call, set_props=None, through=None, extra=(None, None)) -> VideoNode:
     """A pixel filter with several input clips (LimitFilter, AdaptiveBinarize): dst is allocated from `first`."""
     fmt = first.format
 
@@ -627,12 +639,11 @@ def _multi_node(first: VideoNode, others, flt: _Filter, call, set_props=None, th
 
     node = VideoNode(fmt, first.width, first.height, first.num_frames, get)
     node.filter = flt
-    # "diamond" element of a fused chain: `through` is the input that continues the chain, `needs_source` the clip that must turn
-    # out to be the chain's source (checked in _fusable_chain); anything else (a ref clip, ...) is never fused
-    node._chain_info = ("pixel", through, None, None) if through is not None else None
-    node._needs_source = needs_source
+    # in a fused chain `through` is the input the filter works on (the chain's main line), `extra` its second / third clips
+    node._chain_info = ("pixel", through, None, None)
+    node._extra = tuple(extra)
     node._set_props = set_props
-    node._props_from_source = needs_source is not None and first is needs_source   # dst = first.newVideoFrame(): props of `first` only
+    node._props_of = first                       # dst = first.newVideoFrame(): props of `first` only
     return node
 
 
@@ -653,15 +664,19 @@ def _props_node(clipa: VideoNode, clipb: VideoNode | None, flt: _Filter, run, dr
     node = VideoNode(clipa.format, clipa.width, clipa.height, clipa.num_frames, get)
     node.filter = flt
     node._chain_info = ("props", clipa, clipb, (run_fused, drop_keys))
+    node._extra = (clipb, None)
+    node._props_of = clipa
     return node
 
 
-# ---- fused evaluation of linear chains of vszip nodes (vszip_chain_*): one upload, one download
+# ---- fused evaluation of chains of vszip nodes (vszip_chain_*): one upload, one download
 class _Chain:
-    def __init__(self, nodes):
+    def __init__(self, nodes, inputs, second, third):
         self.nodes = nodes  # evaluation order
-        handles = (_P * len(nodes))(*[nd.filter.handle for nd in nodes])
-        self.handle = load_library().vszip_chain_create(handles, len(nodes))
+        n = len(nodes)
+        handles = (_P * n)(*[nd.filter.handle for nd in nodes])
+        arrs = [(C.c_int32 * n)(*v) for v in (inputs, second, third)]
+        self.handle = load_library().vszip_chain_create2(handles, n, *arrs)
         if not self.handle:
             raise Error(_last_error())
         w = (C.c_int32 * 3)()
@@ -678,18 +693,56 @@ class _Chain:
 
 
 def _fusable_chain(node: "VideoNode"):
-    """The chain ending in `node` if it and at least one predecessor are single-input vszip nodes."""
+    """The chain ending in `node` if it and at least one predecessor are vszip nodes whose clips come from inside the chain."""
     cached = getattr(node, "_chain", False)
     if cached is not False:
         return cached
-    nodes, cur = [], node
-    while getattr(cur, "_chain_info", None) is not None and cur._chain_info[2] is None and len(nodes) < 16:
-        nodes.append(cur)
+    main, cur = [], node
+    while getattr(cur, "_chain_info", None) is not None and len(main) < 16:
+        main.append(cur)
         cur = cur._chain_info[1]
-    # diamond elements (LimitFilter's src, AdaptiveBinarize's clip) must read exactly the chain's source
-    ok = all(getattr(nd, "_needs_source", None) is None or nd._needs_source is cur for nd in nodes)
-    node._chain = (_Chain(nodes[::-1]), cur) if len(nodes) >= 2 and ok else None
+    node._chain = _plan_chain(main[::-1], cur)
     return node._chain
+
+
+def _side_input(x, value):
+    """A single-input pixel node that is not on the main line but filters a value of the chain (`src.vszip.BoxBlur()` given as
+    ref / clipb): it joins the chain right before its reader."""
+    return getattr(x, "_chain_info", None) is not None and x._chain_info[0] == "pixel" and not any(
+        e is not None for e in x._extra) and value(x._chain_info[1]) is not None
+
+
+def _plan_chain(main, source):
+    """Elements and value numbers (0 = source, k = output of element k - 1) for vszip_chain_create2.  Walks the main line from the
+    source end; a node with an extra clip from outside the chain becomes the source of what follows it."""
+    while main:
+        elems, vals, cut = [], {id(source): 0}, None
+        value = lambda x: vals.get(id(x))
+        for k, nd in enumerate(main):
+            side = []
+            for x in nd._extra:
+                if x is None or value(x) is not None or any(x is y for y in side):
+                    continue
+                if not _side_input(x, value):
+                    cut = k
+                    break
+                side.append(x)
+            if cut is not None:
+                break
+            for x in side + [nd]:
+                elems.append(x)
+                vals[id(x)] = len(elems) if x._chain_info[0] == "pixel" else value(x._chain_info[1])  # stats pass their input on
+        if cut is not None:
+            source, main = main[cut], main[cut + 1:]
+        elif len(elems) > 16:
+            source, main = main[0], main[1:]
+        else:
+            break
+    if not main or len(elems) < 2:
+        return None
+    inputs = [value(x._chain_info[1]) for x in elems]
+    second, third = ([-1 if x._extra[j] is None else value(x._extra[j]) for x in elems] for j in (0, 1))
+    return _Chain(elems, inputs, second, third), source
 
 
 def _fused_get(chain_and_source, n: int) -> "VideoFrame":
@@ -708,17 +761,18 @@ def _fused_get(chain_and_source, n: int) -> "VideoFrame":
             ptrs[i] = C.cast(C.pointer(o), _P)
         outs.append(o)
     _check(load_library().vszip_chain_get_frame(chain.handle, n, C.byref(s), C.byref(d), ptrs))
-    props = dict(src.props)
-    for nd, o in zip(chain.nodes, outs):        # evaluation order, exactly what the unfused nodes would do to the props
+    # every node's props, in evaluation order, exactly as the unfused nodes derive them from the clip their frame comes from
+    props = {id(source): dict(src.props)}
+    for nd, o in zip(chain.nodes, outs):
+        p = dict(props[id(nd._props_of)])
         if o is not None:
             to_props, drop_keys = nd._chain_info[3]
             for k in drop_keys:
-                props.pop(k, None)
-            props.update(to_props(o))
-        if getattr(nd, "_props_from_source", False):
-            props = dict(src.props)             # e.g. AdaptiveBinarize(src, src.BoxBlur().PlaneMinMax()): clip2's props are not inherited
-        props.update(getattr(nd, "_set_props", None) or {})
-    return VideoFrame(source.format, source.width, source.height, out_planes, props)
+                p.pop(k, None)
+            p.update(to_props(o))
+        p.update(getattr(nd, "_set_props", None) or {})
+        props[id(nd)] = p
+    return VideoFrame(source.format, source.width, source.height, out_planes, props[id(chain.nodes[-1])])
 
 
 # --------------------------------------------------------------------------- device-resident clips
@@ -772,7 +826,7 @@ class DeviceClip:
 class _Core:
     def __init__(self):
         self._ready = False
-        # evaluate linear chains of single-input vszip nodes with one upload and one download (vszip_chain_*)
+        # evaluate chains of vszip nodes with one upload and one download (vszip_chain_*)
         self.fuse_chains = os.environ.get("VSZIP_FUSE_CHAINS", "1") != "0"
 
     def init(self, devices=None) -> int:
@@ -815,6 +869,13 @@ class _Core:
     @property
     def kernel_launches(self) -> int:
         return int(load_library().vszip_cuda_kernel_launches())
+
+    def transfer_bytes(self, direction=None):
+        """vszip_cuda_transfer_bytes: sample bytes of frames copied so far, (host->device, device->host), or one direction (0 / 1)."""
+        lib = load_library()
+        if direction is not None:
+            return int(lib.vszip_cuda_transfer_bytes(direction))
+        return int(lib.vszip_cuda_transfer_bytes(0)), int(lib.vszip_cuda_transfer_bytes(1))
 
     def sync(self, device=0, stream=None):
         _check(load_library().vszip_cuda_stream_sync(device, stream))

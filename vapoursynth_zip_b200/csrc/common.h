@@ -18,6 +18,8 @@ namespace vsz {
 void set_error(const char* fmt, ...);
 extern std::atomic<uint64_t> g_launches;
 inline void count_launch(int n = 1) { g_launches.fetch_add((uint64_t)n, std::memory_order_relaxed); }
+extern std::atomic<uint64_t> g_transfer[2];  // sample bytes of frames moved host -> device [0] / device -> host [1]
+inline void count_transfer(int dir, size_t bytes) { g_transfer[dir].fetch_add((uint64_t)bytes, std::memory_order_relaxed); }
 
 #define VSZ_CUDA(call)                                                                              \
     do {                                                                                            \
@@ -90,6 +92,8 @@ struct Slot {  // one in-flight getFrame request
     size_t cap[4] = {0, 0, 0, 0};
     void* pin_small = nullptr;  // 4 KB pinned scratch for tiny results
     void* dev_small = nullptr;  // 64 KB device scratch for reductions
+    std::vector<char*> xdev;    // device-only frame buffers beyond dev[] (fused chains whose buffer plan needs more), grown on demand
+    std::vector<size_t> xcap;
     bool streaming_copies = false;  // set at acquire(): the host is crowded, staging copies bypass the cache
 };
 
@@ -108,6 +112,7 @@ int num_devices();
 DeviceCtx* device_ctx(int index);                // index into the init list
 DeviceCtx* device_for_frame(int32_t n);          // n mod k routing
 int slot_reserve(DeviceCtx* d, Slot* s, int which, size_t bytes);  // grow pin[which]/dev[which]
+int slot_reserve_extra(DeviceCtx* d, Slot* s, int which, size_t bytes);  // grow xdev[which] (no pinned twin)
 
 // host <-> slot staging of the selected planes of one frame (async on s->stream)
 int stage_in(Slot* s, int which, const FrameLayout& l, const vszip_frame* host, const bool mask[3]);

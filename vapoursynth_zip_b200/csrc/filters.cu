@@ -5,6 +5,7 @@
 #include <cmath>
 #include <cstdio>
 #include <cstring>
+#include <array>
 #include <limits>
 #include <string>
 
@@ -727,13 +728,15 @@ int vszip_planeaverage_device(const vszip_filter* f, const vszip_dev_clip* a, co
 }
 
 // =========================================================================== PlaneMinMax + PlaneAverage from one read (SURVEY 8f rank 4)
-int vszip_planestats_device(const vszip_filter* fm, const vszip_filter* fa, const vszip_dev_clip* a, int32_t first, int32_t count,
-                            vszip_minmax_props* mm_out, vszip_average_props* avg_out, int32_t* fused_out, void* stream) {
+// b: the clipb clip (may be nullptr); a filter created without clipb ignores it.  The pair shares one read only when both filters read
+// b (or neither does).
+static int planestats_run(const vszip_filter* fm, const vszip_filter* fa, const vszip_dev_clip* a, const vszip_dev_clip* b, int32_t first,
+                          int32_t count, bool same_float_sums, vszip_minmax_props* mm_out, vszip_average_props* avg_out, int32_t* fused_out,
+                          void* stream) {
     static const char* name = "PlaneStats";
-    if (fused_out) *fused_out = 0;
-    if (!fm || fm->kind != F_PLANEMINMAX || !fa || fa->kind != F_PLANEAVERAGE) { set_error("PlaneStats: a PlaneMinMax and a PlaneAverage handle are required"); return -1; }
-    if (fm->has_ref || fa->has_ref) { set_error("PlaneStats: filters created with clipb cannot be combined"); return -1; }
     if (!same_clip_shape(a, fm, name) || !same_clip_shape(a, fa, name) || !range_ok(a, first, count, name)) return -1;
+    if (b && (!same_clip_shape(b, fm, name) || !range_ok(b, first, count, name))) return -1;
+    if (b && b->device_index != a->device_index) { set_error("%s: clips live on different devices", name); return -1; }
     DeviceCtx* d = device_ctx(a->device_index);
     if (!d) { set_error("PlaneStats: library not initialised"); return -1; }
     VSZ_CUDA(cudaSetDevice(d->ordinal));
@@ -742,6 +745,9 @@ int vszip_planestats_device(const vszip_filter* fm, const vszip_filter* fa, cons
     if (count == 0) return 0;
     const size_t fs = a->layout.frame_stride;
     const char* base = a->base + (size_t)first * fs;
+    const char* bbase = b ? b->base + (size_t)first * fs : nullptr;
+    const char* bm = fm->has_ref ? bbase : nullptr;
+    const char* ba = fa->has_ref ? bbase : nullptr;
     const bool same_planes = fm->process[0] == fa->process[0] && fm->process[1] == fa->process[1] && fm->process[2] == fa->process[2];
     const size_t sbm = stats_scratch_bytes(count, std::max(npm, 1)), sba = stats_scratch_bytes(count, std::max(npa, 1));
     const size_t rbm = sizeof(StatsRaw) * (size_t)count * npm, rba = sizeof(StatsRaw) * (size_t)count * npa;
@@ -752,16 +758,16 @@ int vszip_planestats_device(const vszip_filter* fm, const vszip_filter* fa, cons
     StatsRaw* raw_m = (StatsRaw*)(scratch + sbm + sba);
     StatsRaw* raw_a = (StatsRaw*)(scratch + sbm + sba + rbm_al);
     int rc = 1;
-    if (same_planes && npm > 0 && fa->exclude_i.size() <= 16)
-        rc = run_planestats_fused(fm->layout, fm->process, base, fs, count, fm->no_thr, fm->minthr, fm->maxthr, fm->hist_size,
-                                  fa->exclude_i.data(), fa->exclude_f.data(), (int)fa->exclude_i.size(), scratch, raw_m, raw_a, st);
+    if (same_planes && npm > 0 && fa->exclude_i.size() <= 16 && bm == ba)
+        rc = run_planestats_fused(fm->layout, fm->process, base, fs, bm, fs, count, fm->no_thr, fm->minthr, fm->maxthr, fm->hist_size,
+                                  fa->exclude_i.data(), fa->exclude_f.data(), (int)fa->exclude_i.size(), same_float_sums, scratch, raw_m, raw_a, st);
     if (rc == 0 && fused_out) *fused_out = 1;
     if (rc == 1) {  // not eligible: the two reductions one after the other (two reads)
         rc = 0;
-        if (npm) rc = run_planeminmax(fm->layout, fm->process, base, fs, nullptr, fs, count, fm->no_thr, fm->minthr, fm->maxthr, fm->hist_size, scratch, raw_m, st);
+        if (npm) rc = run_planeminmax(fm->layout, fm->process, base, fs, bm, fs, count, fm->no_thr, fm->minthr, fm->maxthr, fm->hist_size, scratch, raw_m, st);
         const int32_t* xi; const float* xf;
         if (!rc && npa && average_upload(fa, a->device_index, &xi, &xf)) rc = -1;
-        if (!rc && npa) rc = run_planeaverage(fa->layout, fa->process, base, fs, nullptr, fs, count, fa->exclude_i.data(), fa->exclude_f.data(),
+        if (!rc && npa) rc = run_planeaverage(fa->layout, fa->process, base, fs, ba, fs, count, fa->exclude_i.data(), fa->exclude_f.data(),
                                                (int)fa->exclude_i.size(), xi, xf, scratch + sbm, raw_a, st);
     }
     if (!rc && (mm_out || avg_out)) {
@@ -775,6 +781,22 @@ int vszip_planestats_device(const vszip_filter* fm, const vszip_filter* fa, cons
         }
     }
     return rc;
+}
+
+int vszip_planestats_device(const vszip_filter* fm, const vszip_filter* fa, const vszip_dev_clip* a, int32_t first, int32_t count,
+                            vszip_minmax_props* mm_out, vszip_average_props* avg_out, int32_t* fused_out, void* stream) {
+    if (fused_out) *fused_out = 0;
+    if (!fm || fm->kind != F_PLANEMINMAX || !fa || fa->kind != F_PLANEAVERAGE) { set_error("PlaneStats: a PlaneMinMax and a PlaneAverage handle are required"); return -1; }
+    if (fm->has_ref || fa->has_ref) { set_error("PlaneStats: filters created with clipb cannot be combined"); return -1; }
+    return planestats_run(fm, fa, a, nullptr, first, count, false, mm_out, avg_out, fused_out, stream);
+}
+
+int vszip_planestats_device_b(const vszip_filter* fm, const vszip_filter* fa, const vszip_dev_clip* a, const vszip_dev_clip* b, int32_t first,
+                              int32_t count, vszip_minmax_props* mm_out, vszip_average_props* avg_out, int32_t* fused_out, void* stream) {
+    if (fused_out) *fused_out = 0;
+    if (!fm || fm->kind != F_PLANEMINMAX || !fa || fa->kind != F_PLANEAVERAGE) { set_error("PlaneStats: a PlaneMinMax and a PlaneAverage handle are required"); return -1; }
+    if ((fm->has_ref || fa->has_ref) != (b != nullptr)) { set_error("PlaneStats: clipb presence does not match the filter instances"); return -1; }
+    return planestats_run(fm, fa, a, b, first, count, true, mm_out, avg_out, fused_out, stream);
 }
 
 // =========================================================================== Limiter
@@ -1032,42 +1054,186 @@ int vszip_adaptivebinarize_device(const vszip_filter* f, const vszip_dev_clip* c
 }
 
 // =========================================================================== fused chains
+// Values of a chain: 0 = the source frame, k >= 1 = the pixel output of element k - 1.  Every element reads its main input (the
+// value it filters) and up to two extra inputs; the buffer plan gives every pixel output a frame buffer for as long as a later
+// element reads it (DESIGN.md §5.1).  Buffers 0..2 are the slot's dev[0..2] (0 = the source, never written; 2 = the value the
+// chain returns, the D2H source), buffers 3.. are the slot's device-only extras.
 struct vszip_chain {
     std::vector<const vszip_filter*> fl;
     vsz::FrameLayout layout;
     bool written[3];
     int npixel;
+    std::vector<int> in, in2, in3;  // buffer of each element's main / second / third input (-1: none)
+    std::vector<int> out;           // buffer of each element's pixel output (-1: stats element)
+    std::vector<char> fuse_next;    // stats element i runs together with element i + 1 from one read
+    std::vector<char> used;         // buffers the plan uses (0..2: the slot's dev[], 3..: its device-only extras)
 };
+
+namespace {
+
+bool is_pixel(const vszip_filter* f) {
+    return f->kind == F_BOXBLUR || f->kind == F_BILATERAL || f->kind == F_LIMITER || f->kind == F_LIMITFILTER || f->kind == F_ADAPTIVEBINARIZE;
+}
+
+const char* kind_name(const vszip_filter* f) {
+    switch (f->kind) {
+        case F_BOXBLUR: return "BoxBlur";
+        case F_BILATERAL: return "Bilateral";
+        case F_PLANEMINMAX: return "PlaneMinMax";
+        case F_PLANEAVERAGE: return "PlaneAverage";
+        case F_LIMITER: return "Limiter";
+        case F_LIMITFILTER: return "LimitFilter";
+        default: return "AdaptiveBinarize";
+    }
+}
+
+// The filter's own names for its second / third input and whether it was created with them.
+void extra_inputs(const vszip_filter* f, const char* names[2], bool has[2]) {
+    names[0] = names[1] = nullptr;
+    has[0] = has[1] = false;
+    switch (f->kind) {
+        case F_BILATERAL: names[0] = "ref"; has[0] = f->has_ref; break;
+        case F_PLANEMINMAX: case F_PLANEAVERAGE: names[0] = "clipb"; has[0] = f->has_ref; break;
+        case F_LIMITFILTER: names[0] = "src"; has[0] = true; names[1] = "ref"; has[1] = f->lf_has_ref; break;
+        case F_ADAPTIVEBINARIZE: names[0] = "clip"; has[0] = true; break;
+        default: break;
+    }
+}
+
+bool same_format(const vszip_video_info& a, const vszip_video_info& b) {
+    return a.width == b.width && a.height == b.height && a.color_family == b.color_family && a.sample_type == b.sample_type &&
+           a.bits_per_sample == b.bits_per_sample && a.sub_sampling_w == b.sub_sampling_w && a.sub_sampling_h == b.sub_sampling_h &&
+           a.num_planes == b.num_planes;
+}
+
+bool stats_pair(const vszip_filter* x, const vszip_filter* y) {
+    if (!((x->kind == F_PLANEMINMAX && y->kind == F_PLANEAVERAGE) || (x->kind == F_PLANEAVERAGE && y->kind == F_PLANEMINMAX))) return false;
+    const vszip_filter* fa = x->kind == F_PLANEAVERAGE ? x : y;
+    return x->process[0] == y->process[0] && x->process[1] == y->process[1] && x->process[2] == y->process[2] && processed_planes(x) > 0 &&
+           fa->exclude_i.size() <= 16;
+}
+
+// input / second / third use the value numbering above; input == nullptr: every element reads the latest pixel output (or the source).
+vszip_chain* chain_build(const vszip_filter* const* filters, int count, const int32_t* input, const int32_t* second, const int32_t* third) {
+    const int nv = count + 1;
+    std::vector<int> vin(count), v2(count), v3(count);
+    std::vector<int> last_use(nv, -1), def(nv, -1);
+    int cur = 0;
+    for (int i = 0; i < count; ++i) {
+        vin[i] = input ? input[i] : cur;
+        v2[i] = second ? second[i] : -1;
+        v3[i] = third ? third[i] : -1;
+        if (is_pixel(filters[i])) { cur = i + 1; def[i + 1] = i; }
+    }
+    // the value the chain returns: the last element's pixel output, or the value a final stats element reads
+    const vszip_filter* fl = filters[count - 1];
+    const int result = is_pixel(fl) ? count : vin[count - 1];
+    vszip_chain* c = new vszip_chain();
+    c->fl.assign(filters, filters + count);
+    c->layout = filters[0]->layout;
+    c->npixel = 0;
+    for (int i = 0; i < count; ++i) {
+        for (int v : {vin[i], v2[i], v3[i]}) if (v >= 0) last_use[v] = std::max(last_use[v], i);
+        c->npixel += is_pixel(filters[i]) ? 1 : 0;
+    }
+    // planes in which each value differs from the source
+    std::vector<std::array<bool, 3>> diff(nv, std::array<bool, 3>{false, false, false});
+    for (int i = 0; i < count; ++i)
+        if (is_pixel(filters[i]))
+            for (int p = 0; p < 3; ++p) diff[i + 1][p] = diff[vin[i]][p] || filters[i]->process[p];
+    for (int p = 0; p < 3; ++p) c->written[p] = diff[result][p];
+    // buffer plan: a value occupies its buffer from the element that writes it to the last element that reads it (both inclusive,
+    // so an element never writes the buffer it reads).  The result goes to buffer 2 and lives to the end; the other pixel outputs,
+    // latest first, take the lowest buffer >= 1 that is free over their whole span - for a linear chain that is the 1 / 2
+    // alternation ending in 2.
+    std::vector<int> buf(nv, -1);
+    buf[0] = 0;
+    std::vector<std::vector<std::pair<int, int>>> busy(3);
+    if (result > 0) { buf[result] = 2; busy[2].push_back({def[result], count}); }
+    for (int v = count; v >= 1; --v) {
+        if (def[v] < 0 || v == result) continue;
+        const int lo = def[v], hi = std::max(last_use[v], def[v]);
+        int b = 1;
+        for (;; ++b) {
+            if ((int)busy.size() <= b) busy.resize(b + 1);
+            bool free_ = true;
+            for (auto& r : busy[b]) free_ = free_ && (hi < r.first || r.second < lo);
+            if (free_) break;
+        }
+        buf[v] = b;
+        busy[b].push_back({lo, hi});
+    }
+    c->used.assign(busy.size(), 0);
+    c->used[0] = c->used[2] = 1;
+    for (int v = 1; v < nv; ++v) if (buf[v] >= 0) c->used[buf[v]] = 1;
+    for (int i = 0; i < count; ++i) {
+        c->in.push_back(buf[vin[i]]);
+        c->in2.push_back(v2[i] >= 0 ? buf[v2[i]] : -1);
+        c->in3.push_back(v3[i] >= 0 ? buf[v3[i]] : -1);
+        c->out.push_back(is_pixel(filters[i]) ? buf[i + 1] : -1);
+    }
+    c->fuse_next.assign(count, 0);
+    for (int i = 0; i + 1 < count; ++i) {
+        if (stats_pair(filters[i], filters[i + 1]) && vin[i] == vin[i + 1] && v2[i] == v2[i + 1]) {
+            c->fuse_next[i] = 1;
+            ++i;
+        }
+    }
+    return c;
+}
+
+}  // namespace
 
 vszip_chain* vszip_chain_create(const vszip_filter* const* filters, int32_t count) {
     if (!filters || count < 1 || count > 16) { set_error("chain: between 1 and 16 filters are required"); return nullptr; }
     const vszip_filter* f0 = filters[0];
+    int32_t second[16];
     for (int i = 0; i < count; ++i) {
         const vszip_filter* f = filters[i];
         if (!f) { set_error("chain: filter %d is NULL", i); return nullptr; }
         // LimitFilter (without ref) and AdaptiveBinarize take the chain's SOURCE frame as their second clip ("diamond" elements)
         const bool diamond = (f->kind == F_LIMITFILTER && !f->lf_has_ref) || f->kind == F_ADAPTIVEBINARIZE;
         if (f->has_ref && !diamond) { set_error("chain: filter %d takes a second clip (ref/clipb); only single-input filters can be fused", i); return nullptr; }
-        const vszip_video_info &a = f0->vi, &b = f->vi;
-        if (a.width != b.width || a.height != b.height || a.color_family != b.color_family || a.sample_type != b.sample_type ||
-            a.bits_per_sample != b.bits_per_sample || a.sub_sampling_w != b.sub_sampling_w || a.sub_sampling_h != b.sub_sampling_h ||
-            a.num_planes != b.num_planes) {
+        if (!same_format(f0->vi, f->vi)) {
             set_error("chain: filter %d was created for a different video format than filter 0", i);
             return nullptr;
         }
+        second[i] = diamond ? 0 : -1;
     }
-    vszip_chain* c = new vszip_chain();
-    c->fl.assign(filters, filters + count);
-    c->layout = f0->layout;
-    c->npixel = 0;
-    for (int p = 0; p < 3; ++p) c->written[p] = false;
-    for (const vszip_filter* f : c->fl) {
-        if (f->kind == F_BOXBLUR || f->kind == F_BILATERAL || f->kind == F_LIMITER || f->kind == F_LIMITFILTER || f->kind == F_ADAPTIVEBINARIZE) {
-            ++c->npixel;
-            for (int p = 0; p < 3; ++p) c->written[p] = c->written[p] || f->process[p];
+    return chain_build(filters, count, nullptr, second, nullptr);
+}
+
+vszip_chain* vszip_chain_create2(const vszip_filter* const* filters, int32_t count, const int32_t* input, const int32_t* second,
+                                 const int32_t* third) {
+    if (!filters || count < 1 || count > 16) { set_error("chain: between 1 and 16 filters are required"); return nullptr; }
+    const vszip_filter* f0 = filters[0];
+    for (int i = 0; i < count; ++i) {
+        const vszip_filter* f = filters[i];
+        if (!f) { set_error("chain: filter %d is NULL", i); return nullptr; }
+        if (!same_format(f0->vi, f->vi)) {
+            set_error("chain: filter %d was created for a different video format than filter 0", i);
+            return nullptr;
+        }
+        const char* names[2];
+        bool has[2];
+        extra_inputs(f, names, has);
+        const int32_t refs[3] = {input ? input[i] : 0, second ? second[i] : -1, third ? third[i] : -1};
+        static const char* arr[3] = {"input", "second", "third"};
+        static const char* none[3] = {"", "a second clip", "a third clip"};
+        for (int k = 0; k < 3; ++k) {
+            const int32_t v = refs[k];
+            if (k > 0) {
+                const char* what = names[k - 1] ? names[k - 1] : none[k];
+                if (!has[k - 1] && v != -1) { set_error("chain: filter %d (%s) was created without %s; %s[%d] must be -1", i, kind_name(f), what, arr[k], i); return nullptr; }
+                if (has[k - 1] && v == -1) { set_error("chain: filter %d (%s) was created with %s; %s[%d] must name its input", i, kind_name(f), what, arr[k], i); return nullptr; }
+                if (v == -1) continue;
+            }
+            if (v < 0 || v > count) { set_error("chain: %s[%d] = %d is out of range (0 = the source, k = the output of filter k - 1)", arr[k], i, v); return nullptr; }
+            if (v >= 1 && v - 1 >= i) { set_error("chain: %s[%d] names filter %d, which does not come before filter %d", arr[k], i, v - 1, i); return nullptr; }
+            if (v >= 1 && !is_pixel(filters[v - 1])) { set_error("chain: %s[%d] names filter %d (%s), which has no pixel output", arr[k], i, v - 1, kind_name(filters[v - 1])); return nullptr; }
         }
     }
-    return c;
+    return chain_build(filters, count, input, second, third);
 }
 
 void vszip_chain_free(vszip_chain* c) { delete c; }
@@ -1088,40 +1254,43 @@ int vszip_chain_get_frame(const vszip_chain* c, int32_t n, const vszip_frame* sr
     VSZ_CUDA(cudaSetDevice(d->ordinal));
     const FrameLayout& l = c->layout;
     const size_t bytes = l.frame_stride;
-    if (slot_reserve(d, s, 0, bytes) || slot_reserve(d, s, 2, bytes) || (c->npixel > 1 && slot_reserve(d, s, 1, bytes))) return -1;
+    if (slot_reserve(d, s, 0, bytes) || slot_reserve(d, s, 2, bytes) || (c->used[1] && slot_reserve(d, s, 1, bytes))) return -1;
+    for (int b = 3; b < (int)c->used.size(); ++b)
+        if (slot_reserve_extra(d, s, b - 3, bytes)) return -1;
+    auto B = [&](int b) -> char* { return b < 0 ? nullptr : (b < 3 ? s->dev[b] : s->xdev[b - 3]); };
     bool all[3] = {l.nplanes > 0, l.nplanes > 1, l.nplanes > 2};
     if (stage_in(s, 0, l, src, all)) return -1;  // later filters may read planes that earlier ones do not process
     const int dev_index = device_index_of(d);
-    int cur = 0, pixel_seen = 0, stats_seen = 0;
+    int stats_seen = 0;
     for (size_t i = 0; i < c->fl.size(); ++i) {
         const vszip_filter* f = c->fl[i];
-        if (f->kind == F_BOXBLUR || f->kind == F_BILATERAL || f->kind == F_LIMITER || f->kind == F_LIMITFILTER || f->kind == F_ADAPTIVEBINARIZE) {
-            // the last pixel filter must land in dev[2] (the D2H source), the ones before alternate 1 / 2;
-            // dev[0] is never written, so the source frame stays available to the diamond elements
-            const int nxt = ((c->npixel - 1 - pixel_seen) % 2 == 0) ? 2 : 1;
-            ++pixel_seen;
+        char* cur = B(c->in[i]);
+        const char* in2 = B(c->in2[i]);
+        if (is_pixel(f)) {
+            char* nxt = B(c->out[i]);
             for (int p = 0; p < l.nplanes; ++p) {  // planes this filter passes through
                 if (f->process[p]) continue;
-                VSZ_CUDA(cudaMemcpyAsync(s->dev[nxt] + l.pl[p].offset, s->dev[cur] + l.pl[p].offset, (size_t)l.pl[p].pitch * l.pl[p].h,
+                VSZ_CUDA(cudaMemcpyAsync(nxt + l.pl[p].offset, cur + l.pl[p].offset, (size_t)l.pl[p].pitch * l.pl[p].h,
                                          cudaMemcpyDeviceToDevice, s->stream));
             }
             int rc;
             if (f->kind == F_BOXBLUR) {
-                rc = run_boxblur(l, f->process, s->dev[cur], 0, s->dev[nxt], 0, 1, (int)f->hradius, f->hpasses, (int)f->vradius, f->vpasses, s->stream);
+                rc = run_boxblur(l, f->process, cur, 0, nxt, 0, 1, (int)f->hradius, f->hpasses, (int)f->vradius, f->vpasses, s->stream);
             } else if (f->kind == F_LIMITER) {
-                rc = run_limiter(l, f->process, s->dev[cur], 0, s->dev[nxt], 0, 1, f->lim_lo, f->lim_hi, s->stream);
-            } else if (f->kind == F_LIMITFILTER) {       // flt = the chain's current value, src = the chain's source frame
-                rc = run_limitfilter(l, f->process, s->dev[cur], 0, s->dev[0], 0, nullptr, 0, s->dev[nxt], 0, 1, f->lf_dark, f->lf_bright, f->lf_elast, s->stream);
-            } else if (f->kind == F_ADAPTIVEBINARIZE) {  // clip = the chain's source frame, clip2 = the chain's current value
-                rc = run_adaptivebinarize(l, s->dev[0], 0, s->dev[cur], 0, s->dev[nxt], 0, 1, f->ab_c, s->stream);
+                rc = run_limiter(l, f->process, cur, 0, nxt, 0, 1, f->lim_lo, f->lim_hi, s->stream);
+            } else if (f->kind == F_LIMITFILTER) {       // flt = the main input, src = the second, ref = the third
+                rc = run_limitfilter(l, f->process, cur, 0, in2, 0, B(c->in3[i]), 0, nxt, 0, 1, f->lf_dark, f->lf_bright, f->lf_elast, s->stream);
+            } else if (f->kind == F_ADAPTIVEBINARIZE) {  // clip = the second input, clip2 = the main input
+                rc = run_adaptivebinarize(l, in2, 0, cur, 0, nxt, 0, 1, f->ab_c, s->stream);
             } else {
                 if (bilateral_upload(f, dev_index)) return -1;
-                rc = bilateral_run(f, dev_index, s->dev[cur], 0, nullptr, 0, s->dev[nxt], 0, 1, s->stream);
+                rc = bilateral_run(f, dev_index, cur, 0, in2, 0, nxt, 0, 1, s->stream);
             }
             if (rc) return rc;
-            cur = nxt;
         } else {
-            if (!props_out || !props_out[i]) { set_error("chain: props_out[%d] is required for a PlaneMinMax/PlaneAverage element", (int)i); return -1; }
+            const bool pair = c->fuse_next[i] != 0;
+            for (size_t e = i; e <= i + (pair ? 1 : 0); ++e)
+                if (!props_out || !props_out[e]) { set_error("chain: props_out[%d] is required for a PlaneMinMax/PlaneAverage element", (int)e); return -1; }
             const int np = processed_planes(f);
             if (np == 0) { ++stats_seen; continue; }
             const size_t sb = stats_scratch_bytes(1, np);
@@ -1129,14 +1298,30 @@ int vszip_chain_get_frame(const vszip_chain* c, int32_t n, const vszip_frame* sr
             VSZ_CUDA(stats_mem.alloc(sb, s->stream));
             char* stats_scratch = stats_mem.p;
             StatsRaw* raw_dev = (StatsRaw*)s->dev_small + (size_t)stats_seen * 3;
-            int rc;
+            int rc = 1;
+            if (pair) {  // a PlaneMinMax and a PlaneAverage of the same value, planes and clipb: one read (same results as two)
+                StatsRaw* raw_next = raw_dev + 3;
+                const vszip_filter* g2 = c->fl[i + 1];
+                const vszip_filter* fm = f->kind == F_PLANEMINMAX ? f : g2;
+                const vszip_filter* fa = f->kind == F_PLANEMINMAX ? g2 : f;
+                rc = run_planestats_fused(l, fm->process, cur, 0, in2, 0, 1, fm->no_thr, fm->minthr, fm->maxthr, fm->hist_size, fa->exclude_i.data(),
+                                          fa->exclude_f.data(), (int)fa->exclude_i.size(), true, stats_scratch,
+                                          fm == f ? raw_dev : raw_next, fm == f ? raw_next : raw_dev, s->stream);
+                if (rc < 0) return rc;
+                if (rc == 0) {
+                    VSZ_CUDA(cudaMemcpyAsync((StatsRaw*)s->pin_small + (size_t)stats_seen * 3, raw_dev, sizeof(StatsRaw) * 6, cudaMemcpyDeviceToHost, s->stream));
+                    stats_seen += 2;
+                    ++i;
+                    continue;
+                }
+            }
             if (f->kind == F_PLANEMINMAX) {
-                rc = run_planeminmax(l, f->process, s->dev[cur], 0, nullptr, 0, 1, f->no_thr, f->minthr, f->maxthr, f->hist_size, stats_scratch,
+                rc = run_planeminmax(l, f->process, cur, 0, in2, 0, 1, f->no_thr, f->minthr, f->maxthr, f->hist_size, stats_scratch,
                                      raw_dev, s->stream);
             } else {
                 const int32_t* xi; const float* xf;
                 if (average_upload(f, dev_index, &xi, &xf)) return -1;
-                rc = run_planeaverage(l, f->process, s->dev[cur], 0, nullptr, 0, 1, f->exclude_i.data(), f->exclude_f.data(),
+                rc = run_planeaverage(l, f->process, cur, 0, in2, 0, 1, f->exclude_i.data(), f->exclude_f.data(),
                                       (int)f->exclude_i.size(), xi, xf, stats_scratch, raw_dev, s->stream);
             }
             if (rc) return rc;

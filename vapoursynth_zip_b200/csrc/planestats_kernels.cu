@@ -771,12 +771,13 @@ template <typename T> __device__ __forceinline__ void pack_bins(const uint4& v, 
 // TRACK = false: every bin is valid (full-depth integer or float clip) and both ranks are > 0, so the exact
 // min/max tracking drops out of the per-sample work.  With TRACK the packed min/max give the answers for zero
 // ranks and detect samples above the format's peak (such planes are left to the exact two-pass kernels).
-// AVG >= 0 (8..16-bit integer clips without clipb): the same single read also yields PlaneAverage with AVG distinct in-range exclude
-// values (SURVEY 8f rank 4) - IDP.2A sums both halves of a word, one XOR + VIMNMX.U16x2 per exclude value counts the halves that
-// differ from it (the arithmetic of average_u16_kernel); sum and excluded count travel in the Partial's idiff / excluded fields.
+// AVG >= 0: the same single read also yields PlaneAverage with AVG distinct in-range exclude values (SURVEY 8f rank 4).  8..16-bit
+// integer clips: IDP.2A sums both halves of a word, one XOR + VIMNMX.U16x2 per exclude value counts the halves that differ from it
+// (the arithmetic of average_u16_kernel); sum and excluded count travel in the Partial's idiff / excluded fields - with clipb idiff
+// carries Diff, so the sum travels in fsum instead (a whole plane's sum is below 2^47: exact in a double).  With clipb the one Diff
+// accumulated here is both filters' Diff.
 template <typename T, bool HAS_B, bool TRACK, int AVG = -1>
 __global__ void __launch_bounds__(NT) minmax_bracket_kernel(const StatsJob j) {
-    static_assert(AVG < 0 || !HAS_B, "the fused average is for clips without clipb");
     constexpr bool FAVG = AVG >= 0 && El<T>::flt;  // float clips: per sample AVG compares against the exclude values and one f64 add
     constexpr int V = El<T>::PER16, NW = V / 2, G = HAS_B ? 2 : 4;
     constexpr int NEX = AVG > 0 ? AVG : 1;
@@ -991,7 +992,8 @@ __global__ void __launch_bounds__(NT) minmax_bracket_kernel(const StatsJob j) {
             excluded += cnt;
             removed += (unsigned long long)cnt * (unsigned)j.excl_i[e];
         }
-        acc.idiff = sum64 - removed;  // (no clipb here: the diff field is free)
+        if constexpr (HAS_B) acc.fsum = (double)(sum64 - removed);
+        else acc.idiff = sum64 - removed;
         acc.excluded = excluded;
     }
     drain();
@@ -1017,7 +1019,10 @@ __global__ void __launch_bounds__(NT) minmax_bracket_kernel(const StatsJob j) {
         StatsRaw& r = j.out[fp];
         if constexpr (AVG >= 0) {
             StatsRaw ra{};
-            ra.isum = total.idiff; ra.fsum = total.fsum; ra.excluded = total.excluded;
+            if constexpr (HAS_B && !FAVG) ra.isum = (unsigned long long)total.fsum;
+            else { ra.isum = total.idiff; ra.fsum = total.fsum; }
+            ra.excluded = total.excluded;
+            if constexpr (HAS_B) { ra.idiff = r.idiff = total.idiff; ra.fdiff = r.fdiff = total.fdiff; }
             j.out_avg[fp] = ra;
         } else {
             r.idiff = total.idiff; r.fdiff = total.fdiff;
@@ -1222,14 +1227,14 @@ int run_planeminmax(const FrameLayout& l, const bool mask[3], const char* a, siz
 
 // PlaneMinMax + PlaneAverage of the same planes from ONE read (SURVEY 8f rank 4).  run_planestats_fused returns 1 when the
 // combination is not eligible (the caller then runs the two reductions separately), 0 on success, < 0 on error.
-template <typename T>
+template <typename T, bool HAS_B>
 static int launch_fused_t(const StatsJob& j, int count, int m, cudaStream_t st) {
     bool lean = (j.hist_size == 65536u) || (sizeof(T) == 1 && j.hist_size == 256u);
     for (int k = 0; k < j.nplanes; ++k) lean = lean && j.pl[k].tmin > 0u && j.pl[k].tmax > 0u;
     hist_sample_kernel<T><<<dim3(j.sample_ctas_per_frame, count), NT, 0, st>>>(j);
     const dim3 bgrid(j.bracket_ctas_per_frame, count);
-#define VSZ_FUSED(M) (lean ? (void)(minmax_bracket_kernel<T, false, false, M><<<bgrid, NT, 0, st>>>(j)) \
-                           : (void)(minmax_bracket_kernel<T, false, true, M><<<bgrid, NT, 0, st>>>(j)))
+#define VSZ_FUSED(M) (lean ? (void)(minmax_bracket_kernel<T, HAS_B, false, M><<<bgrid, NT, 0, st>>>(j)) \
+                           : (void)(minmax_bracket_kernel<T, HAS_B, true, M><<<bgrid, NT, 0, st>>>(j)))
     switch (m) {
         case 0: VSZ_FUSED(0); break;
         case 1: VSZ_FUSED(1); break;
@@ -1247,36 +1252,49 @@ static int launch_fused_t(const StatsJob& j, int count, int m, cudaStream_t st) 
     return 0;
 }
 
-template <typename T>
+template <typename T, bool HAS_B>
 static int launch_both_nothr_t(const StatsJob& j, int count, cudaStream_t st) {
     const dim3 grid(j.ctas_per_frame, count);
-    if (j.nex > 4) stats_kernel<T, false, true, true, true><<<grid, NT, 0, st>>>(j);
-    else stats_kernel<T, false, true, false, true><<<grid, NT, 0, st>>>(j);
+    if (j.nex > 4) stats_kernel<T, HAS_B, true, true, true><<<grid, NT, 0, st>>>(j);
+    else stats_kernel<T, HAS_B, true, false, true><<<grid, NT, 0, st>>>(j);
     count_launch();
     VSZ_CUDA(cudaGetLastError());
     return 0;
 }
 
-// Eligible: no clipb, at most 32768 frames; without thresholds any sample type and up to 16 exclude values; with thresholds
-// (sampled fast path enabled) at most 4 distinct exclude values that can match a sample.
-int run_planestats_fused(const FrameLayout& l, const bool mask[3], const char* a, size_t a_fs, int count, bool no_thr, float minthr,
-                         float maxthr, uint32_t hist_size, const int32_t* excl, const float* excl_f, int nex, void* scratch, StatsRaw* out_mm,
-                         StatsRaw* out_avg, cudaStream_t st) {
+template <typename T>
+static int launch_both_nothr(const StatsJob& j, int count, cudaStream_t st) {
+    return j.b ? launch_both_nothr_t<T, true>(j, count, st) : launch_both_nothr_t<T, false>(j, count, st);
+}
+template <typename T>
+static int launch_fused(const StatsJob& j, int count, int m, cudaStream_t st) {
+    return j.b ? launch_fused_t<T, true>(j, count, m, st) : launch_fused_t<T, false>(j, count, m, st);
+}
+
+// Eligible: at most 32768 frames; without thresholds any sample type and up to 16 exclude values; with thresholds (sampled fast
+// path enabled) at most 4 distinct exclude values that can match a sample.  b (clipb, may be nullptr): both filters read it; Diff
+// is accumulated once, in the order of the separate kernels.  same_float_sums: fuse a float clip with thresholds only when its float
+// sums come out bit-identical to the separate calls - the bracket kernel walks a plane whose rows are back to back (no row padding)
+// as one run of vectors, which the separate PlaneAverage kernel does not, so such planes are not fused.  Always on with clipb, so
+// that a float Diff is the same whichever route ran.
+int run_planestats_fused(const FrameLayout& l, const bool mask[3], const char* a, size_t a_fs, const char* b, size_t b_fs, int count,
+                         bool no_thr, float minthr, float maxthr, uint32_t hist_size, const int32_t* excl, const float* excl_f, int nex,
+                         bool same_float_sums, void* scratch, StatsRaw* out_mm, StatsRaw* out_avg, cudaStream_t st) {
     if (count <= 0 || count > 32768) return 1;
     if (no_thr) {
         if (nex > 16) return 1;
         size_t zero = 0;
-        StatsJob j = make_job(l, mask, a, a_fs, nullptr, 0, count, scratch, out_mm, &zero);
+        StatsJob j = make_job(l, mask, a, a_fs, b, b_fs, count, scratch, out_mm, &zero);
         if (j.ctas_per_frame == 0) return 1;
         VSZ_CUDA(cudaMemsetAsync(scratch, 0, zero, st));
         j.out_avg = out_avg;
         j.nex = nex;
         for (int i = 0; i < nex; ++i) { j.excl_i[i] = excl[i]; j.excl_f[i] = excl_f[i]; }
         switch (l.kind) {
-            case K_U8: return launch_both_nothr_t<uint8_t>(j, count, st);
-            case K_U16: return launch_both_nothr_t<uint16_t>(j, count, st);
-            case K_F16: return launch_both_nothr_t<__half>(j, count, st);
-            case K_F32: return launch_both_nothr_t<float>(j, count, st);
+            case K_U8: return launch_both_nothr<uint8_t>(j, count, st);
+            case K_U16: return launch_both_nothr<uint16_t>(j, count, st);
+            case K_F16: return launch_both_nothr<__half>(j, count, st);
+            case K_F32: return launch_both_nothr<float>(j, count, st);
         }
         return -1;
     }
@@ -1298,10 +1316,13 @@ int run_planestats_fused(const FrameLayout& l, const bool mask[3], const char* a
         ++m;
     }
     size_t zero = 0;
-    StatsJob j = make_job(l, mask, a, a_fs, nullptr, 0, count, scratch, out_mm, &zero);
+    StatsJob j = make_job(l, mask, a, a_fs, b, b_fs, count, scratch, out_mm, &zero);
     if (j.ctas_per_frame == 0) return 1;
-    for (int k = 0; k < j.nplanes; ++k)
+    for (int k = 0; k < j.nplanes; ++k) {
         if ((long long)j.pl[k].w * j.pl[k].h >= (1ll << 31)) return 1;
+        const int nvec = j.pl[k].w / (16 / l.bps);  // minmax_bracket_kernel's `contiguous` test
+        if (flt && (same_float_sums || b) && nvec > 0 && j.pl[k].a_pitch == nvec * 16) return 1;
+    }
     VSZ_CUDA(cudaMemsetAsync(scratch, 0, zero, st));
     VSZ_CUDA(cudaMemsetAsync(out_mm, 0, sizeof(StatsRaw) * (size_t)count * j.nplanes, st));
     j.out_avg = out_avg;
@@ -1318,10 +1339,10 @@ int run_planestats_fused(const FrameLayout& l, const bool mask[3], const char* a
     j.nex = m;
     for (int i = 0; i < m; ++i) { j.excl_i[i] = ex[i]; j.excl_f[i] = exf[i]; }
     switch (l.kind) {
-        case K_U8: return launch_fused_t<uint8_t>(j, count, m, st);
-        case K_U16: return launch_fused_t<uint16_t>(j, count, m, st);
-        case K_F16: return launch_fused_t<__half>(j, count, m, st);
-        case K_F32: return launch_fused_t<float>(j, count, m, st);
+        case K_U8: return launch_fused<uint8_t>(j, count, m, st);
+        case K_U16: return launch_fused<uint16_t>(j, count, m, st);
+        case K_F16: return launch_fused<__half>(j, count, m, st);
+        case K_F32: return launch_fused<float>(j, count, m, st);
     }
     return -1;
 }

@@ -16,6 +16,7 @@ namespace vsz {
 
 static thread_local std::string t_error;
 std::atomic<uint64_t> g_launches{0};
+std::atomic<uint64_t> g_transfer[2] = {{0}, {0}};
 
 void set_error(const char* fmt, ...) {
     char buf[1024];
@@ -112,6 +113,19 @@ int slot_reserve(DeviceCtx* d, Slot* s, int which, size_t bytes) {
     VSZ_CUDA(cudaHostAlloc((void**)&s->pin[which], bytes, cudaHostAllocDefault));
     VSZ_CUDA(cudaMalloc((void**)&s->dev[which], bytes));
     s->cap[which] = bytes;
+    return 0;
+}
+
+int slot_reserve_extra(DeviceCtx* d, Slot* s, int which, size_t bytes) {
+    if ((int)s->xdev.size() <= which) { s->xdev.resize(which + 1, nullptr); s->xcap.resize(which + 1, 0); }
+    if (s->xcap[which] >= bytes) return 0;
+    VSZ_CUDA(cudaSetDevice(d->ordinal));
+    VSZ_CUDA(cudaStreamSynchronize(s->stream));
+    if (s->xdev[which]) cudaFree(s->xdev[which]);
+    s->xdev[which] = nullptr;
+    s->xcap[which] = 0;
+    VSZ_CUDA(cudaMalloc((void**)&s->xdev[which], bytes));
+    s->xcap[which] = bytes;
     return 0;
 }
 
@@ -267,7 +281,10 @@ static int pinned_copy(Slot* s, int dev_buf, const FrameLayout& l, const vszip_f
 
 int stage_in(Slot* s, int which, const FrameLayout& l, const vszip_frame* host, const bool mask[3]) {
     bool pinned[3] = {false, false, false};
-    for (int p = 0; p < l.nplanes; ++p) pinned[p] = mask[p] && is_pinned_host(l, p, host);
+    for (int p = 0; p < l.nplanes; ++p) {
+        pinned[p] = mask[p] && is_pinned_host(l, p, host);
+        if (mask[p]) count_transfer(0, (size_t)l.pl[p].w * l.pl[p].h * l.bps);
+    }
     for (int p = 0; p < l.nplanes;) {
         if (!mask[p]) { ++p; continue; }
         const PlaneGeom& g = l.pl[p];
@@ -290,7 +307,10 @@ int stage_in(Slot* s, int which, const FrameLayout& l, const vszip_frame* host, 
 // pinned buffer (stage_out_finish then copies it out after the stream has been synchronised).
 int stage_out_begin(Slot* s, const FrameLayout& l, vszip_frame* host, const bool mask[3], bool direct[3]) {
     bool pinned[3] = {false, false, false};
-    for (int p = 0; p < l.nplanes; ++p) { pinned[p] = mask[p] && is_pinned_host(l, p, host); direct[p] = pinned[p]; }
+    for (int p = 0; p < l.nplanes; ++p) {
+        pinned[p] = mask[p] && is_pinned_host(l, p, host); direct[p] = pinned[p];
+        if (mask[p]) count_transfer(1, (size_t)l.pl[p].w * l.pl[p].h * l.bps);
+    }
     for (int p = 0; p < l.nplanes;) {
         if (!mask[p]) { ++p; continue; }
         const PlaneGeom& g = l.pl[p];
@@ -355,6 +375,7 @@ extern "C" {
 int vszip_cuda_abi_version(void) { return VSZIP_CUDA_ABI_VERSION; }
 const char* vszip_cuda_last_error(void) { return t_error.c_str(); }
 uint64_t vszip_cuda_kernel_launches(void) { return g_launches.load(); }
+uint64_t vszip_cuda_transfer_bytes(int32_t direction) { return (direction == 0 || direction == 1) ? g_transfer[direction].load() : 0; }
 int vszip_cuda_device_count(void) { return num_devices(); }
 
 int vszip_cuda_init(const int32_t* device_ids, int32_t n) {
@@ -412,6 +433,7 @@ void vszip_cuda_shutdown(void) {
         cudaDeviceSynchronize();
         for (Slot* s : d->all) {
             for (int i = 0; i < 4; ++i) { if (s->pin[i]) cudaFreeHost(s->pin[i]); if (s->dev[i]) cudaFree(s->dev[i]); }
+            for (char* x : s->xdev) if (x) cudaFree(x);
             if (s->pin_small) cudaFreeHost(s->pin_small);
             if (s->dev_small) cudaFree(s->dev_small);
             cudaStreamDestroy(s->stream);
@@ -534,6 +556,7 @@ int vszip_dev_clip_upload(vszip_dev_clip* c, int32_t frame, const vszip_frame* h
         const PlaneGeom& g = c->layout.pl[p];
         VSZ_CUDA(cudaMemcpy2D(c->base + (size_t)frame * c->layout.frame_stride + g.offset, g.pitch, host->data[p],
                               host->stride[p], (size_t)g.w * c->layout.bps, g.h, cudaMemcpyHostToDevice));
+        count_transfer(0, (size_t)g.w * g.h * c->layout.bps);
     }
     return 0;
 }
@@ -546,6 +569,7 @@ int vszip_dev_clip_download(const vszip_dev_clip* c, int32_t frame, vszip_frame*
         const PlaneGeom& g = c->layout.pl[p];
         VSZ_CUDA(cudaMemcpy2D(host->data[p], host->stride[p], c->base + (size_t)frame * c->layout.frame_stride + g.offset,
                               g.pitch, (size_t)g.w * c->layout.bps, g.h, cudaMemcpyDeviceToHost));
+        count_transfer(1, (size_t)g.w * g.h * c->layout.bps);
     }
     return 0;
 }
