@@ -1,4 +1,4 @@
-// filter.h — the immutable per-instance data of the four filters (the CUDA-side twin of the
+// filter.h — the immutable per-instance data of the seven filters (the CUDA-side twin of the
 // reference's `Data` structs) and the kernel launchers each filter uses.
 #pragma once
 
@@ -24,7 +24,7 @@ struct vszip_filter {
     vsz::SampleKind sample;
     vsz::FrameLayout layout;
     bool process[3];
-    bool has_ref;  // Bilateral ref / PlaneMinMax+PlaneAverage clipb
+    bool has_input[2];  // created with its second / third input (filters.cu's kind table names them)
 
     // BoxBlur (src/vapoursynth/boxblur.zig:16-25)
     uint32_t hradius, vradius;
@@ -56,7 +56,6 @@ struct vszip_filter {
 
     // LimitFilter (src/vapoursynth/limit_filter.zig:15-25): thresholds already scaled to the clip's depth
     float lf_dark[3], lf_bright[3], lf_elast[3];
-    bool lf_has_ref;
     // AdaptiveBinarize (src/vapoursynth/adaptive_binarize.zig:14-19)
     int ab_c;
 };

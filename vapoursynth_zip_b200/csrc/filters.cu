@@ -1,7 +1,7 @@
-// filters.cu — host side of the four filters: argument parsing/validation with the reference's
-// defaults and error strings (the twin of src/vapoursynth/{boxblur,bilateral,planeminmax,planeaverage}.zig
-// create callbacks), the synchronous getFrame-style entry points (host buffers, staged through the
-// per-request slot) and the batched device-resident entry points.
+// filters.cu — host side of the seven filters: argument parsing/validation with the reference's
+// defaults and error strings (the twin of the create callbacks in src/vapoursynth/{boxblur,bilateral,planeminmax,
+// planeaverage,limiter,limit_filter,adaptive_binarize}.zig), the synchronous getFrame-style entry points (host
+// buffers, staged through the per-request slot), the batched device-resident entry points and the fused chains.
 #include <cmath>
 #include <cstdio>
 #include <cstring>
@@ -153,6 +153,68 @@ bool range_ok(const vszip_dev_clip* c, int first, int count, const char* name) {
     return true;
 }
 
+// The checks of a batched call: every clip it reads or writes matches the instance's format (a NULL clip does not) and holds
+// frames [first, first + count), and all of them live on one initialised device, which becomes current.  *st: the caller's
+// stream, or that device's batch stream.
+int begin_device_call(const vszip_filter* f, const char* name, const vszip_dev_clip* const* clips, int n, int32_t first, int32_t count,
+                      void* stream, cudaStream_t* st) {
+    for (int i = 0; i < n; ++i) if (!same_clip_shape(clips[i], f, name)) return -1;
+    for (int i = 0; i < n; ++i) if (!range_ok(clips[i], first, count, name)) return -1;
+    for (int i = 1; i < n; ++i)
+        if (clips[i]->device_index != clips[0]->device_index) { set_error("%s: clips live on different devices", name); return -1; }
+    DeviceCtx* d = device_ctx(clips[0]->device_index);
+    if (!d) { set_error("%s: library not initialised", name); return -1; }
+    VSZ_CUDA(cudaSetDevice(d->ordinal));
+    *st = stream ? (cudaStream_t)stream : d->batch_stream;
+    return 0;
+}
+
+int device_index_of(DeviceCtx* d) {
+    for (int i = 0; i < num_devices(); ++i) if (device_ctx(i) == d) return i;
+    return 0;
+}
+
+int processed_planes(const vszip_filter* f) {
+    int k = 0;
+    for (int p = 0; p < f->layout.nplanes; ++p) k += f->process[p] ? 1 : 0;
+    return k;
+}
+
+// What each filter kind takes and gives, indexed by FilterKind - 1.
+struct KindInfo {
+    const char* name;
+    bool pixel;            // has a pixel output (else it measures frame statistics)
+    const char* input[2];  // the filter's names for its second and third inputs (nullptr: none)
+    bool optional[2];      // an instance may be created without that input
+};
+constexpr KindInfo kKinds[] = {
+    {"BoxBlur", true, {nullptr, nullptr}, {false, false}},
+    {"Bilateral", true, {"ref", nullptr}, {true, false}},
+    {"PlaneMinMax", false, {"clipb", nullptr}, {true, false}},
+    {"PlaneAverage", false, {"clipb", nullptr}, {true, false}},
+    {"Limiter", true, {nullptr, nullptr}, {false, false}},
+    {"LimitFilter", true, {"src", "ref"}, {false, true}},
+    {"AdaptiveBinarize", true, {"clip", nullptr}, {false, false}},
+};
+static_assert(sizeof kKinds / sizeof kKinds[0] == F_ADAPTIVEBINARIZE, "one row per FilterKind");
+
+const KindInfo& kind_info(int kind) { return kKinds[kind - 1]; }
+bool is_pixel(const vszip_filter* f) { return kind_info(f->kind).pixel; }
+
+// An optional input must be passed exactly when the instance was created with it.  get_frame says "ref frame" / "clipb frame",
+// _device "ref clip" / "clipb".
+bool inputs_match(const vszip_filter* f, const void* second, const void* third, bool device) {
+    const KindInfo& k = kind_info(f->kind);
+    const bool given[2] = {second != nullptr, third != nullptr};
+    for (int i = 0; i < 2; ++i) {
+        if (!k.optional[i] || f->has_input[i] == given[i]) continue;
+        const char* noun = !device ? " frame" : (strcmp(k.input[i], "clipb") ? " clip" : "");
+        set_error("%s: %s%s presence does not match the filter instance", k.name, k.input[i], noun);
+        return false;
+    }
+    return true;
+}
+
 }  // namespace
 
 extern "C" {
@@ -177,6 +239,118 @@ void vszip_filter_free(vszip_filter* f) {
 int vszip_filter_planes(const vszip_filter* f, int32_t process[3]) {
     for (int i = 0; i < 3; ++i) process[i] = (i < f->vi.num_planes && f->process[i]) ? 1 : 0;
     return 0;
+}
+
+// =========================================================================== shared entry-point bodies
+// The dispatchers, defined after the filters' own sections.  `in` holds a pixel filter's main input, then its second and third
+// (the chain's numbering, whatever order the filter's own entry points take them in); consecutive frames are fs bytes apart.
+static int run_pixels(const vszip_filter* f, int dev_index, const char* const in[3], char* out, size_t fs, int count, cudaStream_t st);
+static int run_stats(const vszip_filter* f, int dev_index, const char* a, const char* b, size_t fs, int count, void* scratch,
+                     StatsRaw* raw, cudaStream_t st);
+static void stats_finalize(const vszip_filter* f, const StatsRaw* raw, void* props, int i);  // into element i of a props array
+
+using Frames = std::array<const vszip_frame*, 3>;
+using DevClips = std::array<const vszip_dev_clip*, 3>;
+
+// getFrame of a pixel filter: the inputs staged into slot buffers 0, 1 and 3, the output computed into dev[2] and brought back.
+static int pixel_get_frame(const vszip_filter* f, int kind, int32_t n, const Frames& in, vszip_frame* dst) {
+    const char* name = kind_info(kind).name;
+    if (!f || f->kind != kind) { set_error("%s: bad filter handle", name); return -1; }
+    if (!inputs_match(f, in[1], in[2], false)) return -1;
+    DeviceCtx* d = route(n, name);
+    if (!d) return -1;
+    SlotGuard g(d);
+    Slot* s = g.s;
+    VSZ_CUDA(cudaSetDevice(d->ordinal));
+    static const int buf[3] = {0, 1, 3};  // the slot buffer of each input
+    const size_t bytes = f->layout.frame_stride;
+    if (slot_reserve(d, s, 2, bytes)) return -1;
+    for (int k = 0; k < 3; ++k)  // the main input always, the others when given
+        if ((k == 0 || in[k]) && slot_reserve(d, s, buf[k], bytes)) return -1;
+    const char* dev_in[3] = {nullptr, nullptr, nullptr};
+    for (int k = 0; k < 3; ++k) {
+        if (k > 0 && !in[k]) continue;
+        if (stage_in(s, buf[k], f->layout, in[k], f->process)) return -1;
+        dev_in[k] = s->dev[buf[k]];
+    }
+    const int rc = run_pixels(f, device_index_of(d), dev_in, s->dev[2], 0, 1, s->stream);
+    if (rc) return rc;
+    bool direct[3];
+    if (stage_out_begin(s, f->layout, dst, f->process, direct)) return -1;
+    VSZ_CUDA(cudaStreamSynchronize(s->stream));
+    stage_out_finish(s, f->layout, dst, f->process, direct);
+    return 0;
+}
+
+// getFrame of PlaneMinMax / PlaneAverage: a (and clipb b) staged into slot buffers 0 (and 1), the sums back through the slot's
+// small buffers.
+static int stats_get_frame(const vszip_filter* f, int kind, int32_t n, const vszip_frame* a, const vszip_frame* b, void* out) {
+    const char* name = kind_info(kind).name;
+    if (!f || f->kind != kind) { set_error("%s: bad filter handle", name); return -1; }
+    if (!inputs_match(f, b, nullptr, false)) return -1;
+    DeviceCtx* d = route(n, name);
+    if (!d) return -1;
+    SlotGuard g(d);
+    Slot* s = g.s;
+    VSZ_CUDA(cudaSetDevice(d->ordinal));
+    const size_t bytes = f->layout.frame_stride;
+    const int np = processed_planes(f);
+    const size_t scratch = stats_scratch_bytes(1, np) + 256;
+    if (slot_reserve(d, s, 0, bytes) || (b && slot_reserve(d, s, 1, bytes)) || slot_reserve(d, s, 2, scratch)) return -1;
+    if (stage_in(s, 0, f->layout, a, f->process)) return -1;
+    if (b && stage_in(s, 1, f->layout, b, f->process)) return -1;
+    StatsRaw* raw_dev = (StatsRaw*)s->dev_small;
+    const int rc = run_stats(f, device_index_of(d), s->dev[0], b ? s->dev[1] : nullptr, 0, 1, s->dev[2], raw_dev, s->stream);
+    if (rc) return rc;
+    VSZ_CUDA(cudaMemcpyAsync(s->pin_small, raw_dev, sizeof(StatsRaw) * np, cudaMemcpyDeviceToHost, s->stream));
+    VSZ_CUDA(cudaStreamSynchronize(s->stream));
+    stats_finalize(f, (const StatsRaw*)s->pin_small, out, 0);
+    return 0;
+}
+
+// The batched entry points' checks, in one order: the handle, the optional inputs, then every clip the call reads or writes (a
+// required input that is NULL fails as a clip of the wrong format).  dst: the pixel output, unused for statistics.
+static int device_call(const vszip_filter* f, int kind, const DevClips& in, const vszip_dev_clip* dst, int32_t first, int32_t count,
+                       void* stream, cudaStream_t* st) {
+    const KindInfo& k = kind_info(kind);
+    if (!f || f->kind != kind) { set_error("%s: bad filter handle", k.name); return -1; }
+    if (!inputs_match(f, in[1], in[2], true)) return -1;
+    const vszip_dev_clip* clips[4] = {in[0]};
+    int n = 1;
+    for (int i = 0; i < 2; ++i) if (f->has_input[i]) clips[n++] = in[i + 1];
+    if (k.pixel) clips[n++] = dst;
+    return begin_device_call(f, k.name, clips, n, first, count, stream, st);
+}
+
+static int pixel_device(const vszip_filter* f, int kind, const DevClips& in, vszip_dev_clip* dst, int32_t first, int32_t count, void* stream) {
+    cudaStream_t st;
+    if (device_call(f, kind, in, dst, first, count, stream, &st)) return -1;
+    const size_t fs = dst->layout.frame_stride, off = (size_t)first * fs;
+    const char* p[3];
+    for (int k = 0; k < 3; ++k) p[k] = in[k] ? in[k]->base + off : nullptr;
+    return run_pixels(f, dst->device_index, p, dst->base + off, fs, count, st);
+}
+
+static int stats_device(const vszip_filter* f, int kind, const vszip_dev_clip* a, const vszip_dev_clip* b, int32_t first, int32_t count,
+                        void* out, void* stream) {
+    cudaStream_t st;
+    if (device_call(f, kind, {a, b, nullptr}, nullptr, first, count, stream, &st)) return -1;
+    const int np = processed_planes(f);
+    if (count == 0 || np == 0) return 0;
+    const size_t fs = a->layout.frame_stride;
+    AsyncScratch scratch_mem;
+    const size_t sb = stats_scratch_bytes(count, np), rb = sizeof(StatsRaw) * (size_t)count * np;
+    VSZ_CUDA(scratch_mem.alloc(sb + rb, st));
+    StatsRaw* raw_dev = (StatsRaw*)(scratch_mem.p + sb);
+    const int rc = run_stats(f, a->device_index, a->base + (size_t)first * fs, b ? b->base + (size_t)first * fs : nullptr, fs, count,
+                             scratch_mem.p, raw_dev, st);
+    if (!rc && out) {
+        std::vector<StatsRaw> raw((size_t)count * np);
+        VSZ_CUDA(cudaMemcpyAsync(raw.data(), raw_dev, rb, cudaMemcpyDeviceToHost, st));
+        VSZ_CUDA(cudaStreamSynchronize(st));
+        for (int i = 0; i < count; ++i) stats_finalize(f, raw.data() + (size_t)i * np, out, i);
+    }
+    return rc;
 }
 
 // =========================================================================== BoxBlur
@@ -209,42 +383,16 @@ vszip_filter* vszip_boxblur_create(const vszip_video_info* vi, const vszip_boxbl
     f->sample = kind;
     f->layout = make_layout(*vi, kind);
     for (int i = 0; i < 3; ++i) f->process[i] = process[i] && i < vi->num_planes;
-    f->has_ref = false;
     f->hradius = hr; f->vradius = vr; f->hpasses = hp; f->vpasses = vp;
     return f;
 }
 
 int vszip_boxblur_get_frame(const vszip_filter* f, int32_t n, const vszip_frame* src, vszip_frame* dst) {
-    if (!f || f->kind != F_BOXBLUR) { set_error("BoxBlur: bad filter handle"); return -1; }
-    DeviceCtx* d = route(n, "BoxBlur");
-    if (!d) return -1;
-    SlotGuard g(d);
-    Slot* s = g.s;
-    VSZ_CUDA(cudaSetDevice(d->ordinal));
-    const size_t bytes = f->layout.frame_stride;
-    if (slot_reserve(d, s, 0, bytes) || slot_reserve(d, s, 2, bytes)) return -1;
-    if (stage_in(s, 0, f->layout, src, f->process)) return -1;
-    int rc = run_boxblur(f->layout, f->process, s->dev[0], 0, s->dev[2], 0, 1, (int)f->hradius, f->hpasses, (int)f->vradius, f->vpasses, s->stream);
-    if (rc) return rc;
-    bool direct[3];
-    if (stage_out_begin(s, f->layout, dst, f->process, direct)) return -1;
-    VSZ_CUDA(cudaStreamSynchronize(s->stream));
-    stage_out_finish(s, f->layout, dst, f->process, direct);
-    return 0;
+    return pixel_get_frame(f, F_BOXBLUR, n, {src, nullptr, nullptr}, dst);
 }
 
 int vszip_boxblur_device(const vszip_filter* f, const vszip_dev_clip* src, vszip_dev_clip* dst, int32_t first, int32_t count, void* stream) {
-    static const char* name = "BoxBlur";
-    if (!f || f->kind != F_BOXBLUR) { set_error("BoxBlur: bad filter handle"); return -1; }
-    if (!same_clip_shape(src, f, name) || !same_clip_shape(dst, f, name) || !range_ok(src, first, count, name) || !range_ok(dst, first, count, name)) return -1;
-    if (src->device_index != dst->device_index) { set_error("BoxBlur: clips live on different devices"); return -1; }
-    DeviceCtx* d = device_ctx(src->device_index);
-    if (!d) { set_error("BoxBlur: library not initialised"); return -1; }
-    VSZ_CUDA(cudaSetDevice(d->ordinal));
-    cudaStream_t st = stream ? (cudaStream_t)stream : d->batch_stream;
-    const size_t fs = src->layout.frame_stride;
-    return run_boxblur(f->layout, f->process, src->base + (size_t)first * fs, fs, dst->base + (size_t)first * fs, fs, count,
-                       (int)f->hradius, f->hpasses, (int)f->vradius, f->vpasses, st);
+    return pixel_device(f, F_BOXBLUR, {src, nullptr, nullptr}, dst, first, count, stream);
 }
 
 // =========================================================================== Bilateral
@@ -323,7 +471,7 @@ vszip_filter* vszip_bilateral_create(const vszip_video_info* vi, const vszip_vid
     }
     if (ref_vi && !compare_nodes(*vi, *ref_vi, name)) return fail();
     for (int i = 0; i < 3; ++i) f->process[i] = process[i] && i < vi->num_planes;
-    f->has_ref = ref_vi != nullptr;
+    f->has_input[0] = ref_vi != nullptr;
     // LUTs (src/filters/bilateral.zig:306-334), f64 math rounded to f32, uploaded to every device
     f->gs_host.resize(3); f->gr_host.resize(3);
     for (int i = 0; i < vi->num_planes; ++i) {
@@ -427,49 +575,13 @@ static int bilateral_run(const vszip_filter* f, int dev_index, const char* src, 
     return 0;
 }
 
-static int device_index_of(DeviceCtx* d) {
-    for (int i = 0; i < num_devices(); ++i) if (device_ctx(i) == d) return i;
-    return 0;
-}
-
 int vszip_bilateral_get_frame(const vszip_filter* f, int32_t n, const vszip_frame* src, const vszip_frame* ref, vszip_frame* dst) {
-    if (!f || f->kind != F_BILATERAL) { set_error("Bilateral: bad filter handle"); return -1; }
-    if (f->has_ref != (ref != nullptr)) { set_error("Bilateral: ref frame presence does not match the filter instance"); return -1; }
-    DeviceCtx* d = route(n, "Bilateral");
-    if (!d) return -1;
-    SlotGuard g(d);
-    Slot* s = g.s;
-    VSZ_CUDA(cudaSetDevice(d->ordinal));
-    const size_t bytes = f->layout.frame_stride;
-    if (slot_reserve(d, s, 0, bytes) || slot_reserve(d, s, 2, bytes) || (ref && slot_reserve(d, s, 1, bytes))) return -1;
-    if (stage_in(s, 0, f->layout, src, f->process)) return -1;
-    if (ref && stage_in(s, 1, f->layout, ref, f->process)) return -1;
-    if (bilateral_upload(f, device_index_of(d))) return -1;
-    int rc = bilateral_run(f, device_index_of(d), s->dev[0], 0, ref ? s->dev[1] : nullptr, 0, s->dev[2], 0, 1, s->stream);
-    if (rc) return rc;
-    bool direct[3];
-    if (stage_out_begin(s, f->layout, dst, f->process, direct)) return -1;
-    VSZ_CUDA(cudaStreamSynchronize(s->stream));
-    stage_out_finish(s, f->layout, dst, f->process, direct);
-    return 0;
+    return pixel_get_frame(f, F_BILATERAL, n, {src, ref, nullptr}, dst);
 }
 
 int vszip_bilateral_device(const vszip_filter* f, const vszip_dev_clip* src, const vszip_dev_clip* ref, vszip_dev_clip* dst,
                            int32_t first, int32_t count, void* stream) {
-    static const char* name = "Bilateral";
-    if (!f || f->kind != F_BILATERAL) { set_error("Bilateral: bad filter handle"); return -1; }
-    if (f->has_ref != (ref != nullptr)) { set_error("Bilateral: ref clip presence does not match the filter instance"); return -1; }
-    if (!same_clip_shape(src, f, name) || !same_clip_shape(dst, f, name) || (ref && !same_clip_shape(ref, f, name))) return -1;
-    if (!range_ok(src, first, count, name) || !range_ok(dst, first, count, name) || (ref && !range_ok(ref, first, count, name))) return -1;
-    if (src->device_index != dst->device_index || (ref && ref->device_index != src->device_index)) { set_error("Bilateral: clips live on different devices"); return -1; }
-    DeviceCtx* d = device_ctx(src->device_index);
-    if (!d) { set_error("Bilateral: library not initialised"); return -1; }
-    VSZ_CUDA(cudaSetDevice(d->ordinal));
-    cudaStream_t st = stream ? (cudaStream_t)stream : d->batch_stream;
-    const size_t fs = src->layout.frame_stride;
-    if (bilateral_upload(f, src->device_index)) return -1;
-    return bilateral_run(f, src->device_index, src->base + (size_t)first * fs, fs, ref ? ref->base + (size_t)first * fs : nullptr, fs,
-                         dst->base + (size_t)first * fs, fs, count, st);
+    return pixel_device(f, F_BILATERAL, {src, ref, nullptr}, dst, first, count, stream);
 }
 
 // =========================================================================== PlaneMinMax
@@ -499,7 +611,7 @@ vszip_filter* vszip_planeminmax_create(const vszip_video_info* vi, const vszip_v
     f->sample = kind;
     f->layout = make_layout(*vi, kind);
     for (int i = 0; i < 3; ++i) f->process[i] = process[i] && i < vi->num_planes;
-    f->has_ref = clipb_vi != nullptr;
+    f->has_input[0] = clipb_vi != nullptr;
     f->minthr = minthr; f->maxthr = maxthr; f->hist_size = hist_size; f->no_thr = no_thr;
     return f;
 }
@@ -507,7 +619,7 @@ vszip_filter* vszip_planeminmax_create(const vszip_video_info* vi, const vszip_v
 static void minmax_finalize(const vszip_filter* f, const StatsRaw* raw, vszip_minmax_props* out) {
     const bool flt = f->sample == K_F16 || f->sample == K_F32;
     memset(out, 0, sizeof *out);
-    out->is_float = flt; out->has_diff = f->has_ref;
+    out->is_float = flt; out->has_diff = f->has_input[0];
     const float peakf = (float)(f->hist_size - 1);  // planeminmax.zig:118-119
     int k = 0;
     for (int p = 0; p < f->layout.nplanes; ++p) {
@@ -522,7 +634,7 @@ static void minmax_finalize(const vszip_filter* f, const StatsRaw* raw, vszip_mi
             out->fmin[k] = (double)((float)r.bin_min / 65535.0f);  // src/filters/planeminmax.zig:62-63
             out->fmax[k] = (double)((float)r.bin_max / 65535.0f);
         }
-        if (f->has_ref) {
+        if (f->has_input[0]) {
             const double total = (double)((uint32_t)f->layout.pl[p].w * (uint32_t)f->layout.pl[p].h);
             out->diff[k] = flt ? r.fdiff / total : (double)r.idiff / total / (double)peakf;
         }
@@ -531,64 +643,13 @@ static void minmax_finalize(const vszip_filter* f, const StatsRaw* raw, vszip_mi
     out->count = k;
 }
 
-static int processed_planes(const vszip_filter* f) {
-    int k = 0;
-    for (int p = 0; p < f->layout.nplanes; ++p) k += f->process[p] ? 1 : 0;
-    return k;
-}
-
 int vszip_planeminmax_get_frame(const vszip_filter* f, int32_t n, const vszip_frame* a, const vszip_frame* b, vszip_minmax_props* out) {
-    if (!f || f->kind != F_PLANEMINMAX) { set_error("PlaneMinMax: bad filter handle"); return -1; }
-    if (f->has_ref != (b != nullptr)) { set_error("PlaneMinMax: clipb frame presence does not match the filter instance"); return -1; }
-    DeviceCtx* d = route(n, "PlaneMinMax");
-    if (!d) return -1;
-    SlotGuard g(d);
-    Slot* s = g.s;
-    VSZ_CUDA(cudaSetDevice(d->ordinal));
-    const size_t bytes = f->layout.frame_stride;
-    const int np = processed_planes(f);
-    const size_t scratch = stats_scratch_bytes(1, np) + 256;
-    if (slot_reserve(d, s, 0, bytes) || (b && slot_reserve(d, s, 1, bytes)) || slot_reserve(d, s, 2, scratch)) return -1;
-    if (stage_in(s, 0, f->layout, a, f->process)) return -1;
-    if (b && stage_in(s, 1, f->layout, b, f->process)) return -1;
-    StatsRaw* raw_dev = (StatsRaw*)s->dev_small;
-    int rc = run_planeminmax(f->layout, f->process, s->dev[0], 0, b ? s->dev[1] : nullptr, 0, 1, f->no_thr, f->minthr, f->maxthr,
-                             f->hist_size, s->dev[2], raw_dev, s->stream);
-    if (rc) return rc;
-    VSZ_CUDA(cudaMemcpyAsync(s->pin_small, raw_dev, sizeof(StatsRaw) * np, cudaMemcpyDeviceToHost, s->stream));
-    VSZ_CUDA(cudaStreamSynchronize(s->stream));
-    minmax_finalize(f, (const StatsRaw*)s->pin_small, out);
-    return 0;
+    return stats_get_frame(f, F_PLANEMINMAX, n, a, b, out);
 }
 
 int vszip_planeminmax_device(const vszip_filter* f, const vszip_dev_clip* a, const vszip_dev_clip* b, int32_t first, int32_t count,
                              vszip_minmax_props* out, void* stream) {
-    static const char* name = "PlaneMinMax";
-    if (!f || f->kind != F_PLANEMINMAX) { set_error("PlaneMinMax: bad filter handle"); return -1; }
-    if (f->has_ref != (b != nullptr)) { set_error("PlaneMinMax: clipb presence does not match the filter instance"); return -1; }
-    if (!same_clip_shape(a, f, name) || (b && !same_clip_shape(b, f, name)) || !range_ok(a, first, count, name) || (b && !range_ok(b, first, count, name))) return -1;
-    if (b && b->device_index != a->device_index) { set_error("%s: clips live on different devices", name); return -1; }
-    DeviceCtx* d = device_ctx(a->device_index);
-    if (!d) { set_error("PlaneMinMax: library not initialised"); return -1; }
-    VSZ_CUDA(cudaSetDevice(d->ordinal));
-    cudaStream_t st = stream ? (cudaStream_t)stream : d->batch_stream;
-    const int np = processed_planes(f);
-    if (count == 0 || np == 0) return 0;
-    const size_t fs = a->layout.frame_stride;
-    AsyncScratch scratch_mem;
-    const size_t sb = stats_scratch_bytes(count, np), rb = sizeof(StatsRaw) * (size_t)count * np;
-    VSZ_CUDA(scratch_mem.alloc(sb + rb, st));
-    char* scratch = scratch_mem.p;
-    StatsRaw* raw_dev = (StatsRaw*)(scratch + sb);
-    int rc = run_planeminmax(f->layout, f->process, a->base + (size_t)first * fs, fs, b ? b->base + (size_t)first * fs : nullptr, fs, count,
-                             f->no_thr, f->minthr, f->maxthr, f->hist_size, scratch, raw_dev, st);
-    std::vector<StatsRaw> raw((size_t)count * np);
-    if (!rc && out) {
-        VSZ_CUDA(cudaMemcpyAsync(raw.data(), raw_dev, rb, cudaMemcpyDeviceToHost, st));
-        VSZ_CUDA(cudaStreamSynchronize(st));
-        for (int i = 0; i < count; ++i) minmax_finalize(f, raw.data() + (size_t)i * np, out + i);
-    }
-    return rc;
+    return stats_device(f, F_PLANEMINMAX, a, b, first, count, out, stream);
 }
 
 // =========================================================================== PlaneAverage
@@ -612,7 +673,7 @@ vszip_filter* vszip_planeaverage_create(const vszip_video_info* vi, const vszip_
     f->sample = kind;
     f->layout = make_layout(*vi, kind);
     for (int i = 0; i < 3; ++i) f->process[i] = process[i] && i < vi->num_planes;
-    f->has_ref = clipb_vi != nullptr;
+    f->has_input[0] = clipb_vi != nullptr;
     f->avg_peak = (float)((1ull << vi->bits_per_sample) - 1ull);  // planeaverage.zig:112
     for (int i = 0; i < a->num_exclude; ++i) {
         f->exclude_f.push_back((float)a->exclude[i]);           // planeaverage.zig:122-125
@@ -651,7 +712,7 @@ static int average_upload(const vszip_filter* cf, int dev_index, const int32_t**
 static void average_finalize(const vszip_filter* f, const StatsRaw* raw, vszip_average_props* out) {
     const bool flt = f->sample == K_F16 || f->sample == K_F32;
     memset(out, 0, sizeof *out);
-    out->has_diff = f->has_ref;
+    out->has_diff = f->has_input[0];
     int k = 0;
     for (int p = 0; p < f->layout.nplanes; ++p) {
         if (!f->process[p]) continue;
@@ -663,92 +724,98 @@ static void average_finalize(const vszip_filter* f, const StatsRaw* raw, vszip_a
         if (total == 0) out->avg[k] = 0.0;
         else if (flt) out->avg[k] = r.fsum / total;
         else out->avg[k] = (double)r.isum / total / (double)f->avg_peak;
-        if (f->has_ref) out->diff[k] = flt ? r.fdiff / (double)all : (double)r.idiff / (double)all / (double)f->avg_peak;
+        if (f->has_input[0]) out->diff[k] = flt ? r.fdiff / (double)all : (double)r.idiff / (double)all / (double)f->avg_peak;
         ++k;
     }
     out->count = k;
 }
 
 int vszip_planeaverage_get_frame(const vszip_filter* f, int32_t n, const vszip_frame* a, const vszip_frame* b, vszip_average_props* out) {
-    if (!f || f->kind != F_PLANEAVERAGE) { set_error("PlaneAverage: bad filter handle"); return -1; }
-    if (f->has_ref != (b != nullptr)) { set_error("PlaneAverage: clipb frame presence does not match the filter instance"); return -1; }
-    DeviceCtx* d = route(n, "PlaneAverage");
-    if (!d) return -1;
-    SlotGuard g(d);
-    Slot* s = g.s;
-    VSZ_CUDA(cudaSetDevice(d->ordinal));
-    const size_t bytes = f->layout.frame_stride;
-    const int np = processed_planes(f);
-    const size_t scratch = stats_scratch_bytes(1, np) + 256;
-    if (slot_reserve(d, s, 0, bytes) || (b && slot_reserve(d, s, 1, bytes)) || slot_reserve(d, s, 2, scratch)) return -1;
-    if (stage_in(s, 0, f->layout, a, f->process)) return -1;
-    if (b && stage_in(s, 1, f->layout, b, f->process)) return -1;
-    StatsRaw* raw_dev = (StatsRaw*)s->dev_small;
-    const int32_t* xi; const float* xf;
-    if (average_upload(f, device_index_of(d), &xi, &xf)) return -1;
-    int rc = run_planeaverage(f->layout, f->process, s->dev[0], 0, b ? s->dev[1] : nullptr, 0, 1, f->exclude_i.data(), f->exclude_f.data(),
-                              (int)f->exclude_i.size(), xi, xf, s->dev[2], raw_dev, s->stream);
-    if (rc) return rc;
-    VSZ_CUDA(cudaMemcpyAsync(s->pin_small, raw_dev, sizeof(StatsRaw) * np, cudaMemcpyDeviceToHost, s->stream));
-    VSZ_CUDA(cudaStreamSynchronize(s->stream));
-    average_finalize(f, (const StatsRaw*)s->pin_small, out);
-    return 0;
+    return stats_get_frame(f, F_PLANEAVERAGE, n, a, b, out);
 }
 
 int vszip_planeaverage_device(const vszip_filter* f, const vszip_dev_clip* a, const vszip_dev_clip* b, int32_t first, int32_t count,
                               vszip_average_props* out, void* stream) {
-    static const char* name = "PlaneAverage";
-    if (!f || f->kind != F_PLANEAVERAGE) { set_error("PlaneAverage: bad filter handle"); return -1; }
-    if (f->has_ref != (b != nullptr)) { set_error("PlaneAverage: clipb presence does not match the filter instance"); return -1; }
-    if (!same_clip_shape(a, f, name) || (b && !same_clip_shape(b, f, name)) || !range_ok(a, first, count, name) || (b && !range_ok(b, first, count, name))) return -1;
-    if (b && b->device_index != a->device_index) { set_error("%s: clips live on different devices", name); return -1; }
-    DeviceCtx* d = device_ctx(a->device_index);
-    if (!d) { set_error("PlaneAverage: library not initialised"); return -1; }
-    VSZ_CUDA(cudaSetDevice(d->ordinal));
-    cudaStream_t st = stream ? (cudaStream_t)stream : d->batch_stream;
-    const int np = processed_planes(f);
-    if (count == 0 || np == 0) return 0;
-    const size_t fs = a->layout.frame_stride;
-    AsyncScratch scratch_mem;
-    const size_t sb = stats_scratch_bytes(count, np), rb = sizeof(StatsRaw) * (size_t)count * np;
-    VSZ_CUDA(scratch_mem.alloc(sb + rb, st));
-    char* scratch = scratch_mem.p;
-    StatsRaw* raw_dev = (StatsRaw*)(scratch + sb);
-    const int32_t* xi; const float* xf;
-    if (average_upload(f, a->device_index, &xi, &xf)) return -1;
-    int rc = run_planeaverage(f->layout, f->process, a->base + (size_t)first * fs, fs, b ? b->base + (size_t)first * fs : nullptr, fs, count,
-                              f->exclude_i.data(), f->exclude_f.data(), (int)f->exclude_i.size(), xi, xf, scratch, raw_dev, st);
-    std::vector<StatsRaw> raw((size_t)count * np);
-    if (!rc && out) {
-        VSZ_CUDA(cudaMemcpyAsync(raw.data(), raw_dev, rb, cudaMemcpyDeviceToHost, st));
-        VSZ_CUDA(cudaStreamSynchronize(st));
-        for (int i = 0; i < count; ++i) average_finalize(f, raw.data() + (size_t)i * np, out + i);
+    return stats_device(f, F_PLANEAVERAGE, a, b, first, count, out, stream);
+}
+
+// =========================================================================== dispatch
+static int run_pixels(const vszip_filter* f, int dev_index, const char* const in[3], char* out, size_t fs, int count, cudaStream_t st) {
+    const FrameLayout& l = f->layout;
+    switch (f->kind) {
+        case F_BOXBLUR:
+            return run_boxblur(l, f->process, in[0], fs, out, fs, count, (int)f->hradius, f->hpasses, (int)f->vradius, f->vpasses, st);
+        case F_BILATERAL:
+            if (bilateral_upload(f, dev_index)) return -1;
+            return bilateral_run(f, dev_index, in[0], fs, in[1], fs, out, fs, count, st);
+        case F_LIMITER:
+            return run_limiter(l, f->process, in[0], fs, out, fs, count, f->lim_lo, f->lim_hi, st);
+        case F_LIMITFILTER:  // flt = the main input, src = the second, ref = the third
+            return run_limitfilter(l, f->process, in[0], fs, in[1], fs, in[2], fs, out, fs, count, f->lf_dark, f->lf_bright, f->lf_elast, st);
+        default:  // AdaptiveBinarize: clip = the second input, clip2 = the main one
+            return run_adaptivebinarize(l, in[1], fs, in[0], fs, out, fs, count, f->ab_c, st);
     }
-    return rc;
+}
+
+static int run_stats(const vszip_filter* f, int dev_index, const char* a, const char* b, size_t fs, int count, void* scratch,
+                     StatsRaw* raw, cudaStream_t st) {
+    if (f->kind == F_PLANEMINMAX)
+        return run_planeminmax(f->layout, f->process, a, fs, b, fs, count, f->no_thr, f->minthr, f->maxthr, f->hist_size, scratch, raw, st);
+    const int32_t* xi; const float* xf;
+    if (average_upload(f, dev_index, &xi, &xf)) return -1;
+    return run_planeaverage(f->layout, f->process, a, fs, b, fs, count, f->exclude_i.data(), f->exclude_f.data(), (int)f->exclude_i.size(),
+                            xi, xf, scratch, raw, st);
+}
+
+static void stats_finalize(const vszip_filter* f, const StatsRaw* raw, void* props, int i) {
+    if (f->kind == F_PLANEMINMAX) minmax_finalize(f, raw, (vszip_minmax_props*)props + i);
+    else average_finalize(f, raw, (vszip_average_props*)props + i);
 }
 
 // =========================================================================== PlaneMinMax + PlaneAverage from one read (SURVEY 8f rank 4)
-// b: the clipb clip (may be nullptr); a filter created without clipb ignores it.  The pair shares one read only when both filters read
-// b (or neither does).
+// A PlaneMinMax and a PlaneAverage (either order) that one read can serve: the same planes, at least one of them, and an exclude
+// list short enough for the fused kernels.
+static bool stats_pair(const vszip_filter* x, const vszip_filter* y) {
+    if (!((x->kind == F_PLANEMINMAX && y->kind == F_PLANEAVERAGE) || (x->kind == F_PLANEAVERAGE && y->kind == F_PLANEMINMAX))) return false;
+    const vszip_filter* fa = x->kind == F_PLANEAVERAGE ? x : y;
+    return x->process[0] == y->process[0] && x->process[1] == y->process[1] && x->process[2] == y->process[2] && processed_planes(x) > 0 &&
+           fa->exclude_i.size() <= 16;
+}
+
+// PlaneMinMax and PlaneAverage, f and g in either order, over the same frames a; each reads the clipb b if it was created with it.
+// One read when both read b (or neither does) and run_planestats_fused takes the pair (then *fused is set, if given), else f and
+// then g on their own, in scratch_f and scratch_g.
+static int run_stats_pair(const vszip_filter* f, const vszip_filter* g, int dev_index, const char* a, const char* b, size_t fs, int count,
+                          bool same_float_sums, char* scratch_f, char* scratch_g, StatsRaw* raw_f, StatsRaw* raw_g, cudaStream_t st,
+                          bool* fused) {
+    const char* bf = f->has_input[0] ? b : nullptr;
+    const char* bg = g->has_input[0] ? b : nullptr;
+    if (stats_pair(f, g) && bf == bg) {
+        const vszip_filter* fm = f->kind == F_PLANEMINMAX ? f : g;
+        const vszip_filter* fa = f->kind == F_PLANEMINMAX ? g : f;
+        const int rc = run_planestats_fused(fm->layout, fm->process, a, fs, bf, fs, count, fm->no_thr, fm->minthr, fm->maxthr, fm->hist_size,
+                                            fa->exclude_i.data(), fa->exclude_f.data(), (int)fa->exclude_i.size(), same_float_sums, scratch_f,
+                                            fm == f ? raw_f : raw_g, fm == f ? raw_g : raw_f, st);
+        if (rc == 0 && fused) *fused = true;
+        if (rc != 1) return rc;
+    }
+    int rc = 0;  // not eligible: the two reductions one after the other (two reads)
+    if (processed_planes(f)) rc = run_stats(f, dev_index, a, bf, fs, count, scratch_f, raw_f, st);
+    if (!rc && processed_planes(g)) rc = run_stats(g, dev_index, a, bg, fs, count, scratch_g, raw_g, st);
+    return rc;
+}
+
+// b: the clipb clip (may be nullptr); a filter created without clipb ignores it.
 static int planestats_run(const vszip_filter* fm, const vszip_filter* fa, const vszip_dev_clip* a, const vszip_dev_clip* b, int32_t first,
                           int32_t count, bool same_float_sums, vszip_minmax_props* mm_out, vszip_average_props* avg_out, int32_t* fused_out,
                           void* stream) {
     static const char* name = "PlaneStats";
-    if (!same_clip_shape(a, fm, name) || !same_clip_shape(a, fa, name) || !range_ok(a, first, count, name)) return -1;
-    if (b && (!same_clip_shape(b, fm, name) || !range_ok(b, first, count, name))) return -1;
-    if (b && b->device_index != a->device_index) { set_error("%s: clips live on different devices", name); return -1; }
-    DeviceCtx* d = device_ctx(a->device_index);
-    if (!d) { set_error("PlaneStats: library not initialised"); return -1; }
-    VSZ_CUDA(cudaSetDevice(d->ordinal));
-    cudaStream_t st = stream ? (cudaStream_t)stream : d->batch_stream;
+    const vszip_dev_clip* clips[2] = {a, b};
+    cudaStream_t st;
+    if (!same_clip_shape(a, fa, name) || begin_device_call(fm, name, clips, b ? 2 : 1, first, count, stream, &st)) return -1;
     const int npm = processed_planes(fm), npa = processed_planes(fa);
     if (count == 0) return 0;
     const size_t fs = a->layout.frame_stride;
-    const char* base = a->base + (size_t)first * fs;
-    const char* bbase = b ? b->base + (size_t)first * fs : nullptr;
-    const char* bm = fm->has_ref ? bbase : nullptr;
-    const char* ba = fa->has_ref ? bbase : nullptr;
-    const bool same_planes = fm->process[0] == fa->process[0] && fm->process[1] == fa->process[1] && fm->process[2] == fa->process[2];
     const size_t sbm = stats_scratch_bytes(count, std::max(npm, 1)), sba = stats_scratch_bytes(count, std::max(npa, 1));
     const size_t rbm = sizeof(StatsRaw) * (size_t)count * npm, rba = sizeof(StatsRaw) * (size_t)count * npa;
     const size_t rbm_al = (rbm + 255) & ~(size_t)255;
@@ -757,19 +824,10 @@ static int planestats_run(const vszip_filter* fm, const vszip_filter* fa, const 
     char* scratch = scratch_mem.p;
     StatsRaw* raw_m = (StatsRaw*)(scratch + sbm + sba);
     StatsRaw* raw_a = (StatsRaw*)(scratch + sbm + sba + rbm_al);
-    int rc = 1;
-    if (same_planes && npm > 0 && fa->exclude_i.size() <= 16 && bm == ba)
-        rc = run_planestats_fused(fm->layout, fm->process, base, fs, bm, fs, count, fm->no_thr, fm->minthr, fm->maxthr, fm->hist_size,
-                                  fa->exclude_i.data(), fa->exclude_f.data(), (int)fa->exclude_i.size(), same_float_sums, scratch, raw_m, raw_a, st);
-    if (rc == 0 && fused_out) *fused_out = 1;
-    if (rc == 1) {  // not eligible: the two reductions one after the other (two reads)
-        rc = 0;
-        if (npm) rc = run_planeminmax(fm->layout, fm->process, base, fs, bm, fs, count, fm->no_thr, fm->minthr, fm->maxthr, fm->hist_size, scratch, raw_m, st);
-        const int32_t* xi; const float* xf;
-        if (!rc && npa && average_upload(fa, a->device_index, &xi, &xf)) rc = -1;
-        if (!rc && npa) rc = run_planeaverage(fa->layout, fa->process, base, fs, ba, fs, count, fa->exclude_i.data(), fa->exclude_f.data(),
-                                               (int)fa->exclude_i.size(), xi, xf, scratch + sbm, raw_a, st);
-    }
+    bool fused = false;
+    const int rc = run_stats_pair(fm, fa, a->device_index, a->base + (size_t)first * fs, b ? b->base + (size_t)first * fs : nullptr, fs, count,
+                                  same_float_sums, scratch, scratch + sbm, raw_m, raw_a, st, &fused);
+    if (fused && fused_out) *fused_out = 1;
     if (!rc && (mm_out || avg_out)) {
         std::vector<StatsRaw> hm((size_t)count * npm), ha((size_t)count * npa);
         if (mm_out && npm) VSZ_CUDA(cudaMemcpyAsync(hm.data(), raw_m, rbm, cudaMemcpyDeviceToHost, st));
@@ -787,7 +845,7 @@ int vszip_planestats_device(const vszip_filter* fm, const vszip_filter* fa, cons
                             vszip_minmax_props* mm_out, vszip_average_props* avg_out, int32_t* fused_out, void* stream) {
     if (fused_out) *fused_out = 0;
     if (!fm || fm->kind != F_PLANEMINMAX || !fa || fa->kind != F_PLANEAVERAGE) { set_error("PlaneStats: a PlaneMinMax and a PlaneAverage handle are required"); return -1; }
-    if (fm->has_ref || fa->has_ref) { set_error("PlaneStats: filters created with clipb cannot be combined"); return -1; }
+    if (fm->has_input[0] || fa->has_input[0]) { set_error("PlaneStats: filters created with clipb cannot be combined"); return -1; }
     return planestats_run(fm, fa, a, nullptr, first, count, false, mm_out, avg_out, fused_out, stream);
 }
 
@@ -795,7 +853,7 @@ int vszip_planestats_device_b(const vszip_filter* fm, const vszip_filter* fa, co
                               int32_t count, vszip_minmax_props* mm_out, vszip_average_props* avg_out, int32_t* fused_out, void* stream) {
     if (fused_out) *fused_out = 0;
     if (!fm || fm->kind != F_PLANEMINMAX || !fa || fa->kind != F_PLANEAVERAGE) { set_error("PlaneStats: a PlaneMinMax and a PlaneAverage handle are required"); return -1; }
-    if ((fm->has_ref || fa->has_ref) != (b != nullptr)) { set_error("PlaneStats: clipb presence does not match the filter instances"); return -1; }
+    if ((fm->has_input[0] || fa->has_input[0]) != (b != nullptr)) { set_error("PlaneStats: clipb presence does not match the filter instances"); return -1; }
     return planestats_run(fm, fa, a, b, first, count, true, mm_out, avg_out, fused_out, stream);
 }
 
@@ -877,40 +935,15 @@ vszip_filter* vszip_limiter_create(const vszip_video_info* vi, const vszip_limit
     f->sample = kind;
     f->layout = make_layout(*vi, kind);
     for (int i = 0; i < 3; ++i) { f->process[i] = process[i] && i < np; f->lim_lo[i] = lo[i]; f->lim_hi[i] = hi[i]; }
-    f->has_ref = false;
     return f;
 }
 
 int vszip_limiter_get_frame(const vszip_filter* f, int32_t n, const vszip_frame* src, vszip_frame* dst) {
-    if (!f || f->kind != F_LIMITER) { set_error("Limiter: bad filter handle"); return -1; }
-    DeviceCtx* d = route(n, "Limiter");
-    if (!d) return -1;
-    SlotGuard g(d);
-    Slot* s = g.s;
-    VSZ_CUDA(cudaSetDevice(d->ordinal));
-    const size_t bytes = f->layout.frame_stride;
-    if (slot_reserve(d, s, 0, bytes) || slot_reserve(d, s, 2, bytes)) return -1;
-    if (stage_in(s, 0, f->layout, src, f->process)) return -1;
-    int rc = run_limiter(f->layout, f->process, s->dev[0], 0, s->dev[2], 0, 1, f->lim_lo, f->lim_hi, s->stream);
-    if (rc) return rc;
-    bool direct[3];
-    if (stage_out_begin(s, f->layout, dst, f->process, direct)) return -1;
-    VSZ_CUDA(cudaStreamSynchronize(s->stream));
-    stage_out_finish(s, f->layout, dst, f->process, direct);
-    return 0;
+    return pixel_get_frame(f, F_LIMITER, n, {src, nullptr, nullptr}, dst);
 }
 
 int vszip_limiter_device(const vszip_filter* f, const vszip_dev_clip* src, vszip_dev_clip* dst, int32_t first, int32_t count, void* stream) {
-    static const char* name = "Limiter";
-    if (!f || f->kind != F_LIMITER) { set_error("Limiter: bad filter handle"); return -1; }
-    if (!same_clip_shape(src, f, name) || !same_clip_shape(dst, f, name) || !range_ok(src, first, count, name) || !range_ok(dst, first, count, name)) return -1;
-    if (src->device_index != dst->device_index) { set_error("Limiter: clips live on different devices"); return -1; }
-    DeviceCtx* d = device_ctx(src->device_index);
-    if (!d) { set_error("Limiter: library not initialised"); return -1; }
-    VSZ_CUDA(cudaSetDevice(d->ordinal));
-    cudaStream_t st = stream ? (cudaStream_t)stream : d->batch_stream;
-    const size_t fs = src->layout.frame_stride;
-    return run_limiter(f->layout, f->process, src->base + (size_t)first * fs, fs, dst->base + (size_t)first * fs, fs, count, f->lim_lo, f->lim_hi, st);
+    return pixel_device(f, F_LIMITER, {src, nullptr, nullptr}, dst, first, count, stream);
 }
 
 // =========================================================================== LimitFilter
@@ -944,8 +977,8 @@ vszip_filter* vszip_limitfilter_create(const vszip_video_info* flt_vi, const vsz
         f->lf_bright[i] = scale_value8(bright[i], *flt_vi, limited);
         f->lf_elast[i] = elast[i];
     }
-    f->lf_has_ref = ref_vi != nullptr;
-    f->has_ref = true;  // multi-input: not fusable into a linear chain
+    f->has_input[0] = true;
+    f->has_input[1] = ref_vi != nullptr;
     return f;
 }
 
@@ -957,46 +990,13 @@ int vszip_limitfilter_get_info(const vszip_filter* f, float dark_thr[3], float b
 
 int vszip_limitfilter_get_frame(const vszip_filter* f, int32_t n, const vszip_frame* flt, const vszip_frame* src, const vszip_frame* ref,
                                 vszip_frame* dst) {
-    if (!f || f->kind != F_LIMITFILTER) { set_error("LimitFilter: bad filter handle"); return -1; }
     if (!flt || !src || !dst) { set_error("LimitFilter: flt, src and dst frames are required"); return -1; }
-    if (f->lf_has_ref != (ref != nullptr)) { set_error("LimitFilter: ref frame presence does not match the filter instance"); return -1; }
-    DeviceCtx* d = route(n, "LimitFilter");
-    if (!d) return -1;
-    SlotGuard g(d);
-    Slot* s = g.s;
-    VSZ_CUDA(cudaSetDevice(d->ordinal));
-    const size_t bytes = f->layout.frame_stride;
-    if (slot_reserve(d, s, 0, bytes) || slot_reserve(d, s, 1, bytes) || slot_reserve(d, s, 2, bytes) || (ref && slot_reserve(d, s, 3, bytes))) return -1;
-    if (stage_in(s, 0, f->layout, flt, f->process) || stage_in(s, 1, f->layout, src, f->process)) return -1;
-    if (ref && stage_in(s, 3, f->layout, ref, f->process)) return -1;
-    int rc = run_limitfilter(f->layout, f->process, s->dev[0], 0, s->dev[1], 0, ref ? s->dev[3] : nullptr, 0, s->dev[2], 0, 1, f->lf_dark,
-                             f->lf_bright, f->lf_elast, s->stream);
-    if (rc) return rc;
-    bool direct[3];
-    if (stage_out_begin(s, f->layout, dst, f->process, direct)) return -1;
-    VSZ_CUDA(cudaStreamSynchronize(s->stream));
-    stage_out_finish(s, f->layout, dst, f->process, direct);
-    return 0;
+    return pixel_get_frame(f, F_LIMITFILTER, n, {flt, src, ref}, dst);
 }
 
 int vszip_limitfilter_device(const vszip_filter* f, const vszip_dev_clip* flt, const vszip_dev_clip* src, const vszip_dev_clip* ref,
                              vszip_dev_clip* dst, int32_t first, int32_t count, void* stream) {
-    static const char* name = "LimitFilter";
-    if (!f || f->kind != F_LIMITFILTER) { set_error("LimitFilter: bad filter handle"); return -1; }
-    if (f->lf_has_ref != (ref != nullptr)) { set_error("LimitFilter: ref clip presence does not match the filter instance"); return -1; }
-    if (!same_clip_shape(flt, f, name) || !same_clip_shape(src, f, name) || !same_clip_shape(dst, f, name) || (ref && !same_clip_shape(ref, f, name))) return -1;
-    if (!range_ok(flt, first, count, name) || !range_ok(src, first, count, name) || !range_ok(dst, first, count, name) || (ref && !range_ok(ref, first, count, name))) return -1;
-    if (flt->device_index != dst->device_index || src->device_index != dst->device_index || (ref && ref->device_index != dst->device_index)) {
-        set_error("LimitFilter: clips live on different devices");
-        return -1;
-    }
-    DeviceCtx* d = device_ctx(dst->device_index);
-    if (!d) { set_error("LimitFilter: library not initialised"); return -1; }
-    VSZ_CUDA(cudaSetDevice(d->ordinal));
-    cudaStream_t st = stream ? (cudaStream_t)stream : d->batch_stream;
-    const size_t fs = dst->layout.frame_stride, off = (size_t)first * fs;
-    return run_limitfilter(f->layout, f->process, flt->base + off, fs, src->base + off, fs, ref ? ref->base + off : nullptr, fs, dst->base + off, fs,
-                           count, f->lf_dark, f->lf_bright, f->lf_elast, st);
+    return pixel_device(f, F_LIMITFILTER, {flt, src, ref}, dst, first, count, stream);
 }
 
 // =========================================================================== AdaptiveBinarize
@@ -1014,43 +1014,19 @@ vszip_filter* vszip_adaptivebinarize_create(const vszip_video_info* vi, const vs
     f->layout = make_layout(*vi, K_U8);
     for (int i = 0; i < 3; ++i) f->process[i] = i < vi->num_planes;
     f->ab_c = (int)std::min<int64_t>(std::max<int64_t>(c, -256), 256);               // :97-99
-    f->has_ref = true;
+    f->has_input[0] = true;
     return f;
 }
 
+// In the chain's numbering clip2 is the main input (the one binarised) and clip the second.
 int vszip_adaptivebinarize_get_frame(const vszip_filter* f, int32_t n, const vszip_frame* clip, const vszip_frame* clip2, vszip_frame* dst) {
-    if (!f || f->kind != F_ADAPTIVEBINARIZE) { set_error("AdaptiveBinarize: bad filter handle"); return -1; }
     if (!clip || !clip2 || !dst) { set_error("AdaptiveBinarize: clip, clip2 and dst frames are required"); return -1; }
-    DeviceCtx* d = route(n, "AdaptiveBinarize");
-    if (!d) return -1;
-    SlotGuard g(d);
-    Slot* s = g.s;
-    VSZ_CUDA(cudaSetDevice(d->ordinal));
-    const size_t bytes = f->layout.frame_stride;
-    if (slot_reserve(d, s, 0, bytes) || slot_reserve(d, s, 1, bytes) || slot_reserve(d, s, 2, bytes)) return -1;
-    if (stage_in(s, 0, f->layout, clip, f->process) || stage_in(s, 1, f->layout, clip2, f->process)) return -1;
-    int rc = run_adaptivebinarize(f->layout, s->dev[0], 0, s->dev[1], 0, s->dev[2], 0, 1, f->ab_c, s->stream);
-    if (rc) return rc;
-    bool direct[3];
-    if (stage_out_begin(s, f->layout, dst, f->process, direct)) return -1;
-    VSZ_CUDA(cudaStreamSynchronize(s->stream));
-    stage_out_finish(s, f->layout, dst, f->process, direct);
-    return 0;
+    return pixel_get_frame(f, F_ADAPTIVEBINARIZE, n, {clip2, clip, nullptr}, dst);
 }
 
 int vszip_adaptivebinarize_device(const vszip_filter* f, const vszip_dev_clip* clip, const vszip_dev_clip* clip2, vszip_dev_clip* dst,
                                   int32_t first, int32_t count, void* stream) {
-    static const char* name = "AdaptiveBinarize";
-    if (!f || f->kind != F_ADAPTIVEBINARIZE) { set_error("AdaptiveBinarize: bad filter handle"); return -1; }
-    if (!same_clip_shape(clip, f, name) || !same_clip_shape(clip2, f, name) || !same_clip_shape(dst, f, name)) return -1;
-    if (!range_ok(clip, first, count, name) || !range_ok(clip2, first, count, name) || !range_ok(dst, first, count, name)) return -1;
-    if (clip->device_index != dst->device_index || clip2->device_index != dst->device_index) { set_error("AdaptiveBinarize: clips live on different devices"); return -1; }
-    DeviceCtx* d = device_ctx(dst->device_index);
-    if (!d) { set_error("AdaptiveBinarize: library not initialised"); return -1; }
-    VSZ_CUDA(cudaSetDevice(d->ordinal));
-    cudaStream_t st = stream ? (cudaStream_t)stream : d->batch_stream;
-    const size_t fs = dst->layout.frame_stride, off = (size_t)first * fs;
-    return run_adaptivebinarize(f->layout, clip->base + off, fs, clip2->base + off, fs, dst->base + off, fs, count, f->ab_c, st);
+    return pixel_device(f, F_ADAPTIVEBINARIZE, {clip2, clip, nullptr}, dst, first, count, stream);
 }
 
 // =========================================================================== fused chains
@@ -1071,46 +1047,10 @@ struct vszip_chain {
 
 namespace {
 
-bool is_pixel(const vszip_filter* f) {
-    return f->kind == F_BOXBLUR || f->kind == F_BILATERAL || f->kind == F_LIMITER || f->kind == F_LIMITFILTER || f->kind == F_ADAPTIVEBINARIZE;
-}
-
-const char* kind_name(const vszip_filter* f) {
-    switch (f->kind) {
-        case F_BOXBLUR: return "BoxBlur";
-        case F_BILATERAL: return "Bilateral";
-        case F_PLANEMINMAX: return "PlaneMinMax";
-        case F_PLANEAVERAGE: return "PlaneAverage";
-        case F_LIMITER: return "Limiter";
-        case F_LIMITFILTER: return "LimitFilter";
-        default: return "AdaptiveBinarize";
-    }
-}
-
-// The filter's own names for its second / third input and whether it was created with them.
-void extra_inputs(const vszip_filter* f, const char* names[2], bool has[2]) {
-    names[0] = names[1] = nullptr;
-    has[0] = has[1] = false;
-    switch (f->kind) {
-        case F_BILATERAL: names[0] = "ref"; has[0] = f->has_ref; break;
-        case F_PLANEMINMAX: case F_PLANEAVERAGE: names[0] = "clipb"; has[0] = f->has_ref; break;
-        case F_LIMITFILTER: names[0] = "src"; has[0] = true; names[1] = "ref"; has[1] = f->lf_has_ref; break;
-        case F_ADAPTIVEBINARIZE: names[0] = "clip"; has[0] = true; break;
-        default: break;
-    }
-}
-
 bool same_format(const vszip_video_info& a, const vszip_video_info& b) {
     return a.width == b.width && a.height == b.height && a.color_family == b.color_family && a.sample_type == b.sample_type &&
            a.bits_per_sample == b.bits_per_sample && a.sub_sampling_w == b.sub_sampling_w && a.sub_sampling_h == b.sub_sampling_h &&
            a.num_planes == b.num_planes;
-}
-
-bool stats_pair(const vszip_filter* x, const vszip_filter* y) {
-    if (!((x->kind == F_PLANEMINMAX && y->kind == F_PLANEAVERAGE) || (x->kind == F_PLANEAVERAGE && y->kind == F_PLANEMINMAX))) return false;
-    const vszip_filter* fa = x->kind == F_PLANEAVERAGE ? x : y;
-    return x->process[0] == y->process[0] && x->process[1] == y->process[1] && x->process[2] == y->process[2] && processed_planes(x) > 0 &&
-           fa->exclude_i.size() <= 16;
 }
 
 // input / second / third use the value numbering above; input == nullptr: every element reads the latest pixel output (or the source).
@@ -1192,8 +1132,8 @@ vszip_chain* vszip_chain_create(const vszip_filter* const* filters, int32_t coun
         const vszip_filter* f = filters[i];
         if (!f) { set_error("chain: filter %d is NULL", i); return nullptr; }
         // LimitFilter (without ref) and AdaptiveBinarize take the chain's SOURCE frame as their second clip ("diamond" elements)
-        const bool diamond = (f->kind == F_LIMITFILTER && !f->lf_has_ref) || f->kind == F_ADAPTIVEBINARIZE;
-        if (f->has_ref && !diamond) { set_error("chain: filter %d takes a second clip (ref/clipb); only single-input filters can be fused", i); return nullptr; }
+        const bool diamond = (f->kind == F_LIMITFILTER && !f->has_input[1]) || f->kind == F_ADAPTIVEBINARIZE;
+        if (f->has_input[0] && !diamond) { set_error("chain: filter %d takes a second clip (ref/clipb); only single-input filters can be fused", i); return nullptr; }
         if (!same_format(f0->vi, f->vi)) {
             set_error("chain: filter %d was created for a different video format than filter 0", i);
             return nullptr;
@@ -1214,23 +1154,21 @@ vszip_chain* vszip_chain_create2(const vszip_filter* const* filters, int32_t cou
             set_error("chain: filter %d was created for a different video format than filter 0", i);
             return nullptr;
         }
-        const char* names[2];
-        bool has[2];
-        extra_inputs(f, names, has);
+        const KindInfo& info = kind_info(f->kind);
         const int32_t refs[3] = {input ? input[i] : 0, second ? second[i] : -1, third ? third[i] : -1};
         static const char* arr[3] = {"input", "second", "third"};
         static const char* none[3] = {"", "a second clip", "a third clip"};
         for (int k = 0; k < 3; ++k) {
             const int32_t v = refs[k];
             if (k > 0) {
-                const char* what = names[k - 1] ? names[k - 1] : none[k];
-                if (!has[k - 1] && v != -1) { set_error("chain: filter %d (%s) was created without %s; %s[%d] must be -1", i, kind_name(f), what, arr[k], i); return nullptr; }
-                if (has[k - 1] && v == -1) { set_error("chain: filter %d (%s) was created with %s; %s[%d] must name its input", i, kind_name(f), what, arr[k], i); return nullptr; }
+                const char* what = info.input[k - 1] ? info.input[k - 1] : none[k];
+                if (!f->has_input[k - 1] && v != -1) { set_error("chain: filter %d (%s) was created without %s; %s[%d] must be -1", i, info.name, what, arr[k], i); return nullptr; }
+                if (f->has_input[k - 1] && v == -1) { set_error("chain: filter %d (%s) was created with %s; %s[%d] must name its input", i, info.name, what, arr[k], i); return nullptr; }
                 if (v == -1) continue;
             }
             if (v < 0 || v > count) { set_error("chain: %s[%d] = %d is out of range (0 = the source, k = the output of filter k - 1)", arr[k], i, v); return nullptr; }
             if (v >= 1 && v - 1 >= i) { set_error("chain: %s[%d] names filter %d, which does not come before filter %d", arr[k], i, v - 1, i); return nullptr; }
-            if (v >= 1 && !is_pixel(filters[v - 1])) { set_error("chain: %s[%d] names filter %d (%s), which has no pixel output", arr[k], i, v - 1, kind_name(filters[v - 1])); return nullptr; }
+            if (v >= 1 && !is_pixel(filters[v - 1])) { set_error("chain: %s[%d] names filter %d (%s), which has no pixel output", arr[k], i, v - 1, kind_info(filters[v - 1]->kind).name); return nullptr; }
         }
     }
     return chain_build(filters, count, input, second, third);
@@ -1264,70 +1202,36 @@ int vszip_chain_get_frame(const vszip_chain* c, int32_t n, const vszip_frame* sr
     int stats_seen = 0;
     for (size_t i = 0; i < c->fl.size(); ++i) {
         const vszip_filter* f = c->fl[i];
-        char* cur = B(c->in[i]);
-        const char* in2 = B(c->in2[i]);
+        const char* in[3] = {B(c->in[i]), B(c->in2[i]), B(c->in3[i])};
         if (is_pixel(f)) {
             char* nxt = B(c->out[i]);
             for (int p = 0; p < l.nplanes; ++p) {  // planes this filter passes through
                 if (f->process[p]) continue;
-                VSZ_CUDA(cudaMemcpyAsync(nxt + l.pl[p].offset, cur + l.pl[p].offset, (size_t)l.pl[p].pitch * l.pl[p].h,
+                VSZ_CUDA(cudaMemcpyAsync(nxt + l.pl[p].offset, in[0] + l.pl[p].offset, (size_t)l.pl[p].pitch * l.pl[p].h,
                                          cudaMemcpyDeviceToDevice, s->stream));
             }
-            int rc;
-            if (f->kind == F_BOXBLUR) {
-                rc = run_boxblur(l, f->process, cur, 0, nxt, 0, 1, (int)f->hradius, f->hpasses, (int)f->vradius, f->vpasses, s->stream);
-            } else if (f->kind == F_LIMITER) {
-                rc = run_limiter(l, f->process, cur, 0, nxt, 0, 1, f->lim_lo, f->lim_hi, s->stream);
-            } else if (f->kind == F_LIMITFILTER) {       // flt = the main input, src = the second, ref = the third
-                rc = run_limitfilter(l, f->process, cur, 0, in2, 0, B(c->in3[i]), 0, nxt, 0, 1, f->lf_dark, f->lf_bright, f->lf_elast, s->stream);
-            } else if (f->kind == F_ADAPTIVEBINARIZE) {  // clip = the second input, clip2 = the main input
-                rc = run_adaptivebinarize(l, in2, 0, cur, 0, nxt, 0, 1, f->ab_c, s->stream);
-            } else {
-                if (bilateral_upload(f, dev_index)) return -1;
-                rc = bilateral_run(f, dev_index, cur, 0, in2, 0, nxt, 0, 1, s->stream);
-            }
+            const int rc = run_pixels(f, dev_index, in, nxt, 0, 1, s->stream);
             if (rc) return rc;
-        } else {
-            const bool pair = c->fuse_next[i] != 0;
-            for (size_t e = i; e <= i + (pair ? 1 : 0); ++e)
-                if (!props_out || !props_out[e]) { set_error("chain: props_out[%d] is required for a PlaneMinMax/PlaneAverage element", (int)e); return -1; }
-            const int np = processed_planes(f);
-            if (np == 0) { ++stats_seen; continue; }
-            const size_t sb = stats_scratch_bytes(1, np);
-            AsyncScratch stats_mem;
-            VSZ_CUDA(stats_mem.alloc(sb, s->stream));
-            char* stats_scratch = stats_mem.p;
-            StatsRaw* raw_dev = (StatsRaw*)s->dev_small + (size_t)stats_seen * 3;
-            int rc = 1;
-            if (pair) {  // a PlaneMinMax and a PlaneAverage of the same value, planes and clipb: one read (same results as two)
-                StatsRaw* raw_next = raw_dev + 3;
-                const vszip_filter* g2 = c->fl[i + 1];
-                const vszip_filter* fm = f->kind == F_PLANEMINMAX ? f : g2;
-                const vszip_filter* fa = f->kind == F_PLANEMINMAX ? g2 : f;
-                rc = run_planestats_fused(l, fm->process, cur, 0, in2, 0, 1, fm->no_thr, fm->minthr, fm->maxthr, fm->hist_size, fa->exclude_i.data(),
-                                          fa->exclude_f.data(), (int)fa->exclude_i.size(), true, stats_scratch,
-                                          fm == f ? raw_dev : raw_next, fm == f ? raw_next : raw_dev, s->stream);
-                if (rc < 0) return rc;
-                if (rc == 0) {
-                    VSZ_CUDA(cudaMemcpyAsync((StatsRaw*)s->pin_small + (size_t)stats_seen * 3, raw_dev, sizeof(StatsRaw) * 6, cudaMemcpyDeviceToHost, s->stream));
-                    stats_seen += 2;
-                    ++i;
-                    continue;
-                }
-            }
-            if (f->kind == F_PLANEMINMAX) {
-                rc = run_planeminmax(l, f->process, cur, 0, in2, 0, 1, f->no_thr, f->minthr, f->maxthr, f->hist_size, stats_scratch,
-                                     raw_dev, s->stream);
-            } else {
-                const int32_t* xi; const float* xf;
-                if (average_upload(f, dev_index, &xi, &xf)) return -1;
-                rc = run_planeaverage(l, f->process, cur, 0, in2, 0, 1, f->exclude_i.data(), f->exclude_f.data(),
-                                      (int)f->exclude_i.size(), xi, xf, stats_scratch, raw_dev, s->stream);
-            }
-            if (rc) return rc;
-            VSZ_CUDA(cudaMemcpyAsync((StatsRaw*)s->pin_small + (size_t)stats_seen * 3, raw_dev, sizeof(StatsRaw) * np, cudaMemcpyDeviceToHost, s->stream));
-            ++stats_seen;
+            continue;
         }
+        // a PlaneMinMax and a PlaneAverage of the same value, planes and clipb run as a pair (one read when the kernels allow it)
+        const int ne = c->fuse_next[i] ? 2 : 1;
+        for (size_t e = i; e < i + ne; ++e)
+            if (!props_out || !props_out[e]) { set_error("chain: props_out[%d] is required for a PlaneMinMax/PlaneAverage element", (int)e); return -1; }
+        const int np = processed_planes(f);
+        if (np == 0) { ++stats_seen; continue; }
+        const size_t sb = stats_scratch_bytes(1, np);
+        AsyncScratch stats_mem;
+        VSZ_CUDA(stats_mem.alloc(sb * ne, s->stream));
+        StatsRaw* raw_dev = (StatsRaw*)s->dev_small + (size_t)stats_seen * 3;
+        const int rc = ne == 2 ? run_stats_pair(f, c->fl[i + 1], dev_index, in[0], in[1], 0, 1, true, stats_mem.p, stats_mem.p + sb, raw_dev,
+                                                raw_dev + 3, s->stream, nullptr)
+                               : run_stats(f, dev_index, in[0], in[1], 0, 1, stats_mem.p, raw_dev, s->stream);
+        if (rc) return rc;
+        VSZ_CUDA(cudaMemcpyAsync((StatsRaw*)s->pin_small + (size_t)stats_seen * 3, raw_dev, sizeof(StatsRaw) * (ne == 2 ? 6 : np),
+                                 cudaMemcpyDeviceToHost, s->stream));
+        stats_seen += ne;
+        i += ne - 1;
     }
     bool direct[3] = {false, false, false};
     if (c->npixel > 0 && stage_out_begin(s, l, dst, c->written, direct)) return -1;
@@ -1336,16 +1240,11 @@ int vszip_chain_get_frame(const vszip_chain* c, int32_t n, const vszip_frame* sr
     stats_seen = 0;
     for (size_t i = 0; i < c->fl.size(); ++i) {
         const vszip_filter* f = c->fl[i];
-        if (f->kind != F_PLANEMINMAX && f->kind != F_PLANEAVERAGE) continue;
+        if (is_pixel(f)) continue;
         const StatsRaw* raw = (const StatsRaw*)s->pin_small + (size_t)stats_seen * 3;
-        if (processed_planes(f) == 0) {
-            if (f->kind == F_PLANEMINMAX) ((vszip_minmax_props*)props_out[i])->count = 0;
-            else ((vszip_average_props*)props_out[i])->count = 0;
-        } else if (f->kind == F_PLANEMINMAX) {
-            minmax_finalize(f, raw, (vszip_minmax_props*)props_out[i]);
-        } else {
-            average_finalize(f, raw, (vszip_average_props*)props_out[i]);
-        }
+        if (processed_planes(f) > 0) stats_finalize(f, raw, props_out[i], 0);
+        else if (f->kind == F_PLANEMINMAX) ((vszip_minmax_props*)props_out[i])->count = 0;
+        else ((vszip_average_props*)props_out[i])->count = 0;
         ++stats_seen;
     }
     return 0;
