@@ -262,6 +262,8 @@ class VideoFrame:
 class VideoNode:
     """A clip: format + geometry + a frame getter.  `clip.vszip.X(...)` mirrors the plugin namespace."""
 
+    _op = None  # a vszip node's _Op
+
     def __init__(self, fmt: VideoFormat, width: int, height: int, num_frames: int, getter):
         self.format, self.width, self.height, self.num_frames = fmt, width, height, num_frames
         self._getter = getter
@@ -302,7 +304,13 @@ _live_filters = weakref.WeakSet()
 
 
 class _Filter:
-    """Owns one vszip_filter handle."""
+    """Owns one vszip_filter handle.  Each filter class states how its kind runs, like the library's KindInfo table:
+    GET_FRAME is its `vszip_*_get_frame` symbol; ARGS lists that entry point's frame arguments by the chain's numbering of the
+    clips (0 = the main input, 1 = the second clip, 2 = the third), and the first of them is the clip whose frame gives the output
+    its untouched planes and its props; PROPS is the props struct a stats filter fills (None: the filter has a pixel output), DROP
+    the props it rewrites, without their prefix."""
+
+    GET_FRAME, ARGS, PROPS, DROP = None, (0,), None, ()
 
     def __init__(self, handle, node: VideoNode | None = None):
         if not handle:
@@ -312,6 +320,18 @@ class _Filter:
         load_library().vszip_filter_planes(handle, C.byref(mask))
         self.process = [bool(m) for m in mask]
         _live_filters.add(self)
+
+    def _device(self, fn, clips, first, count, stream, prop=None):
+        """One `vszip_*_device` call on `clips`, in its argument order (None: an optional clip left out), for `count` frames from
+        `first` (default: the rest of the first clip).  A stats filter returns its props, one dict per frame."""
+        count = clips[0].num_frames - first if count is None else count
+        handles = [c.handle if c else None for c in clips]
+        if self.PROPS is None:
+            _check(fn(self.handle, *handles, first, count, stream))
+            return None
+        out = (self.PROPS * max(count, 1))()
+        _check(fn(self.handle, *handles, first, count, out, stream))
+        return _props_list(self.to_props, out, count, prop)
 
     def close(self):
         """vszip_filter_free (xxxFree in the reference's glue); also called by core.shutdown() for every instance still alive."""
@@ -339,6 +359,8 @@ def _planes_arg(planes):
 
 # ---- BoxBlur
 class BoxBlurFilter(_Filter):
+    GET_FRAME = "vszip_boxblur_get_frame"
+
     def __init__(self, vi: _VideoInfo, planes=None, hradius=None, hpasses=None, vradius=None, vpasses=None):
         pl, npl = _planes_arg(planes)
         a = _BoxBlurArgs(pl, npl, hradius is not None, int(hradius or 0), hpasses is not None, int(hpasses or 0),
@@ -346,11 +368,12 @@ class BoxBlurFilter(_Filter):
         super().__init__(load_library().vszip_boxblur_create(C.byref(vi), C.byref(a)))
 
     def run_device(self, src: "DeviceClip", dst: "DeviceClip", first=0, count=None, stream=None):
-        count = src.num_frames - first if count is None else count
-        _check(load_library().vszip_boxblur_device(self.handle, src.handle, dst.handle, first, count, stream))
+        self._device(load_library().vszip_boxblur_device, (src, dst), first, count, stream)
 
 
 class BilateralFilter(_Filter):
+    GET_FRAME, ARGS = "vszip_bilateral_get_frame", (0, 1)
+
     def __init__(self, vi: _VideoInfo, ref_vi: _VideoInfo | None = None, sigmaS=None, sigmaR=None, planes=None, algorithm=None, PBFICnum=None):
         s, ns = _f64(_as_list(sigmaS) or [])
         r, nr = _f64(_as_list(sigmaR) or [])
@@ -366,8 +389,7 @@ class BilateralFilter(_Filter):
         return out
 
     def run_device(self, src, dst, ref=None, first=0, count=None, stream=None):
-        count = src.num_frames - first if count is None else count
-        _check(load_library().vszip_bilateral_device(self.handle, src.handle, ref.handle if ref else None, dst.handle, first, count, stream))
+        self._device(load_library().vszip_bilateral_device, (src, ref, dst), first, count, stream)
 
 
 def _props_from(prop, keys, count, getter):
@@ -379,7 +401,14 @@ def _props_from(prop, keys, count, getter):
     return out
 
 
+def _props_list(to_props, arr, count, prop):
+    """The props of `count` frames from an array of props structs."""
+    return [to_props(arr[i], prop) for i in range(count)]
+
+
 class PlaneMinMaxFilter(_Filter):
+    GET_FRAME, ARGS, PROPS, DROP = "vszip_planeminmax_get_frame", (0, 1), _MinMaxProps, ("Diff", "Max", "Min")
+
     def __init__(self, vi: _VideoInfo, clipb_vi: _VideoInfo | None = None, minthr=None, maxthr=None, planes=None):
         pl, npl = _planes_arg(planes)
         a = _MinMaxArgs(minthr is not None, float(minthr or 0), maxthr is not None, float(maxthr or 0), pl, npl)
@@ -398,13 +427,12 @@ class PlaneMinMaxFilter(_Filter):
         return _props_from(prop, ("Min", "Max") + (("Diff",) if p.has_diff else ()), p.count, get)
 
     def run_device(self, clipa, clipb=None, first=0, count=None, stream=None, prop="psm"):
-        count = clipa.num_frames - first if count is None else count
-        out = (_MinMaxProps * max(count, 1))()
-        _check(load_library().vszip_planeminmax_device(self.handle, clipa.handle, clipb.handle if clipb else None, first, count, out, stream))
-        return [self.to_props(out[i], prop) for i in range(count)]
+        return self._device(load_library().vszip_planeminmax_device, (clipa, clipb), first, count, stream, prop)
 
 
 class PlaneAverageFilter(_Filter):
+    GET_FRAME, ARGS, PROPS, DROP = "vszip_planeaverage_get_frame", (0, 1), _AverageProps, ("Diff", "Avg")
+
     def __init__(self, vi: _VideoInfo, clipb_vi: _VideoInfo | None = None, exclude=None, planes=None):
         pl, npl = _planes_arg(planes)
         if exclude is None:
@@ -424,10 +452,7 @@ class PlaneAverageFilter(_Filter):
         return out
 
     def run_device(self, clipa, clipb=None, first=0, count=None, stream=None, prop="psm"):
-        count = clipa.num_frames - first if count is None else count
-        out = (_AverageProps * max(count, 1))()
-        _check(load_library().vszip_planeaverage_device(self.handle, clipa.handle, clipb.handle if clipb else None, first, count, out, stream))
-        return [self.to_props(out[i], prop) for i in range(count)]
+        return self._device(load_library().vszip_planeaverage_device, (clipa, clipb), first, count, stream, prop)
 
 
 def plane_stats_device(minmax: "PlaneMinMaxFilter", average: "PlaneAverageFilter", clipa, first=0, count=None, stream=None, prop="psm", fetch=True,
@@ -446,15 +471,15 @@ def plane_stats_device(minmax: "PlaneMinMaxFilter", average: "PlaneAverageFilter
                                                         C.byref(fused), stream))
     if not fetch:
         return None, bool(fused.value)
-    out = []
-    for i in range(count):
-        p = PlaneMinMaxFilter.to_props(mm[i], prop)
-        p.update(PlaneAverageFilter.to_props(av[i], prop))
-        out.append(p)
+    out = _props_list(PlaneMinMaxFilter.to_props, mm, count, prop)
+    for p, q in zip(out, _props_list(PlaneAverageFilter.to_props, av, count, prop)):
+        p.update(q)
     return out, bool(fused.value)
 
 
 class LimiterFilter(_Filter):
+    GET_FRAME = "vszip_limiter_get_frame"
+
     def __init__(self, vi: _VideoInfo, min=None, max=None, tv_range=None, mask=None, planes=None):
         pl, npl = _planes_arg(planes)
         mn, nmn = (None, -1) if min is None else _f64(_as_list(min))
@@ -463,12 +488,13 @@ class LimiterFilter(_Filter):
         super().__init__(load_library().vszip_limiter_create(C.byref(vi), C.byref(a)))
 
     def run_device(self, src: "DeviceClip", dst: "DeviceClip", first=0, count=None, stream=None):
-        count = src.num_frames - first if count is None else count
-        _check(load_library().vszip_limiter_device(self.handle, src.handle, dst.handle, first, count, stream))
+        self._device(load_library().vszip_limiter_device, (src, dst), first, count, stream)
 
 
 class LimitFilterFilter(_Filter):
     """vszip.LimitFilter (src/vapoursynth/limit_filter.zig:93-124).  color_range: the flt clip's _ColorRange (0 full, 1 limited, None absent)."""
+
+    GET_FRAME, ARGS = "vszip_limitfilter_get_frame", (0, 1, 2)
 
     def __init__(self, flt_vi: _VideoInfo, src_vi: _VideoInfo, ref_vi: _VideoInfo | None = None, dark_thr=None, bright_thr=None, elast=None,
                  planes=None, color_range=None):
@@ -486,20 +512,21 @@ class LimitFilterFilter(_Filter):
         return {"dark_thr": list(d), "bright_thr": list(b), "elast": list(e)}
 
     def run_device(self, flt, src, dst, ref=None, first=0, count=None, stream=None):
-        count = flt.num_frames - first if count is None else count
-        _check(load_library().vszip_limitfilter_device(self.handle, flt.handle, src.handle, ref.handle if ref else None, dst.handle, first, count, stream))
+        self._device(load_library().vszip_limitfilter_device, (flt, src, ref, dst), first, count, stream)
 
 
 class AdaptiveBinarizeFilter(_Filter):
-    """vszip.AdaptiveBinarize (src/vapoursynth/adaptive_binarize.zig:79-116)."""
+    """vszip.AdaptiveBinarize (src/vapoursynth/adaptive_binarize.zig:79-116).  It filters clip2, the chain's main input; the
+    output frame is made from clip, which get_frame takes first."""
+
+    GET_FRAME, ARGS = "vszip_adaptivebinarize_get_frame", (1, 0)
 
     def __init__(self, vi: _VideoInfo, clip2_vi: _VideoInfo, c=None):
         a = _AdaptiveBinarizeArgs(c is not None, int(c or 0))
         super().__init__(load_library().vszip_adaptivebinarize_create(C.byref(vi), C.byref(clip2_vi) if clip2_vi is not None else None, C.byref(a)))
 
     def run_device(self, clip, clip2, dst, first=0, count=None, stream=None):
-        count = clip.num_frames - first if count is None else count
-        _check(load_library().vszip_adaptivebinarize_device(self.handle, clip.handle, clip2.handle, dst.handle, first, count, stream))
+        self._device(load_library().vszip_adaptivebinarize_device, (clip, clip2, dst), first, count, stream)
 
 
 class _Namespace:
@@ -516,13 +543,11 @@ class _Namespace:
 
     def BoxBlur(self, clip=None, planes=None, hradius=None, hpasses=None, vradius=None, vpasses=None) -> VideoNode:
         clip = self._c(clip)
-        flt = BoxBlurFilter(clip._info(), planes, hradius, hpasses, vradius, vpasses)
-        return _pixel_node(clip, None, flt, lambda n, s, r, d: load_library().vszip_boxblur_get_frame(flt.handle, n, C.byref(s), C.byref(d)))
+        return _node(BoxBlurFilter(clip._info(), planes, hradius, hpasses, vradius, vpasses), clip)
 
     def Limiter(self, clip=None, min=None, max=None, tv_range=None, mask=None, planes=None) -> VideoNode:
         clip = self._c(clip)
-        flt = LimiterFilter(clip._info(), min, max, tv_range, mask, planes)
-        return _pixel_node(clip, None, flt, lambda n, s, r, d: load_library().vszip_limiter_get_frame(flt.handle, n, C.byref(s), C.byref(d)))
+        return _node(LimiterFilter(clip._info(), min, max, tv_range, mask, planes), clip)
 
     def _bind(self, names, pos, kw):
         """VapourSynth binding rule: `clip.vszip.F(a, b)` puts the bound clip first and shifts the positional arguments."""
@@ -549,123 +574,79 @@ class _Namespace:
             cr = flt.get_frame(0).props.get("_ColorRange")
             if cr is not None:
                 f = LimitFilterFilter(flt._info(), src._info(), ref._info() if ref is not None else None, dark_thr, bright_thr, elast, planes, cr)
-        return _multi_node(flt, [src] + ([ref] if ref is not None else []), f, lambda n, a, others, d: load_library().vszip_limitfilter_get_frame(
-            f.handle, n, C.byref(a), C.byref(others[0]), C.byref(others[1]) if len(others) > 1 else None, C.byref(d)),
-            through=flt, extra=(src, ref))
+        return _node(f, flt, src, ref)
 
     def AdaptiveBinarize(self, *pos, **kw) -> VideoNode:
         clip, clip2, c = self._bind(("clip", "clip2", "c"), pos, kw)
         if clip is None or clip2 is None:
             raise Error("AdaptiveBinarize: clip and clip2 are required")
         f = AdaptiveBinarizeFilter(clip._info(), clip2._info(), c)
-        return _multi_node(clip, [clip2], f, lambda n, a, others, d: load_library().vszip_adaptivebinarize_get_frame(
-            f.handle, n, C.byref(a), C.byref(others[0]), C.byref(d)), {"_ColorRange": 0},  # dst_prop.setColorRange(.FULL)
-            through=clip2, extra=(clip, None))
+        return _node(f, clip2, clip, set_props={"_ColorRange": 0})  # dst_prop.setColorRange(.FULL)
 
     def Bilateral(self, clip=None, ref=None, sigmaS=None, sigmaR=None, planes=None, algorithm=None, PBFICnum=None) -> VideoNode:
         clip = self._c(clip)
         flt = BilateralFilter(clip._info(), ref._info() if ref is not None else None, sigmaS, sigmaR, planes, algorithm, PBFICnum)
-        return _pixel_node(clip, ref, flt, lambda n, s, r, d: load_library().vszip_bilateral_get_frame(
-            flt.handle, n, C.byref(s), C.byref(r) if r is not None else None, C.byref(d)))
+        return _node(flt, clip, ref)
 
     def PlaneMinMax(self, clipa=None, minthr=None, maxthr=None, clipb=None, planes=None, prop=None) -> VideoNode:
         clipa = self._c(clipa)
         flt = PlaneMinMaxFilter(clipa._info(), clipb._info() if clipb is not None else None, minthr, maxthr, planes)
-        prefix = "psm" if prop is None else str(prop)
-
-        def run(n, a, b):
-            out = _MinMaxProps()
-            _check(load_library().vszip_planeminmax_get_frame(flt.handle, n, C.byref(a), C.byref(b) if b is not None else None, C.byref(out)))
-            return PlaneMinMaxFilter.to_props(out, prefix)
-        return _props_node(clipa, clipb, flt, run, [prefix + k for k in ("Diff", "Max", "Min")], lambda o: PlaneMinMaxFilter.to_props(o, prefix))
+        return _node(flt, clipa, clipb, prefix="psm" if prop is None else str(prop))
 
     def PlaneAverage(self, clipa=None, exclude=None, clipb=None, planes=None, prop=None) -> VideoNode:
         clipa = self._c(clipa)
         flt = PlaneAverageFilter(clipa._info(), clipb._info() if clipb is not None else None, exclude, planes)
-        prefix = "psm" if prop is None else str(prop)
-
-        def run(n, a, b):
-            out = _AverageProps()
-            _check(load_library().vszip_planeaverage_get_frame(flt.handle, n, C.byref(a), C.byref(b) if b is not None else None, C.byref(out)))
-            return PlaneAverageFilter.to_props(out, prefix)
-        return _props_node(clipa, clipb, flt, run, [prefix + k for k in ("Diff", "Avg")], lambda o: PlaneAverageFilter.to_props(o, prefix))
+        return _node(flt, clipa, clipb, prefix="psm" if prop is None else str(prop))
 
 
-def _second_frame(second: VideoNode | None, n: int):
-    if second is None:
-        return None
-    return second.get_frame(min(n, second.num_frames - 1))  # rpFrameReuseLastOnly for a shorter-or-equal second clip
+@dataclass(frozen=True)
+class _Op:
+    """What a vszip node computes: the record its unfused get and the chain planner read."""
+    filter: _Filter
+    input: VideoNode              # the clip it filters: the chain's input[i]
+    second: VideoNode | None      # its second and third clips: the chain's second[i] and third[i]
+    third: VideoNode | None
+    base: VideoNode               # the clip whose frame gives the output's untouched planes and props
+    set_props: dict               # props set on every output frame
+    prefix: str                   # stats filters: the prefix of the props they write
 
+    def props(self, base_props, stats=None):
+        """The output props: the base frame's, minus the stats props this node rewrites, plus the ones it writes and sets."""
+        p = dict(base_props)
+        if stats is not None:
+            for k in self.filter.DROP:
+                p.pop(self.prefix + k, None)
+            p.update(self.filter.to_props(stats, self.prefix))
+        p.update(self.set_props)
+        return p
 
-def _pixel_node(clip: VideoNode, ref: VideoNode | None, flt: _Filter, call) -> VideoNode:
-    fmt = clip.format
-
-    def get(n):
+    def get(self, n):
+        """Unfused evaluation: the filter's get_frame on frame n of each input; an extra clip that is shorter repeats its last
+        frame (rpFrameReuseLastOnly).  Inputs pass their processed planes; a pixel filter's output gets fresh processed planes
+        and shares the others with the base frame (newVideoFrame2), a stats filter's shares every plane (copyFrame)."""
         core._ensure_init()
-        src = clip.get_frame(n)
-        rf = _second_frame(ref, n)
-        # newVideoFrame2(planes): processed planes are fresh, the others are shared with the source
-        out_planes = [np.empty_like(p, order="C") if flt.process[i] else p for i, p in enumerate(src.planes)]
-        s = _cframe([_rows(p) if flt.process[i] else None for i, p in enumerate(src.planes)])
-        keep = [_rows(p) for p in rf.planes] if rf is not None else None
-        r = _cframe(keep) if rf is not None else None
-        d = _cframe([p if flt.process[i] else None for i, p in enumerate(out_planes)])
-        _check(call(n, s, r, d))
-        return VideoFrame(fmt, clip.width, clip.height, out_planes, src.props)
-
-    node = VideoNode(fmt, clip.width, clip.height, clip.num_frames, get)
-    node.filter = flt
-    node._chain_info = ("pixel", clip, ref, None)
-    node._extra = (ref, None)
-    node._props_of = clip
-    return node
+        flt, clips = self.filter, (self.input, self.second, self.third)
+        frames = [None if clips[i] is None else clips[i].get_frame(min(n, clips[i].num_frames - 1)) for i in flt.ARGS]
+        base = frames[0]
+        args = [None if fr is None else C.byref(_cframe([_rows(p) if flt.process[i] else None for i, p in enumerate(fr.planes)]))
+                for fr in frames]
+        if flt.PROPS is None:
+            planes = [np.empty_like(p, order="C") if flt.process[i] else p for i, p in enumerate(base.planes)]
+            stats, out = None, _cframe([p if flt.process[i] else None for i, p in enumerate(planes)])
+        else:
+            planes = base.planes
+            stats = out = flt.PROPS()
+        _check(getattr(load_library(), flt.GET_FRAME)(flt.handle, n, *args, C.byref(out)))
+        return VideoFrame(base.format, base.width, base.height, planes, self.props(base.props, stats))
 
 
-def _multi_node(first: VideoNode, others, flt: _Filter, call, set_props=None, through=None, extra=(None, None)) -> VideoNode:
-    """A pixel filter with several input clips (LimitFilter, AdaptiveBinarize): dst is allocated from `first`."""
-    fmt = first.format
-
-    def get(n):
-        core._ensure_init()
-        src = first.get_frame(n)
-        ofr = [_second_frame(o, n) for o in others]
-        out_planes = [np.empty_like(p, order="C") if flt.process[i] else p for i, p in enumerate(src.planes)]
-        keep = [[_rows(p) if flt.process[i] else None for i, p in enumerate(fr.planes)] for fr in [src] + ofr]
-        d = _cframe([p if flt.process[i] else None for i, p in enumerate(out_planes)])
-        _check(call(n, _cframe(keep[0]), [_cframe(k) for k in keep[1:]], d))
-        props = dict(src.props)
-        props.update(set_props or {})
-        return VideoFrame(fmt, first.width, first.height, out_planes, props)
-
-    node = VideoNode(fmt, first.width, first.height, first.num_frames, get)
-    node.filter = flt
-    # in a fused chain `through` is the input the filter works on (the chain's main line), `extra` its second / third clips
-    node._chain_info = ("pixel", through, None, None)
-    node._extra = tuple(extra)
-    node._set_props = set_props
-    node._props_of = first                       # dst = first.newVideoFrame(): props of `first` only
-    return node
-
-
-def _props_node(clipa: VideoNode, clipb: VideoNode | None, flt: _Filter, run, drop_keys, run_fused=None) -> VideoNode:
-    def get(n):
-        core._ensure_init()
-        src = clipa.get_frame(n)
-        bf = _second_frame(clipb, n)
-        a = _cframe([_rows(p) if flt.process[i] else None for i, p in enumerate(src.planes)])
-        keep = [_rows(p) for p in bf.planes] if bf is not None else None
-        b = _cframe(keep) if bf is not None else None
-        props = dict(src.props)                      # copyFrame: pixels shared, props copied
-        for k in drop_keys:
-            props.pop(k, None)
-        props.update(run(n, a, b))
-        return VideoFrame(src.format, src.width, src.height, src.planes, props)
-
-    node = VideoNode(clipa.format, clipa.width, clipa.height, clipa.num_frames, get)
-    node.filter = flt
-    node._chain_info = ("props", clipa, clipb, (run_fused, drop_keys))
-    node._extra = (clipb, None)
-    node._props_of = clipa
+def _node(flt: _Filter, main: VideoNode, second: VideoNode | None = None, third: VideoNode | None = None, set_props=None,
+          prefix="") -> VideoNode:
+    """A vszip node on `main`, `second` and `third` (the chain's numbering)."""
+    base = (main, second, third)[flt.ARGS[0]]
+    op = _Op(flt, main, second, third, base, set_props or {}, prefix)
+    node = VideoNode(base.format, base.width, base.height, base.num_frames, op.get)
+    node.filter, node._op = flt, op
     return node
 
 
@@ -698,9 +679,9 @@ def _fusable_chain(node: "VideoNode"):
     if cached is not False:
         return cached
     main, cur = [], node
-    while getattr(cur, "_chain_info", None) is not None and len(main) < 16:
+    while cur._op is not None and len(main) < 16:
         main.append(cur)
-        cur = cur._chain_info[1]
+        cur = cur._op.input
     node._chain = _plan_chain(main[::-1], cur)
     return node._chain
 
@@ -708,8 +689,8 @@ def _fusable_chain(node: "VideoNode"):
 def _side_input(x, value):
     """A single-input pixel node that is not on the main line but filters a value of the chain (`src.vszip.BoxBlur()` given as
     ref / clipb): it joins the chain right before its reader."""
-    return getattr(x, "_chain_info", None) is not None and x._chain_info[0] == "pixel" and not any(
-        e is not None for e in x._extra) and value(x._chain_info[1]) is not None
+    op = x._op
+    return op is not None and op.filter.PROPS is None and op.second is None and op.third is None and value(op.input) is not None
 
 
 def _plan_chain(main, source):
@@ -720,7 +701,7 @@ def _plan_chain(main, source):
         value = lambda x: vals.get(id(x))
         for k, nd in enumerate(main):
             side = []
-            for x in nd._extra:
+            for x in (nd._op.second, nd._op.third):
                 if x is None or value(x) is not None or any(x is y for y in side):
                     continue
                 if not _side_input(x, value):
@@ -731,7 +712,7 @@ def _plan_chain(main, source):
                 break
             for x in side + [nd]:
                 elems.append(x)
-                vals[id(x)] = len(elems) if x._chain_info[0] == "pixel" else value(x._chain_info[1])  # stats pass their input on
+                vals[id(x)] = len(elems) if x._op.filter.PROPS is None else value(x._op.input)  # stats pass their input on
         if cut is not None:
             source, main = main[cut], main[cut + 1:]
         elif len(elems) > 16:
@@ -740,8 +721,9 @@ def _plan_chain(main, source):
             break
     if not main or len(elems) < 2:
         return None
-    inputs = [value(x._chain_info[1]) for x in elems]
-    second, third = ([-1 if x._extra[j] is None else value(x._extra[j]) for x in elems] for j in (0, 1))
+    inputs = [value(x._op.input) for x in elems]
+    second = [-1 if x._op.second is None else value(x._op.second) for x in elems]
+    third = [-1 if x._op.third is None else value(x._op.third) for x in elems]
     return _Chain(elems, inputs, second, third), source
 
 
@@ -754,24 +736,16 @@ def _fused_get(chain_and_source, n: int) -> "VideoFrame":
     d = _cframe([p if chain.written[i] else None for i, p in enumerate(out_planes)])
     outs, ptrs = [], (_P * len(chain.nodes))()
     for i, nd in enumerate(chain.nodes):
-        kind = nd._chain_info[0]
         o = None
-        if kind == "props":
-            o = _MinMaxProps() if isinstance(nd.filter, PlaneMinMaxFilter) else _AverageProps()
+        if nd._op.filter.PROPS is not None:
+            o = nd._op.filter.PROPS()
             ptrs[i] = C.cast(C.pointer(o), _P)
         outs.append(o)
     _check(load_library().vszip_chain_get_frame(chain.handle, n, C.byref(s), C.byref(d), ptrs))
     # every node's props, in evaluation order, exactly as the unfused nodes derive them from the clip their frame comes from
-    props = {id(source): dict(src.props)}
+    props = {id(source): src.props}
     for nd, o in zip(chain.nodes, outs):
-        p = dict(props[id(nd._props_of)])
-        if o is not None:
-            to_props, drop_keys = nd._chain_info[3]
-            for k in drop_keys:
-                p.pop(k, None)
-            p.update(to_props(o))
-        p.update(getattr(nd, "_set_props", None) or {})
-        props[id(nd)] = p
+        props[id(nd)] = nd._op.props(props[id(nd._op.base)], o)
     return VideoFrame(source.format, source.width, source.height, out_planes, props[id(chain.nodes[-1])])
 
 
