@@ -5,7 +5,7 @@ NVFLAGS := $(ARCH) -O3 -std=c++17 -lineinfo -fmad=false -Xcompiler -fPIC,-Wall,-
 SRC_DIR := vapoursynth_zip_b200/csrc
 OBJ_DIR := build/obj
 LIB := vapoursynth_zip_b200/lib/libvszip_cuda.so
-SRCS := runtime.cu filters.cu boxblur_kernels.cu boxblur_seg_h.cu boxblur_seg_v.cu boxblur_seg_ct.cu boxblur_ctf.cu bilateral_kernels.cu pbfic_kernels.cu planestats_kernels.cu pointwise_kernels.cu
+SRCS := runtime.cu filters.cu boxblur_kernels.cu boxblur_seg_h.cu boxblur_seg_v.cu boxblur_seg_ct.cu boxblur_ctf.cu bilateral_kernels.cu pbfic_kernels.cu planestats_kernels.cu pointwise_kernels.cu clahe_kernels.cu
 HOST_SRCS := host_copy.cpp
 OBJS := $(SRCS:%.cu=$(OBJ_DIR)/%.o) $(HOST_SRCS:%.cpp=$(OBJ_DIR)/%.o)
 CXX ?= g++

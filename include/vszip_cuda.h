@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define VSZIP_CUDA_ABI_VERSION 5  /* 2: + vszip_chain_*, vszip_limiter_*; 3: + vszip_limitfilter_*, vszip_adaptivebinarize_*, vszip_planestats_device; 4: + vszip_cuda_host_forget, vszip_cuda_host_registered_bytes, vszip_cuda_host_register_limit; 5: + vszip_cuda_reserve, and additions that leave every earlier entry point unchanged: vszip_chain_create2, vszip_planestats_device_b, vszip_cuda_transfer_bytes (a caller that needs them resolves them by name) */
+#define VSZIP_CUDA_ABI_VERSION 5  /* 2: + vszip_chain_*, vszip_limiter_*; 3: + vszip_limitfilter_*, vszip_adaptivebinarize_*, vszip_planestats_device; 4: + vszip_cuda_host_forget, vszip_cuda_host_registered_bytes, vszip_cuda_host_register_limit; 5: + vszip_cuda_reserve, and additions that leave every earlier entry point unchanged: vszip_chain_create2, vszip_planestats_device_b, vszip_cuda_transfer_bytes, vszip_clahe_create, vszip_clahe_get_frame, vszip_clahe_device (a caller that needs them resolves them by name) */
 
 /* VapourSynth4.h values (VSColorFamily / VSSampleType) so the Zig glue can pass vi.format as is. */
 enum { VSZIP_CF_GRAY = 1, VSZIP_CF_RGB = 2, VSZIP_CF_YUV = 3 };
@@ -236,6 +236,19 @@ vszip_filter* vszip_adaptivebinarize_create(const vszip_video_info* vi, const vs
 int vszip_adaptivebinarize_get_frame(const vszip_filter* f, int32_t n, const vszip_frame* clip, const vszip_frame* clip2,
                                      vszip_frame* dst);
 
+/* ------------------------------------------------------------------ CLAHE
+ * Contrast-limited adaptive histogram equalisation of every plane of an 8..16-bit integer clip, bit-exact with OpenCV's
+ * cv::createCLAHE(limit, (tiles[0], tiles[1])).apply on each plane (histogram size 2^bits; samples above 2^bits - 1 count as
+ * 2^bits - 1).  Argument string: "clip:vnode;limit:float:opt;tiles:int[]:opt;".  has_limit == 0: limit 15; num_tiles == 0:
+ * tiles [3, 3]; one value applies to both axes.  limit >= 0 (0: no clipping), every tile count >= 1, tiles[0] * tiles[1] <= 256.
+ * The names, defaults and messages are this library's (the reference's source is not part of this tree). */
+typedef struct vszip_clahe_args {
+    int32_t has_limit; double limit;
+    const int64_t* tiles; int32_t num_tiles;
+} vszip_clahe_args;
+vszip_filter* vszip_clahe_create(const vszip_video_info* vi, const vszip_clahe_args* args);
+int vszip_clahe_get_frame(const vszip_filter* f, int32_t n, const vszip_frame* src, vszip_frame* dst);
+
 /* ------------------------------------------------------------------ common filter calls */
 void vszip_filter_free(vszip_filter* f);                         /* replaces xxxFree */
 int vszip_filter_planes(const vszip_filter* f, int32_t process[3]); /* d.planes after create */
@@ -294,6 +307,8 @@ int vszip_limitfilter_device(const vszip_filter* f, const vszip_dev_clip* flt, c
                              const vszip_dev_clip* ref, vszip_dev_clip* dst, int32_t first, int32_t count, void* stream);
 int vszip_adaptivebinarize_device(const vszip_filter* f, const vszip_dev_clip* clip, const vszip_dev_clip* clip2,
                                   vszip_dev_clip* dst, int32_t first, int32_t count, void* stream);
+int vszip_clahe_device(const vszip_filter* f, const vszip_dev_clip* src, vszip_dev_clip* dst,
+                       int32_t first, int32_t count, void* stream);
 int vszip_cuda_stream_sync(int32_t device, void* stream);
 
 /* ------------------------------------------------------------------ fused chains of vszip filters (SURVEY 8f rank 1)

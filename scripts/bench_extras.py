@@ -1,6 +1,7 @@
 """Secondary measurements: the other BASELINE.json configs, device-resident, CUDA-event timed.
 Not the contract line (bench.py prints that); results go to stdout as JSON and, with --out, to a file.
-usage: python scripts/bench_extras.py [--frames N] [--reps R] [--only REGEX] [--out profiles/bench_extras_rXX.json]"""
+usage: python scripts/bench_extras.py [--frames N] [--reps R] [--only REGEX] [--out profiles/bench_extras_rXX.json]
+--only clahe: the CLAHE group (device batches, get_frame on pinned frames, and OpenCV on every host core for comparison)."""
 import argparse
 import json
 import sys
@@ -113,17 +114,23 @@ multi_cfg("C7 LimitFilter(flt, src, dark_thr=8, bright_thr=8, elast=3) (8f rank 
           lambda c: _lf.setdefault("a", vz.LimitFilterFilter(c[0].info(), c[0].info(), None, dark_thr=8, bright_thr=8, elast=3)).run_device(c[0], c[1], c[2], count=N, stream=st.cuda_stream))
 multi_cfg("C7 LimitFilter(flt, src, ref, ...) three inputs", "YUV420P16", 1920, 1080, N, 3,
           lambda c: _lf.setdefault("b", vz.LimitFilterFilter(c[0].info(), c[0].info(), c[0].info(), dark_thr=8, bright_thr=8, elast=3)).run_device(c[0], c[1], c[3], ref=c[2], count=N, stream=st.cuda_stream))
+def _smooth_noise(dst):
+    """noise smoothed by BoxBlur(13, 3 passes): image-like gradients"""
+    tmp = vz.DeviceClip(dst.format, dst.width, dst.height, dst.num_frames)
+    tmp.fill_noise(99)
+    vz.BoxBlurFilter(tmp.info(), hradius=13, hpasses=3, vradius=13, vpasses=3).run_device(tmp, dst, stream=st.cuda_stream)
+    torch.cuda.synchronize()
+    tmp.free()
+
+
 def _image_like(c):
     """src = noise smoothed by BoxBlur(13, 3 passes) (image-like gradients), flt = BoxBlur(src, 2), ref = BoxBlur(src, 4):
     the reference's own LimitFilter usage (tests/test_int_parity.py:158-167)"""
-    tmp = vz.DeviceClip("YUV420P16", 1920, 1080, c[0].num_frames)
-    tmp.fill_noise(99)
-    vz.BoxBlurFilter(tmp.info(), hradius=13, hpasses=3, vradius=13, vpasses=3).run_device(tmp, c[1], stream=st.cuda_stream)   # src
-    vz.BoxBlurFilter(tmp.info(), hradius=2, vradius=2).run_device(c[1], c[0], stream=st.cuda_stream)                             # flt
+    _smooth_noise(c[1])                                                                                                         # src
+    vz.BoxBlurFilter(c[1].info(), hradius=2, vradius=2).run_device(c[1], c[0], stream=st.cuda_stream)                           # flt
     if len(c) > 3:
-        vz.BoxBlurFilter(tmp.info(), hradius=4, vradius=4).run_device(c[1], c[2], stream=st.cuda_stream)                         # ref
+        vz.BoxBlurFilter(c[1].info(), hradius=4, vradius=4).run_device(c[1], c[2], stream=st.cuda_stream)                       # ref
     torch.cuda.synchronize()
-    tmp.free()
 
 
 multi_cfg("C7' LimitFilter(flt=BoxBlur(src,2), src, dark_thr=1, bright_thr=1, elast=2) image-like content", "YUV420P16", 1920, 1080, N, 2,
@@ -163,7 +170,87 @@ both_stats_cfg("GRAYS", 3840, 2160, M, dict(minthr=0.1, maxthr=0.1), [0, 1])
 K = max(4, N // 16)
 pixel_cfg("C5a BoxBlur(13,1,13,1) YUV444PS 4K (comptime float)", "YUV444PS", 3840, 2160, K, lambda s: vz.BoxBlurFilter(s.info(), hradius=13, vradius=13))
 pixel_cfg("C5b Bilateral(2,2) YUV444PS 4K", "YUV444PS", 3840, 2160, K, lambda s: vz.BilateralFilter(s.info(), sigmaS=2, sigmaR=2))
-out = {"peak_GBps": PEAK, "results": results}
+
+
+def _cv2_clahe(job):
+    import cv2
+    cv2.setNumThreads(1)
+    planes, limit, tiles = job
+    c = cv2.createCLAHE(limit, tiles)
+    return [c.apply(p) for p in planes]
+
+
+def clahe_cfgs():
+    """Device-resident batches (frames/s, read-once-write-once GB/s), get_frame on pinned host frames from 8 threads, and OpenCV's
+    CPU CLAHE on the same frames over every host core (one frame per worker, one OpenCV thread per worker) for comparison."""
+    import ctypes as C
+    import multiprocessing
+    import os
+    import time
+    from concurrent.futures import ProcessPoolExecutor, ThreadPoolExecutor
+
+    lib = vz.load_library()
+    for fmt, w, h in (("YUV420P8", 1920, 1080), ("YUV420P16", 1920, 1080), ("GRAY16", 3840, 2160)):
+        frames = N if fmt == "YUV420P8" else max(8, N // 4)
+        for content in ("noise", "image-like"):
+            tag = f"clahe {fmt} {w}x{h} {content}"
+            if skip(tag):
+                continue
+            src, dst = vz.DeviceClip(fmt, w, h, frames), vz.DeviceClip(fmt, w, h, frames)
+            if content == "noise":
+                src.fill_noise(1234)
+            else:
+                _smooth_noise(src)
+            host = [src.download(i) for i in range(4)]
+            for tiles in ([3, 3], [8, 8]):
+                f = vz.CLAHEFilter(src.info(), limit=15, tiles=tiles)
+                ms = timed(lambda: f.run_device(src, dst, first=0, count=frames, stream=st.cuda_stream), args.reps)
+                record(f"{tag} limit=15 tiles={tiles} device batch", fmt, w, h, frames, 2 * src.frame_bytes, ms)
+                # get_frame: page-locked host planes, 8 requests in flight on one handle
+                def pinned(a):
+                    t = torch.empty(a.nbytes, dtype=torch.uint8, pin_memory=True)
+                    return t.numpy().view(a.dtype).reshape(a.shape), t
+                ins = [[pinned(p) for p in fr] for fr in host]
+                for fr, pf in zip(host, ins):
+                    for p, (q, _) in zip(fr, pf):
+                        q[...] = p
+                outs = [[pinned(p) for p in fr] for fr in host for _ in range(2)]
+                def one(i):
+                    s = vz._cframe([q for q, _ in ins[i % 4]])
+                    d = vz._cframe([q for q, _ in outs[i % 8]])
+                    vz._check(lib.vszip_clahe_get_frame(f.handle, i, C.byref(s), C.byref(d)))
+                n_e2e = 4 * frames
+                with ThreadPoolExecutor(8) as ex:
+                    list(ex.map(one, range(16)))
+                    t0 = time.perf_counter()
+                    list(ex.map(one, range(n_e2e)))
+                    e2e = time.perf_counter() - t0
+                record(f"{tag} limit=15 tiles={tiles} get_frame, pinned frames, 8 threads (end to end)", fmt, w, h, n_e2e,
+                       2 * src.frame_bytes, e2e * 1e3)
+                workers = os.cpu_count() or 1
+                n_cpu = 2 * workers
+                with ProcessPoolExecutor(workers, mp_context=multiprocessing.get_context("fork")) as ex:
+                    list(ex.map(_cv2_clahe, [(host[0], 15.0, tuple(tiles))] * workers))
+                    t0 = time.perf_counter()
+                    list(ex.map(_cv2_clahe, [(host[i % 4], 15.0, tuple(tiles)) for i in range(n_cpu)]))
+                    cpu = time.perf_counter() - t0
+                record(f"{tag} limit=15 tiles={tiles} OpenCV 4.13, not the reference: cv2.createCLAHE on {workers} host cores",
+                       fmt, w, h, n_cpu, 2 * src.frame_bytes, cpu * 1e3)
+            src.free(); dst.free()
+
+
+clahe_cfgs()
+
+
+def _gpu():
+    """the card the numbers were measured on, read in the same run"""
+    import subprocess
+    q = subprocess.run(["nvidia-smi", "-i", "0", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
+                       capture_output=True, text=True).stdout.strip()
+    return {"torch_name": torch.cuda.get_device_name(0), "nvidia_smi": q}
+
+
+out = {"peak_GBps": PEAK, "gpu": _gpu(), "results": results}
 print(json.dumps(out))
 if args.out:
     Path(args.out).write_text(json.dumps(out, indent=1) + "\n")

@@ -2,7 +2,7 @@
 
 The product is the C-ABI library (include/vszip_cuda.h, built into lib/libvszip_cuda.so from
 csrc/*.cu).  This module is the thin host side used where the reference would be driven through
-VapourSynth: it mirrors the `clip.vszip.BoxBlur / Bilateral / PlaneMinMax / PlaneAverage` call
+VapourSynth: it mirrors the `clip.vszip.BoxBlur / Bilateral / PlaneMinMax / PlaneAverage / ... / CLAHE` call
 surface (same names, arguments, defaults, frame props and error messages; src/vszip.zig:46-69,
 :184-199) on top of a minimal clip/frame model, so the parity tests read like the reference's own
 tests (tests/test_boxblur.py etc. of the reference).  All arithmetic happens in the CUDA library;
@@ -89,6 +89,10 @@ class _AdaptiveBinarizeArgs(C.Structure):
     _fields_ = [("has_c", C.c_int32), ("c", C.c_int64)]
 
 
+class _ClaheArgs(C.Structure):
+    _fields_ = [("has_limit", C.c_int32), ("limit", C.c_double), ("tiles", C.POINTER(C.c_int64)), ("num_tiles", C.c_int32)]
+
+
 class _AverageProps(C.Structure):
     _fields_ = [("count", C.c_int32), ("plane", C.c_int32 * 3), ("has_diff", C.c_int32), ("avg", C.c_double * 3), ("diff", C.c_double * 3)]
 
@@ -143,6 +147,9 @@ ABI = {
     "vszip_adaptivebinarize_create": (_P, [C.POINTER(_VideoInfo), C.POINTER(_VideoInfo), C.POINTER(_AdaptiveBinarizeArgs)]),
     "vszip_adaptivebinarize_get_frame": (C.c_int, [_P, C.c_int32, C.POINTER(_Frame), C.POINTER(_Frame), C.POINTER(_Frame)]),
     "vszip_adaptivebinarize_device": (C.c_int, [_P, _P, _P, _P, C.c_int32, C.c_int32, _P]),
+    "vszip_clahe_create": (_P, [C.POINTER(_VideoInfo), C.POINTER(_ClaheArgs)]),
+    "vszip_clahe_get_frame": (C.c_int, [_P, C.c_int32, C.POINTER(_Frame), C.POINTER(_Frame)]),
+    "vszip_clahe_device": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int32, _P]),
     "vszip_chain_create": (_P, [C.POINTER(_P), C.c_int32]),
     "vszip_chain_create2": (_P, [C.POINTER(_P), C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "vszip_chain_free": (None, [_P]),
@@ -529,6 +536,20 @@ class AdaptiveBinarizeFilter(_Filter):
         self._device(load_library().vszip_adaptivebinarize_device, (clip, clip2, dst), first, count, stream)
 
 
+class CLAHEFilter(_Filter):
+    """Contrast-limited adaptive histogram equalisation of every plane, bit-exact with OpenCV's CLAHE::apply (DESIGN.md §4.7)."""
+
+    GET_FRAME = "vszip_clahe_get_frame"
+
+    def __init__(self, vi: _VideoInfo, limit=None, tiles=None):
+        t, nt = _i64(_as_list(tiles) or [])
+        a = _ClaheArgs(limit is not None, float(limit or 0), t, nt)
+        super().__init__(load_library().vszip_clahe_create(C.byref(vi), C.byref(a)))
+
+    def run_device(self, src: "DeviceClip", dst: "DeviceClip", first=0, count=None, stream=None):
+        self._device(load_library().vszip_clahe_device, (src, dst), first, count, stream)
+
+
 class _Namespace:
     """`clip.vszip` / `core.vszip`: the plugin functions with the reference's argument names."""
 
@@ -548,6 +569,12 @@ class _Namespace:
     def Limiter(self, clip=None, min=None, max=None, tv_range=None, mask=None, planes=None) -> VideoNode:
         clip = self._c(clip)
         return _node(LimiterFilter(clip._info(), min, max, tv_range, mask, planes), clip)
+
+    def CLAHE(self, *pos, **kw) -> VideoNode:
+        clip, limit, tiles = self._bind(("clip", "limit", "tiles"), pos, kw)
+        if clip is None:
+            raise Error("clip argument is required")
+        return _node(CLAHEFilter(clip._info(), limit, tiles), clip)
 
     def _bind(self, names, pos, kw):
         """VapourSynth binding rule: `clip.vszip.F(a, b)` puts the bound clip first and shifts the positional arguments."""

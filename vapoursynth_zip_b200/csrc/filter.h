@@ -1,4 +1,4 @@
-// filter.h — the immutable per-instance data of the seven filters (the CUDA-side twin of the
+// filter.h — the immutable per-instance data of the eight filters (the CUDA-side twin of the
 // reference's `Data` structs) and the kernel launchers each filter uses.
 #pragma once
 
@@ -6,7 +6,8 @@
 
 namespace vsz {
 
-enum FilterKind { F_BOXBLUR = 1, F_BILATERAL = 2, F_PLANEMINMAX = 3, F_PLANEAVERAGE = 4, F_LIMITER = 5, F_LIMITFILTER = 6, F_ADAPTIVEBINARIZE = 7 };
+enum FilterKind { F_BOXBLUR = 1, F_BILATERAL = 2, F_PLANEMINMAX = 3, F_PLANEAVERAGE = 4, F_LIMITER = 5, F_LIMITFILTER = 6, F_ADAPTIVEBINARIZE = 7,
+                  F_CLAHE = 8 };
 
 struct BilateralPlane {
     double sigmaS = 0, sigmaR = 0;
@@ -58,6 +59,10 @@ struct vszip_filter {
     float lf_dark[3], lf_bright[3], lf_elast[3];
     // AdaptiveBinarize (src/vapoursynth/adaptive_binarize.zig:14-19)
     int ab_c;
+    // CLAHE (DESIGN.md §4.7): clip limit, tiles along x / y, histogram size 2^bits
+    double clahe_limit;
+    int clahe_tiles[2];
+    int clahe_hs;
 };
 
 namespace vsz {
@@ -105,6 +110,11 @@ int run_limitfilter(const FrameLayout& l, const bool mask[3], const char* flt, s
                     const float elast[3], cudaStream_t st);
 int run_adaptivebinarize(const FrameLayout& l, const char* a, size_t a_fs, const char* b, size_t b_fs, char* dst, size_t dst_fs, int count,
                          int c, cudaStream_t st);
+
+// clahe_kernels.cu: every processed plane of an 8..16-bit integer clip; hs = 2^bits, limit >= 0 (0: no clipping), tx * ty tiles.
+// Scratch for the histograms and LUTs comes from the stream-ordered pool.
+int run_clahe(const FrameLayout& l, const bool mask[3], const char* src, size_t src_fs, char* dst, size_t dst_fs, int count, int hs,
+              double limit, int tx, int ty, cudaStream_t st);
 
 // planestats_kernels.cu
 struct StatsRaw {  // one per (frame, processed plane), written by the kernels

@@ -195,8 +195,9 @@ constexpr KindInfo kKinds[] = {
     {"Limiter", true, {nullptr, nullptr}, {false, false}},
     {"LimitFilter", true, {"src", "ref"}, {false, true}},
     {"AdaptiveBinarize", true, {"clip", nullptr}, {false, false}},
+    {"CLAHE", true, {nullptr, nullptr}, {false, false}},
 };
-static_assert(sizeof kKinds / sizeof kKinds[0] == F_ADAPTIVEBINARIZE, "one row per FilterKind");
+static_assert(sizeof kKinds / sizeof kKinds[0] == F_CLAHE, "one row per FilterKind");
 
 const KindInfo& kind_info(int kind) { return kKinds[kind - 1]; }
 bool is_pixel(const vszip_filter* f) { return kind_info(f->kind).pixel; }
@@ -752,6 +753,8 @@ static int run_pixels(const vszip_filter* f, int dev_index, const char* const in
             return run_limiter(l, f->process, in[0], fs, out, fs, count, f->lim_lo, f->lim_hi, st);
         case F_LIMITFILTER:  // flt = the main input, src = the second, ref = the third
             return run_limitfilter(l, f->process, in[0], fs, in[1], fs, in[2], fs, out, fs, count, f->lf_dark, f->lf_bright, f->lf_elast, st);
+        case F_CLAHE:
+            return run_clahe(l, f->process, in[0], fs, out, fs, count, f->clahe_hs, f->clahe_limit, f->clahe_tiles[0], f->clahe_tiles[1], st);
         default:  // AdaptiveBinarize: clip = the second input, clip2 = the main one
             return run_adaptivebinarize(l, in[1], fs, in[0], fs, out, fs, count, f->ab_c, st);
     }
@@ -1027,6 +1030,47 @@ int vszip_adaptivebinarize_get_frame(const vszip_filter* f, int32_t n, const vsz
 int vszip_adaptivebinarize_device(const vszip_filter* f, const vszip_dev_clip* clip, const vszip_dev_clip* clip2, vszip_dev_clip* dst,
                                   int32_t first, int32_t count, void* stream) {
     return pixel_device(f, F_ADAPTIVEBINARIZE, {clip2, clip, nullptr}, dst, first, count, stream);
+}
+
+// =========================================================================== CLAHE
+// OpenCV's CLAHE::apply on every plane (DESIGN.md §4.7).  The argument names, defaults and messages are this library's.
+vszip_filter* vszip_clahe_create(const vszip_video_info* vi, const vszip_clahe_args* a) {
+    static const char* name = "CLAHE";
+    if (!basic_vi_ok(vi, name)) return nullptr;
+    if (vi->sample_type != VSZIP_ST_INTEGER || vi->bits_per_sample < 8 || vi->bits_per_sample > 16) {
+        set_error("CLAHE: only 8-16 bit int formats supported.");
+        return nullptr;
+    }
+    SampleKind kind;
+    if (!select_kind(*vi, name, false, &kind)) return nullptr;
+    const double limit = a && a->has_limit ? a->limit : 15.0;
+    if (!(limit >= 0)) { set_error("CLAHE: limit must be non-negative."); return nullptr; }
+    const int n = a && a->tiles ? std::max(a->num_tiles, 0) : 0;
+    if (n > 2) { set_error("CLAHE: tiles has too many elements (got %d, max 2).", n); return nullptr; }
+    int64_t t[2] = {3, 3};
+    if (n >= 1) t[0] = t[1] = a->tiles[0];
+    if (n == 2) t[1] = a->tiles[1];
+    if (t[0] < 1 || t[1] < 1) { set_error("CLAHE: tiles values must be at least 1."); return nullptr; }
+    if (t[0] > 256 || t[1] > 256 || t[0] * t[1] > 256) { set_error("CLAHE: at most 256 tiles per plane (tiles[0] * tiles[1])."); return nullptr; }
+    vszip_filter* f = new vszip_filter();
+    f->kind = F_CLAHE;
+    f->vi = *vi;
+    f->sample = kind;
+    f->layout = make_layout(*vi, kind);
+    for (int i = 0; i < 3; ++i) f->process[i] = i < vi->num_planes;
+    f->clahe_limit = limit;
+    f->clahe_tiles[0] = (int)t[0];
+    f->clahe_tiles[1] = (int)t[1];
+    f->clahe_hs = 1 << vi->bits_per_sample;
+    return f;
+}
+
+int vszip_clahe_get_frame(const vszip_filter* f, int32_t n, const vszip_frame* src, vszip_frame* dst) {
+    return pixel_get_frame(f, F_CLAHE, n, {src, nullptr, nullptr}, dst);
+}
+
+int vszip_clahe_device(const vszip_filter* f, const vszip_dev_clip* src, vszip_dev_clip* dst, int32_t first, int32_t count, void* stream) {
+    return pixel_device(f, F_CLAHE, {src, nullptr, nullptr}, dst, first, count, stream);
 }
 
 // =========================================================================== fused chains
