@@ -9,7 +9,7 @@ SRCS := runtime.cu filters.cu boxblur_kernels.cu boxblur_seg_h.cu boxblur_seg_v.
 HOST_SRCS := host_copy.cpp
 OBJS := $(SRCS:%.cu=$(OBJ_DIR)/%.o) $(HOST_SRCS:%.cpp=$(OBJ_DIR)/%.o)
 CXX ?= g++
-HDRS := include/vszip_cuda.h $(SRC_DIR)/common.h $(SRC_DIR)/filter.h $(SRC_DIR)/boxblur_seg_core.h $(SRC_DIR)/boxblur_seg.cuh
+HDRS := include/vszip_cuda.h $(SRC_DIR)/common.h $(SRC_DIR)/filter.h $(SRC_DIR)/boxblur_seg_core.h $(SRC_DIR)/boxblur_seg.cuh $(SRC_DIR)/colormap_tables.h
 
 all: $(LIB) oracle
 

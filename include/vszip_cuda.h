@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define VSZIP_CUDA_ABI_VERSION 5  /* 2: + vszip_chain_*, vszip_limiter_*; 3: + vszip_limitfilter_*, vszip_adaptivebinarize_*, vszip_planestats_device; 4: + vszip_cuda_host_forget, vszip_cuda_host_registered_bytes, vszip_cuda_host_register_limit; 5: + vszip_cuda_reserve, and additions that leave every earlier entry point unchanged: vszip_chain_create2, vszip_planestats_device_b, vszip_cuda_transfer_bytes, vszip_clahe_create, vszip_clahe_get_frame, vszip_clahe_device (a caller that needs them resolves them by name) */
+#define VSZIP_CUDA_ABI_VERSION 5  /* 2: + vszip_chain_*, vszip_limiter_*; 3: + vszip_limitfilter_*, vszip_adaptivebinarize_*, vszip_planestats_device; 4: + vszip_cuda_host_forget, vszip_cuda_host_registered_bytes, vszip_cuda_host_register_limit; 5: + vszip_cuda_reserve, and additions that leave every earlier entry point unchanged: vszip_chain_create2, vszip_planestats_device_b, vszip_cuda_transfer_bytes, vszip_clahe_create, vszip_clahe_get_frame, vszip_clahe_device, vszip_colormap_create, vszip_colormap_get_frame, vszip_colormap_device, vszip_colormap_get_lut, vszip_filter_output_info (a caller that needs them resolves them by name) */
 
 /* VapourSynth4.h values (VSColorFamily / VSSampleType) so the Zig glue can pass vi.format as is. */
 enum { VSZIP_CF_GRAY = 1, VSZIP_CF_RGB = 2, VSZIP_CF_YUV = 3 };
@@ -249,9 +249,28 @@ typedef struct vszip_clahe_args {
 vszip_filter* vszip_clahe_create(const vszip_video_info* vi, const vszip_clahe_args* args);
 int vszip_clahe_get_frame(const vszip_filter* f, int32_t n, const vszip_frame* src, vszip_frame* dst);
 
+/* ------------------------------------------------------------------ ColorMap
+ * OpenCV's colormaps (cv::applyColorMap) on the luma of an 8..16-bit integer GRAY or YUV clip; the output is RGB24 of the same size
+ * and length (vszip_filter_output_info), the first filter whose output format differs from its input's.  Plane 0 only is read:
+ * i = min(x >> (bits - 8), 255), (R, G, B) = table[color][i]; for 8-bit input the result equals cv2.applyColorMap(y)[..., ::-1].
+ * Argument string: "clip:vnode;color:int:opt;".  has_color == 0: color 20 (COLORMAP_TURBO); color is cv::ColormapTypes 0..21.
+ * The Zig side sets _ColorRange = 0 and _Matrix = 0 on the output frame.  The names, default and messages are this library's. */
+typedef struct vszip_colormap_args {
+    int32_t has_color; int64_t color;
+} vszip_colormap_args;
+vszip_filter* vszip_colormap_create(const vszip_video_info* vi, const vszip_colormap_args* args);
+/* dst: the three planes of an RGB24 frame, all written. */
+int vszip_colormap_get_frame(const vszip_filter* f, int32_t n, const vszip_frame* src, vszip_frame* dst);
+/* The selected table, rgb[3 * i + c] = channel c (R, G, B) of index i (for inspection and tests). */
+int vszip_colormap_get_lut(const vszip_filter* f, uint8_t rgb[768]);
+
 /* ------------------------------------------------------------------ common filter calls */
 void vszip_filter_free(vszip_filter* f);                         /* replaces xxxFree */
-int vszip_filter_planes(const vszip_filter* f, int32_t process[3]); /* d.planes after create */
+int vszip_filter_planes(const vszip_filter* f, int32_t process[3]); /* d.planes after create: the planes the filter reads */
+/* The format of the clip the filter's node returns (the output node's vi): the input format for every filter except ColorMap,
+ * whose output is RGB24.  A filter that changes the format writes every plane of its output; any other pixel filter writes the
+ * planes vszip_filter_planes reports and leaves the others to the input frame. */
+int vszip_filter_output_info(const vszip_filter* f, vszip_video_info* out);
 
 /* ------------------------------------------------------------------ device-resident clips
  * Frames that stay in HBM: used to chain vszip filters without PCIe round trips and to measure
@@ -274,7 +293,8 @@ void* vszip_dev_clip_plane_ptr(const vszip_dev_clip* c, int32_t frame, int32_t p
 /* Batched, asynchronous, device-resident execution on frames [first, first+count) of the clips.
  * `stream` is a cudaStream_t (as void*) on the clips' device, or NULL for the library's own stream
  * of that device; work is enqueued and NOT synchronised (use vszip_cuda_stream_sync or your own
- * event).  src and dst must have the same format/size and live on the same device. */
+ * event).  src and dst must have the same format/size and live on the same device; for ColorMap dst has the filter's output format
+ * (vszip_filter_output_info). */
 int vszip_boxblur_device(const vszip_filter* f, const vszip_dev_clip* src, vszip_dev_clip* dst,
                          int32_t first, int32_t count, void* stream);
 int vszip_bilateral_device(const vszip_filter* f, const vszip_dev_clip* src, const vszip_dev_clip* ref,
@@ -309,6 +329,8 @@ int vszip_adaptivebinarize_device(const vszip_filter* f, const vszip_dev_clip* c
                                   vszip_dev_clip* dst, int32_t first, int32_t count, void* stream);
 int vszip_clahe_device(const vszip_filter* f, const vszip_dev_clip* src, vszip_dev_clip* dst,
                        int32_t first, int32_t count, void* stream);
+int vszip_colormap_device(const vszip_filter* f, const vszip_dev_clip* src, vszip_dev_clip* dst,
+                          int32_t first, int32_t count, void* stream);
 int vszip_cuda_stream_sync(int32_t device, void* stream);
 
 /* ------------------------------------------------------------------ fused chains of vszip filters (SURVEY 8f rank 1)
@@ -317,7 +339,8 @@ int vszip_cuda_stream_sync(int32_t device, void* stream);
  * (a create-time registry node -> vszip_filter makes that visible, see INTEGRATION.md): its getFrame requests the
  * chain's SOURCE frame instead of its immediate input and calls this.  Results are identical to calling the
  * per-filter get_frame functions one after the other.
- *  - filters: 1..16 handles in evaluation order, all created for the same video format and without ref/clipb;
+ *  - filters: 1..16 handles in evaluation order, each created for the format of the values it reads (the source's, or, after a
+ *    ColorMap, RGB24) and without ref/clipb;
  *    the chain borrows them (they must outlive it).  Two "diamond" elements are accepted as well, with the chain's
  *    SOURCE frame as their second clip: a LimitFilter created without ref (flt = the chain's current value, src = the
  *    source frame: `flt = src.vszip.X(); flt.vszip.LimitFilter(src)`) and an AdaptiveBinarize (clip = the source frame,
@@ -341,7 +364,9 @@ vszip_chain* vszip_chain_create(const vszip_filter* const* filters, int32_t coun
  * vszip_chain_planes reports the planes in which that value differs from the source.  Intermediates live in HBM as long as a
  * later element reads them.  vszip_chain_create(f, n) equals vszip_chain_create2 with input == NULL and second[i] = 0 for its
  * diamond elements.  An adjacent PlaneMinMax + PlaneAverage that read the same value with the same planes and clipb (or none) share
- * one read when vszip_planestats_device_b would fuse them, with bit-identical results. */
+ * one read when vszip_planestats_device_b would fuse them, with bit-identical results.  Value 0 has filter 0's format and value k
+ * the output format of filter k - 1 (vszip_filter_output_info); every element must have been created for the format of each value
+ * it reads.  After a ColorMap every plane of the result is written, and dst has the result's format. */
 vszip_chain* vszip_chain_create2(const vszip_filter* const* filters, int32_t count, const int32_t* input, const int32_t* second,
                                  const int32_t* third);
 void vszip_chain_free(vszip_chain* c);

@@ -1,13 +1,15 @@
 """Secondary measurements: the other BASELINE.json configs, device-resident, CUDA-event timed.
 Not the contract line (bench.py prints that); results go to stdout as JSON and, with --out, to a file.
 usage: python scripts/bench_extras.py [--frames N] [--reps R] [--only REGEX] [--out profiles/bench_extras_rXX.json]
---only clahe: the CLAHE group (device batches, get_frame on pinned frames, and OpenCV on every host core for comparison)."""
+--only clahe: the CLAHE group (device batches, get_frame on pinned frames, and OpenCV on every host core for comparison);
+--only colormap: the same for ColorMap."""
 import argparse
 import json
 import sys
 from pathlib import Path
 
 sys.path.insert(0, str(Path(__file__).resolve().parents[1]))
+import numpy as np
 import torch
 
 import vapoursynth_zip_b200 as vz
@@ -240,6 +242,71 @@ def clahe_cfgs():
 
 
 clahe_cfgs()
+
+
+def _cv2_colormap(job):
+    import cv2
+    cv2.setNumThreads(1)
+    y, color = job
+    return cv2.applyColorMap(y, color)
+
+
+def colormap_cfgs():
+    """ColorMap: device-resident batches (frames/s; algorithmic bytes = the luma read + 3 * w * h written), get_frame on pinned host
+    frames from 8 threads, and OpenCV's applyColorMap on 8-bit luma over every host core (one frame per worker, one OpenCV thread per
+    worker) for comparison.  Each batch (1 GB and more) is larger than the L2."""
+    import ctypes as C
+    import multiprocessing
+    import os
+    import time
+    from concurrent.futures import ProcessPoolExecutor, ThreadPoolExecutor
+
+    lib = vz.load_library()
+    for fmt, w, h in (("GRAY8", 1920, 1080), ("GRAY16", 3840, 2160)):
+        tag = f"colormap {fmt} {w}x{h} noise"
+        if skip(tag):
+            continue
+        frames = N if fmt == "GRAY8" else max(8, N // 4)
+        src, dst = vz.DeviceClip(fmt, w, h, frames), vz.DeviceClip("RGB24", w, h, frames)
+        src.fill_noise(1234)
+        algo = src.frame_bytes + 3 * w * h
+        f = vz.ColorMapFilter(src.info(), 20)
+        ms = timed(lambda: f.run_device(src, dst, first=0, count=frames, stream=st.cuda_stream), args.reps)
+        record(f"{tag} device batch", fmt, w, h, frames, algo, ms)
+        host = [src.download(i) for i in range(4)]
+
+        def pinned(shape, dtype):
+            t = torch.empty(int(np.prod(shape)) * np.dtype(dtype).itemsize, dtype=torch.uint8, pin_memory=True)
+            return t.numpy().view(dtype).reshape(shape), t
+        ins = [pinned(fr[0].shape, fr[0].dtype) for fr in host]
+        for (q, _), fr in zip(ins, host):
+            q[...] = fr[0]
+        outs = [[pinned((h, w), np.uint8) for _ in range(3)] for _ in range(8)]
+
+        def one(i):
+            s = vz._cframe([ins[i % 4][0]])
+            d = vz._cframe([q for q, _ in outs[i % 8]])
+            vz._check(lib.vszip_colormap_get_frame(f.handle, i, C.byref(s), C.byref(d)))
+        n_e2e = 4 * frames
+        with ThreadPoolExecutor(8) as ex:
+            list(ex.map(one, range(16)))
+            t0 = time.perf_counter()
+            list(ex.map(one, range(n_e2e)))
+            e2e = time.perf_counter() - t0
+        record(f"{tag} get_frame, pinned frames, 8 threads (end to end)", fmt, w, h, n_e2e, algo, e2e * 1e3)
+        if fmt == "GRAY8":
+            workers = os.cpu_count() or 1
+            n_cpu = 8 * workers
+            with ProcessPoolExecutor(workers, mp_context=multiprocessing.get_context("fork")) as ex:
+                list(ex.map(_cv2_colormap, [(host[0][0], 20)] * workers))
+                t0 = time.perf_counter()
+                list(ex.map(_cv2_colormap, [(host[i % 4][0], 20) for i in range(n_cpu)], chunksize=4))
+                cpu = time.perf_counter() - t0
+            record(f"{tag} OpenCV 4.13: cv2.applyColorMap on {workers} host cores", fmt, w, h, n_cpu, algo, cpu * 1e3)
+        src.free(); dst.free()
+
+
+colormap_cfgs()
 
 
 def _gpu():

@@ -2,7 +2,7 @@
 
 The product is the C-ABI library (include/vszip_cuda.h, built into lib/libvszip_cuda.so from
 csrc/*.cu).  This module is the thin host side used where the reference would be driven through
-VapourSynth: it mirrors the `clip.vszip.BoxBlur / Bilateral / PlaneMinMax / PlaneAverage / ... / CLAHE` call
+VapourSynth: it mirrors the `clip.vszip.BoxBlur / Bilateral / PlaneMinMax / PlaneAverage / ... / CLAHE / ColorMap` call
 surface (same names, arguments, defaults, frame props and error messages; src/vszip.zig:46-69,
 :184-199) on top of a minimal clip/frame model, so the parity tests read like the reference's own
 tests (tests/test_boxblur.py etc. of the reference).  All arithmetic happens in the CUDA library;
@@ -93,6 +93,10 @@ class _ClaheArgs(C.Structure):
     _fields_ = [("has_limit", C.c_int32), ("limit", C.c_double), ("tiles", C.POINTER(C.c_int64)), ("num_tiles", C.c_int32)]
 
 
+class _ColorMapArgs(C.Structure):
+    _fields_ = [("has_color", C.c_int32), ("color", C.c_int64)]
+
+
 class _AverageProps(C.Structure):
     _fields_ = [("count", C.c_int32), ("plane", C.c_int32 * 3), ("has_diff", C.c_int32), ("avg", C.c_double * 3), ("diff", C.c_double * 3)]
 
@@ -150,6 +154,11 @@ ABI = {
     "vszip_clahe_create": (_P, [C.POINTER(_VideoInfo), C.POINTER(_ClaheArgs)]),
     "vszip_clahe_get_frame": (C.c_int, [_P, C.c_int32, C.POINTER(_Frame), C.POINTER(_Frame)]),
     "vszip_clahe_device": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int32, _P]),
+    "vszip_colormap_create": (_P, [C.POINTER(_VideoInfo), C.POINTER(_ColorMapArgs)]),
+    "vszip_colormap_get_frame": (C.c_int, [_P, C.c_int32, C.POINTER(_Frame), C.POINTER(_Frame)]),
+    "vszip_colormap_device": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int32, _P]),
+    "vszip_colormap_get_lut": (C.c_int, [_P, C.POINTER(C.c_uint8 * 768)]),
+    "vszip_filter_output_info": (C.c_int, [_P, C.POINTER(_VideoInfo)]),
     "vszip_chain_create": (_P, [C.POINTER(_P), C.c_int32]),
     "vszip_chain_create2": (_P, [C.POINTER(_P), C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "vszip_chain_free": (None, [_P]),
@@ -225,6 +234,15 @@ globals().update(FORMATS)  # vz.GRAY16, vz.YUV420P16, ... like the vs.* presets
 
 def _fmt(f) -> VideoFormat:
     return f if isinstance(f, VideoFormat) else FORMATS[f]
+
+
+def _format_of(vi: _VideoInfo) -> VideoFormat:
+    """The preset with this video info's format."""
+    key = (vi.color_family, vi.sample_type, vi.bits_per_sample, vi.bytes_per_sample, vi.sub_sampling_w, vi.sub_sampling_h, vi.num_planes)
+    for f in FORMATS.values():
+        if (f.color_family, f.sample_type, f.bits_per_sample, f.bytes_per_sample, f.subsampling_w, f.subsampling_h, f.num_planes) == key:
+            return f
+    raise Error(f"no format preset for {key}")
 
 
 def _vi(fmt: VideoFormat, width, height, num_frames) -> _VideoInfo:
@@ -325,7 +343,9 @@ class _Filter:
         self.handle = handle
         mask = (C.c_int32 * 3)()
         load_library().vszip_filter_planes(handle, C.byref(mask))
-        self.process = [bool(m) for m in mask]
+        self.process = [bool(m) for m in mask]  # the planes it reads
+        self.out_info = _VideoInfo()            # the format of the frames it returns
+        _check(load_library().vszip_filter_output_info(handle, C.byref(self.out_info)))
         _live_filters.add(self)
 
     def _device(self, fn, clips, first, count, stream, prop=None):
@@ -550,6 +570,25 @@ class CLAHEFilter(_Filter):
         self._device(load_library().vszip_clahe_device, (src, dst), first, count, stream)
 
 
+class ColorMapFilter(_Filter):
+    """OpenCV's colormap `color` (cv::ColormapTypes 0..21) on the luma, RGB24 out (DESIGN.md §4.8)."""
+
+    GET_FRAME = "vszip_colormap_get_frame"
+
+    def __init__(self, vi: _VideoInfo, color=None):
+        a = _ColorMapArgs(color is not None, int(color or 0))
+        super().__init__(load_library().vszip_colormap_create(C.byref(vi), C.byref(a)))
+
+    def lut(self):
+        """The selected table as a (256, 3) uint8 array of R, G, B."""
+        out = (C.c_uint8 * 768)()
+        _check(load_library().vszip_colormap_get_lut(self.handle, C.byref(out)))
+        return np.frombuffer(bytes(out), np.uint8).reshape(256, 3).copy()
+
+    def run_device(self, src: "DeviceClip", dst: "DeviceClip", first=0, count=None, stream=None):
+        self._device(load_library().vszip_colormap_device, (src, dst), first, count, stream)
+
+
 class _Namespace:
     """`clip.vszip` / `core.vszip`: the plugin functions with the reference's argument names."""
 
@@ -575,6 +614,12 @@ class _Namespace:
         if clip is None:
             raise Error("clip argument is required")
         return _node(CLAHEFilter(clip._info(), limit, tiles), clip)
+
+    def ColorMap(self, *pos, **kw) -> VideoNode:
+        clip, color = self._bind(("clip", "color"), pos, kw)
+        if clip is None:
+            raise Error("clip argument is required")
+        return _node(ColorMapFilter(clip._info(), color), clip, set_props={"_ColorRange": 0, "_Matrix": 0})
 
     def _bind(self, names, pos, kw):
         """VapourSynth binding rule: `clip.vszip.F(a, b)` puts the bound clip first and shifts the positional arguments."""
@@ -634,6 +679,7 @@ class _Op:
     second: VideoNode | None      # its second and third clips: the chain's second[i] and third[i]
     third: VideoNode | None
     base: VideoNode               # the clip whose frame gives the output's untouched planes and props
+    format: VideoFormat           # the format of the frames it returns: the base clip's unless the filter changes it
     set_props: dict               # props set on every output frame
     prefix: str                   # stats filters: the prefix of the props they write
 
@@ -650,29 +696,38 @@ class _Op:
     def get(self, n):
         """Unfused evaluation: the filter's get_frame on frame n of each input; an extra clip that is shorter repeats its last
         frame (rpFrameReuseLastOnly).  Inputs pass their processed planes; a pixel filter's output gets fresh processed planes
-        and shares the others with the base frame (newVideoFrame2), a stats filter's shares every plane (copyFrame)."""
+        and shares the others with the base frame (newVideoFrame2), or fresh planes of its own format when it changes the format;
+        a stats filter's shares every plane (copyFrame)."""
         core._ensure_init()
         flt, clips = self.filter, (self.input, self.second, self.third)
         frames = [None if clips[i] is None else clips[i].get_frame(min(n, clips[i].num_frames - 1)) for i in flt.ARGS]
         base = frames[0]
         args = [None if fr is None else C.byref(_cframe([_rows(p) if flt.process[i] else None for i, p in enumerate(fr.planes)]))
                 for fr in frames]
-        if flt.PROPS is None:
+        fmt = self.format
+        if flt.PROPS is None and fmt is not base.format:
+            planes = [np.empty(fmt.plane_shape(base.width, base.height, i), fmt.dtype) for i in range(fmt.num_planes)]
+            stats, out = None, _cframe(planes)
+        elif flt.PROPS is None:
             planes = [np.empty_like(p, order="C") if flt.process[i] else p for i, p in enumerate(base.planes)]
             stats, out = None, _cframe([p if flt.process[i] else None for i, p in enumerate(planes)])
         else:
             planes = base.planes
             stats = out = flt.PROPS()
         _check(getattr(load_library(), flt.GET_FRAME)(flt.handle, n, *args, C.byref(out)))
-        return VideoFrame(base.format, base.width, base.height, planes, self.props(base.props, stats))
+        return VideoFrame(fmt, base.width, base.height, planes, self.props(base.props, stats))
 
 
 def _node(flt: _Filter, main: VideoNode, second: VideoNode | None = None, third: VideoNode | None = None, set_props=None,
           prefix="") -> VideoNode:
     """A vszip node on `main`, `second` and `third` (the chain's numbering)."""
     base = (main, second, third)[flt.ARGS[0]]
-    op = _Op(flt, main, second, third, base, set_props or {}, prefix)
-    node = VideoNode(base.format, base.width, base.height, base.num_frames, op.get)
+    o, b = flt.out_info, base.format  # the library's output format (vszip_filter_output_info): the base clip's but for ColorMap
+    same = (o.color_family, o.sample_type, o.bits_per_sample, o.sub_sampling_w, o.sub_sampling_h, o.num_planes) == (
+        b.color_family, b.sample_type, b.bits_per_sample, b.subsampling_w, b.subsampling_h, b.num_planes)
+    fmt = b if same else _format_of(o)
+    op = _Op(flt, main, second, third, base, fmt, set_props or {}, prefix)
+    node = VideoNode(fmt, base.width, base.height, base.num_frames, op.get)
     node.filter, node._op = flt, op
     return node
 
@@ -758,7 +813,10 @@ def _fused_get(chain_and_source, n: int) -> "VideoFrame":
     chain, source = chain_and_source
     core._ensure_init()
     src = source.get_frame(n)
-    out_planes = [np.empty_like(p, order="C") if chain.written[i] else p for i, p in enumerate(src.planes)]
+    last = chain.nodes[-1]  # the result has the last node's format: the source's, or RGB24 after a ColorMap
+    fmt = last.format
+    out_planes = [np.empty(fmt.plane_shape(src.width, src.height, i), fmt.dtype) if chain.written[i] else src.planes[i]
+                  for i in range(fmt.num_planes)]
     s = _cframe([_rows(p) for p in src.planes])
     d = _cframe([p if chain.written[i] else None for i, p in enumerate(out_planes)])
     outs, ptrs = [], (_P * len(chain.nodes))()
@@ -773,7 +831,7 @@ def _fused_get(chain_and_source, n: int) -> "VideoFrame":
     props = {id(source): src.props}
     for nd, o in zip(chain.nodes, outs):
         props[id(nd)] = nd._op.props(props[id(nd._op.base)], o)
-    return VideoFrame(source.format, source.width, source.height, out_planes, props[id(chain.nodes[-1])])
+    return VideoFrame(fmt, source.width, source.height, out_planes, props[id(last)])
 
 
 # --------------------------------------------------------------------------- device-resident clips

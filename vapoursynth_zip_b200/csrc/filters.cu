@@ -9,6 +9,7 @@
 #include <limits>
 #include <string>
 
+#include "colormap_tables.h"
 #include "filter.h"
 
 using namespace vsz;
@@ -137,28 +138,32 @@ DeviceCtx* route(int32_t n, const char* name) {
     return d;
 }
 
-bool same_clip_shape(const vszip_dev_clip* a, const vszip_filter* f, const char* name) {
-    if (!a || a->vi.width != f->vi.width || a->vi.height != f->vi.height || a->layout.kind != f->sample ||
-        a->vi.num_planes != f->vi.num_planes || a->vi.sub_sampling_w != f->vi.sub_sampling_w ||
-        a->vi.sub_sampling_h != f->vi.sub_sampling_h || a->vi.bits_per_sample != f->vi.bits_per_sample ||
-        a->vi.sample_type != f->vi.sample_type) {
+bool same_clip_format(const vszip_dev_clip* a, const vszip_video_info& vi, SampleKind kind, const char* name) {
+    if (!a || a->vi.width != vi.width || a->vi.height != vi.height || a->layout.kind != kind || a->vi.num_planes != vi.num_planes ||
+        a->vi.sub_sampling_w != vi.sub_sampling_w || a->vi.sub_sampling_h != vi.sub_sampling_h ||
+        a->vi.bits_per_sample != vi.bits_per_sample || a->vi.sample_type != vi.sample_type) {
         set_error("%s: device clip does not match the format the filter was created for", name);
         return false;
     }
     return true;
 }
 
+bool same_clip_shape(const vszip_dev_clip* a, const vszip_filter* f, const char* name) { return same_clip_format(a, f->vi, f->sample, name); }
+
 bool range_ok(const vszip_dev_clip* c, int first, int count, const char* name) {
     if (first < 0 || count < 0 || first + count > c->num_frames) { set_error("%s: frame range out of bounds", name); return false; }
     return true;
 }
 
-// The checks of a batched call: every clip it reads or writes matches the instance's format (a NULL clip does not) and holds
-// frames [first, first + count), and all of them live on one initialised device, which becomes current.  *st: the caller's
-// stream, or that device's batch stream.
+// The checks of a batched call: every clip it reads matches the instance's format and the clip it writes (the last one, when
+// `output` is set) the format of the frames it returns (a NULL clip does not match); every clip holds frames [first, first + count),
+// and all of them live on one initialised device, which becomes current.  *st: the caller's stream, or that device's batch stream.
 int begin_device_call(const vszip_filter* f, const char* name, const vszip_dev_clip* const* clips, int n, int32_t first, int32_t count,
-                      void* stream, cudaStream_t* st) {
-    for (int i = 0; i < n; ++i) if (!same_clip_shape(clips[i], f, name)) return -1;
+                      void* stream, cudaStream_t* st, bool output = false) {
+    for (int i = 0; i < n; ++i) {
+        const bool out = output && i == n - 1;
+        if (!same_clip_format(clips[i], out ? f->out_vi : f->vi, out ? f->out_layout.kind : f->sample, name)) return -1;
+    }
     for (int i = 0; i < n; ++i) if (!range_ok(clips[i], first, count, name)) return -1;
     for (int i = 1; i < n; ++i)
         if (clips[i]->device_index != clips[0]->device_index) { set_error("%s: clips live on different devices", name); return -1; }
@@ -172,6 +177,27 @@ int begin_device_call(const vszip_filter* f, const char* name, const vszip_dev_c
 int device_index_of(DeviceCtx* d) {
     for (int i = 0; i < num_devices(); ++i) if (device_ctx(i) == d) return i;
     return 0;
+}
+
+bool same_format(const vszip_video_info& a, const vszip_video_info& b) {
+    return a.width == b.width && a.height == b.height && a.color_family == b.color_family && a.sample_type == b.sample_type &&
+           a.bits_per_sample == b.bits_per_sample && a.sub_sampling_w == b.sub_sampling_w && a.sub_sampling_h == b.sub_sampling_h &&
+           a.num_planes == b.num_planes;
+}
+
+// The format every create function gives its instance: it reads and returns frames of vi (ColorMap then sets its output format).
+void set_format(vszip_filter* f, const vszip_video_info& vi, SampleKind kind) {
+    f->vi = f->out_vi = vi;
+    f->sample = kind;
+    f->layout = f->out_layout = make_layout(vi, kind);
+}
+
+// A filter whose output format differs from its input's: it writes every plane of its output.
+bool converts(const vszip_filter* f) { return !same_format(f->vi, f->out_vi); }
+
+// The planes of the output frame a pixel filter writes: the ones it processes, or all of them when it changes the format.
+void written_planes(const vszip_filter* f, bool w[3]) {
+    for (int p = 0; p < 3; ++p) w[p] = converts(f) ? p < f->out_layout.nplanes : f->process[p];
 }
 
 int processed_planes(const vszip_filter* f) {
@@ -196,8 +222,9 @@ constexpr KindInfo kKinds[] = {
     {"LimitFilter", true, {"src", "ref"}, {false, true}},
     {"AdaptiveBinarize", true, {"clip", nullptr}, {false, false}},
     {"CLAHE", true, {nullptr, nullptr}, {false, false}},
+    {"ColorMap", true, {nullptr, nullptr}, {false, false}},
 };
-static_assert(sizeof kKinds / sizeof kKinds[0] == F_CLAHE, "one row per FilterKind");
+static_assert(sizeof kKinds / sizeof kKinds[0] == F_COLORMAP, "one row per FilterKind");
 
 const KindInfo& kind_info(int kind) { return kKinds[kind - 1]; }
 bool is_pixel(const vszip_filter* f) { return kind_info(f->kind).pixel; }
@@ -242,10 +269,18 @@ int vszip_filter_planes(const vszip_filter* f, int32_t process[3]) {
     return 0;
 }
 
+int vszip_filter_output_info(const vszip_filter* f, vszip_video_info* out) {
+    if (!f || !out) { set_error("vszip_filter_output_info: bad filter handle"); return -1; }
+    *out = f->out_vi;
+    return 0;
+}
+
 // =========================================================================== shared entry-point bodies
 // The dispatchers, defined after the filters' own sections.  `in` holds a pixel filter's main input, then its second and third
-// (the chain's numbering, whatever order the filter's own entry points take them in); consecutive frames are fs bytes apart.
-static int run_pixels(const vszip_filter* f, int dev_index, const char* const in[3], char* out, size_t fs, int count, cudaStream_t st);
+// (the chain's numbering, whatever order the filter's own entry points take them in); consecutive frames are in_fs bytes apart in
+// the inputs and out_fs bytes apart in the output (they differ only for a filter that changes the format).
+static int run_pixels(const vszip_filter* f, int dev_index, const char* const in[3], size_t in_fs, char* out, size_t out_fs, int count,
+                      cudaStream_t st);
 static int run_stats(const vszip_filter* f, int dev_index, const char* a, const char* b, size_t fs, int count, void* scratch,
                      StatsRaw* raw, cudaStream_t st);
 static void stats_finalize(const vszip_filter* f, const StatsRaw* raw, void* props, int i);  // into element i of a props array
@@ -253,7 +288,8 @@ static void stats_finalize(const vszip_filter* f, const StatsRaw* raw, void* pro
 using Frames = std::array<const vszip_frame*, 3>;
 using DevClips = std::array<const vszip_dev_clip*, 3>;
 
-// getFrame of a pixel filter: the inputs staged into slot buffers 0, 1 and 3, the output computed into dev[2] and brought back.
+// getFrame of a pixel filter: the inputs staged into slot buffers 0, 1 and 3, the output computed into dev[2] and brought back
+// (the planes it writes, in the output format).
 static int pixel_get_frame(const vszip_filter* f, int kind, int32_t n, const Frames& in, vszip_frame* dst) {
     const char* name = kind_info(kind).name;
     if (!f || f->kind != kind) { set_error("%s: bad filter handle", name); return -1; }
@@ -265,7 +301,7 @@ static int pixel_get_frame(const vszip_filter* f, int kind, int32_t n, const Fra
     VSZ_CUDA(cudaSetDevice(d->ordinal));
     static const int buf[3] = {0, 1, 3};  // the slot buffer of each input
     const size_t bytes = f->layout.frame_stride;
-    if (slot_reserve(d, s, 2, bytes)) return -1;
+    if (slot_reserve(d, s, 2, f->out_layout.frame_stride)) return -1;
     for (int k = 0; k < 3; ++k)  // the main input always, the others when given
         if ((k == 0 || in[k]) && slot_reserve(d, s, buf[k], bytes)) return -1;
     const char* dev_in[3] = {nullptr, nullptr, nullptr};
@@ -274,12 +310,13 @@ static int pixel_get_frame(const vszip_filter* f, int kind, int32_t n, const Fra
         if (stage_in(s, buf[k], f->layout, in[k], f->process)) return -1;
         dev_in[k] = s->dev[buf[k]];
     }
-    const int rc = run_pixels(f, device_index_of(d), dev_in, s->dev[2], 0, 1, s->stream);
+    const int rc = run_pixels(f, device_index_of(d), dev_in, 0, s->dev[2], 0, 1, s->stream);
     if (rc) return rc;
-    bool direct[3];
-    if (stage_out_begin(s, f->layout, dst, f->process, direct)) return -1;
+    bool written[3], direct[3];
+    written_planes(f, written);
+    if (stage_out_begin(s, f->out_layout, dst, written, direct)) return -1;
     VSZ_CUDA(cudaStreamSynchronize(s->stream));
-    stage_out_finish(s, f->layout, dst, f->process, direct);
+    stage_out_finish(s, f->out_layout, dst, written, direct);
     return 0;
 }
 
@@ -320,16 +357,16 @@ static int device_call(const vszip_filter* f, int kind, const DevClips& in, cons
     int n = 1;
     for (int i = 0; i < 2; ++i) if (f->has_input[i]) clips[n++] = in[i + 1];
     if (k.pixel) clips[n++] = dst;
-    return begin_device_call(f, k.name, clips, n, first, count, stream, st);
+    return begin_device_call(f, k.name, clips, n, first, count, stream, st, k.pixel);
 }
 
 static int pixel_device(const vszip_filter* f, int kind, const DevClips& in, vszip_dev_clip* dst, int32_t first, int32_t count, void* stream) {
     cudaStream_t st;
     if (device_call(f, kind, in, dst, first, count, stream, &st)) return -1;
-    const size_t fs = dst->layout.frame_stride, off = (size_t)first * fs;
     const char* p[3];
-    for (int k = 0; k < 3; ++k) p[k] = in[k] ? in[k]->base + off : nullptr;
-    return run_pixels(f, dst->device_index, p, dst->base + off, fs, count, st);
+    for (int k = 0; k < 3; ++k) p[k] = in[k] ? in[k]->base + (size_t)first * in[k]->layout.frame_stride : nullptr;
+    const size_t out_fs = dst->layout.frame_stride;
+    return run_pixels(f, dst->device_index, p, in[0]->layout.frame_stride, dst->base + (size_t)first * out_fs, out_fs, count, st);
 }
 
 static int stats_device(const vszip_filter* f, int kind, const vszip_dev_clip* a, const vszip_dev_clip* b, int32_t first, int32_t count,
@@ -380,9 +417,7 @@ vszip_filter* vszip_boxblur_create(const vszip_video_info* vi, const vszip_boxbl
     }
     vszip_filter* f = new vszip_filter();
     f->kind = F_BOXBLUR;
-    f->vi = *vi;
-    f->sample = kind;
-    f->layout = make_layout(*vi, kind);
+    set_format(f, *vi, kind);
     for (int i = 0; i < 3; ++i) f->process[i] = process[i] && i < vi->num_planes;
     f->hradius = hr; f->vradius = vr; f->hpasses = hp; f->vpasses = vp;
     return f;
@@ -405,9 +440,7 @@ vszip_filter* vszip_bilateral_create(const vszip_video_info* vi, const vszip_vid
     vszip_filter* f = new vszip_filter();
     auto fail = [&]() { vszip_filter_free(f); return (vszip_filter*)nullptr; };
     f->kind = F_BILATERAL;
-    f->vi = *vi;
-    f->sample = kind;
-    f->layout = make_layout(*vi, kind);
+    set_format(f, *vi, kind);
     const bool yuv = vi->color_family == VSZIP_CF_YUV;
     f->hist_len = vi->sample_type == VSZIP_ST_INTEGER ? (1 << vi->bits_per_sample) : 65536;  // hz.getHistLen
     f->peak = (float)(f->hist_len - 1);
@@ -608,9 +641,7 @@ vszip_filter* vszip_planeminmax_create(const vszip_video_info* vi, const vszip_v
     }
     vszip_filter* f = new vszip_filter();
     f->kind = F_PLANEMINMAX;
-    f->vi = *vi;
-    f->sample = kind;
-    f->layout = make_layout(*vi, kind);
+    set_format(f, *vi, kind);
     for (int i = 0; i < 3; ++i) f->process[i] = process[i] && i < vi->num_planes;
     f->has_input[0] = clipb_vi != nullptr;
     f->minthr = minthr; f->maxthr = maxthr; f->hist_size = hist_size; f->no_thr = no_thr;
@@ -670,9 +701,7 @@ vszip_filter* vszip_planeaverage_create(const vszip_video_info* vi, const vszip_
     if (u32) { set_error("PlaneAverage: exclude is not supported for 32-bit integer clips."); return nullptr; }
     vszip_filter* f = new vszip_filter();
     f->kind = F_PLANEAVERAGE;
-    f->vi = *vi;
-    f->sample = kind;
-    f->layout = make_layout(*vi, kind);
+    set_format(f, *vi, kind);
     for (int i = 0; i < 3; ++i) f->process[i] = process[i] && i < vi->num_planes;
     f->has_input[0] = clipb_vi != nullptr;
     f->avg_peak = (float)((1ull << vi->bits_per_sample) - 1ull);  // planeaverage.zig:112
@@ -741,8 +770,10 @@ int vszip_planeaverage_device(const vszip_filter* f, const vszip_dev_clip* a, co
 }
 
 // =========================================================================== dispatch
-static int run_pixels(const vszip_filter* f, int dev_index, const char* const in[3], char* out, size_t fs, int count, cudaStream_t st) {
+static int run_pixels(const vszip_filter* f, int dev_index, const char* const in[3], size_t in_fs, char* out, size_t out_fs, int count,
+                      cudaStream_t st) {
     const FrameLayout& l = f->layout;
+    const size_t fs = in_fs;  // every filter but ColorMap: out_fs == in_fs
     switch (f->kind) {
         case F_BOXBLUR:
             return run_boxblur(l, f->process, in[0], fs, out, fs, count, (int)f->hradius, f->hpasses, (int)f->vradius, f->vpasses, st);
@@ -755,6 +786,8 @@ static int run_pixels(const vszip_filter* f, int dev_index, const char* const in
             return run_limitfilter(l, f->process, in[0], fs, in[1], fs, in[2], fs, out, fs, count, f->lf_dark, f->lf_bright, f->lf_elast, st);
         case F_CLAHE:
             return run_clahe(l, f->process, in[0], fs, out, fs, count, f->clahe_hs, f->clahe_limit, f->clahe_tiles[0], f->clahe_tiles[1], st);
+        case F_COLORMAP:
+            return run_colormap(l, in[0], in_fs, f->out_layout, out, out_fs, count, f->cmap_lut, st);
         default:  // AdaptiveBinarize: clip = the second input, clip2 = the main one
             return run_adaptivebinarize(l, in[1], fs, in[0], fs, out, fs, count, f->ab_c, st);
     }
@@ -934,9 +967,7 @@ vszip_filter* vszip_limiter_create(const vszip_video_info* vi, const vszip_limit
     if (!has_min) limiter_table(*vi, tv_range, yuv, lo, hi);
     vszip_filter* f = new vszip_filter();
     f->kind = F_LIMITER;
-    f->vi = *vi;
-    f->sample = kind;
-    f->layout = make_layout(*vi, kind);
+    set_format(f, *vi, kind);
     for (int i = 0; i < 3; ++i) { f->process[i] = process[i] && i < np; f->lim_lo[i] = lo[i]; f->lim_hi[i] = hi[i]; }
     return f;
 }
@@ -971,9 +1002,7 @@ vszip_filter* vszip_limitfilter_create(const vszip_video_info* flt_vi, const vsz
     const bool limited = a->color_range < 0 ? flt_vi->color_family != VSZIP_CF_RGB : a->color_range == 1;
     vszip_filter* f = new vszip_filter();
     f->kind = F_LIMITFILTER;
-    f->vi = *flt_vi;
-    f->sample = kind;
-    f->layout = make_layout(*flt_vi, kind);
+    set_format(f, *flt_vi, kind);
     for (int i = 0; i < 3; ++i) {
         f->process[i] = process[i] && i < flt_vi->num_planes;
         f->lf_dark[i] = scale_value8(dark[i], *flt_vi, limited);                       // :114-118
@@ -1012,9 +1041,7 @@ vszip_filter* vszip_adaptivebinarize_create(const vszip_video_info* vi, const vs
     const int64_t c = a && a->has_c ? (int64_t)sat_i32(a->c) : 3;                      // getValue(i32, "c") orelse 3
     vszip_filter* f = new vszip_filter();
     f->kind = F_ADAPTIVEBINARIZE;
-    f->vi = *vi;
-    f->sample = K_U8;
-    f->layout = make_layout(*vi, K_U8);
+    set_format(f, *vi, K_U8);
     for (int i = 0; i < 3; ++i) f->process[i] = i < vi->num_planes;
     f->ab_c = (int)std::min<int64_t>(std::max<int64_t>(c, -256), 256);               // :97-99
     f->has_input[0] = true;
@@ -1054,9 +1081,7 @@ vszip_filter* vszip_clahe_create(const vszip_video_info* vi, const vszip_clahe_a
     if (t[0] > 256 || t[1] > 256 || t[0] * t[1] > 256) { set_error("CLAHE: at most 256 tiles per plane (tiles[0] * tiles[1])."); return nullptr; }
     vszip_filter* f = new vszip_filter();
     f->kind = F_CLAHE;
-    f->vi = *vi;
-    f->sample = kind;
-    f->layout = make_layout(*vi, kind);
+    set_format(f, *vi, kind);
     for (int i = 0; i < 3; ++i) f->process[i] = i < vi->num_planes;
     f->clahe_limit = limit;
     f->clahe_tiles[0] = (int)t[0];
@@ -1073,28 +1098,83 @@ int vszip_clahe_device(const vszip_filter* f, const vszip_dev_clip* src, vszip_d
     return pixel_device(f, F_CLAHE, {src, nullptr, nullptr}, dst, first, count, stream);
 }
 
+// =========================================================================== ColorMap
+// OpenCV's applyColorMap on plane 0 (DESIGN.md §4.8): GRAY / YUV in, RGB24 out.  The argument names, default and messages are this
+// library's.
+vszip_filter* vszip_colormap_create(const vszip_video_info* vi, const vszip_colormap_args* a) {
+    static const char* name = "ColorMap";
+    if (!basic_vi_ok(vi, name)) return nullptr;
+    if (vi->sample_type != VSZIP_ST_INTEGER || vi->bits_per_sample < 8 || vi->bits_per_sample > 16) {
+        set_error("ColorMap: only 8-16 bit int formats supported.");
+        return nullptr;
+    }
+    if (vi->color_family != VSZIP_CF_GRAY && vi->color_family != VSZIP_CF_YUV) { set_error("ColorMap: clip must be GRAY or YUV."); return nullptr; }
+    const int64_t color = a && a->has_color ? a->color : 20;  // COLORMAP_TURBO
+    if (color < 0 || color >= kColormapCount) { set_error("ColorMap: color must be between 0 and 21."); return nullptr; }
+    SampleKind kind;
+    if (!select_kind(*vi, name, false, &kind)) return nullptr;
+    vszip_filter* f = new vszip_filter();
+    f->kind = F_COLORMAP;
+    set_format(f, *vi, kind);
+    vszip_video_info o = *vi;  // RGB24 of the same size and length
+    o.color_family = VSZIP_CF_RGB;
+    o.sample_type = VSZIP_ST_INTEGER;
+    o.bits_per_sample = 8;
+    o.bytes_per_sample = 1;
+    o.sub_sampling_w = o.sub_sampling_h = 0;
+    o.num_planes = 3;
+    f->out_vi = o;
+    f->out_layout = make_layout(o, K_U8);
+    for (int i = 0; i < 3; ++i) f->process[i] = i == 0;  // the planes it reads: the luma
+    memcpy(f->cmap_lut, kColormapTables[color], sizeof f->cmap_lut);
+    return f;
+}
+
+int vszip_colormap_get_lut(const vszip_filter* f, uint8_t rgb[768]) {
+    if (!f || f->kind != F_COLORMAP || !rgb) { set_error("ColorMap: bad filter handle"); return -1; }
+    for (int i = 0; i < 256; ++i)
+        for (int c = 0; c < 3; ++c) rgb[3 * i + c] = (uint8_t)(f->cmap_lut[i] >> (8 * c));
+    return 0;
+}
+
+int vszip_colormap_get_frame(const vszip_filter* f, int32_t n, const vszip_frame* src, vszip_frame* dst) {
+    return pixel_get_frame(f, F_COLORMAP, n, {src, nullptr, nullptr}, dst);
+}
+
+int vszip_colormap_device(const vszip_filter* f, const vszip_dev_clip* src, vszip_dev_clip* dst, int32_t first, int32_t count, void* stream) {
+    return pixel_device(f, F_COLORMAP, {src, nullptr, nullptr}, dst, first, count, stream);
+}
+
 // =========================================================================== fused chains
 // Values of a chain: 0 = the source frame, k >= 1 = the pixel output of element k - 1.  Every element reads its main input (the
 // value it filters) and up to two extra inputs; the buffer plan gives every pixel output a frame buffer for as long as a later
 // element reads it (DESIGN.md §5.1).  Buffers 0..2 are the slot's dev[0..2] (0 = the source, never written; 2 = the value the
-// chain returns, the D2H source), buffers 3.. are the slot's device-only extras.
+// chain returns, the D2H source), buffers 3.. are the slot's device-only extras.  Every value has a format: value 0 filter 0's,
+// value k the output format of element k - 1, which differs from its input's for ColorMap.
 struct vszip_chain {
     std::vector<const vszip_filter*> fl;
-    vsz::FrameLayout layout;
+    vsz::FrameLayout in_layout, out_layout;  // the source's and the returned value's
     bool written[3];
     int npixel;
     std::vector<int> in, in2, in3;  // buffer of each element's main / second / third input (-1: none)
     std::vector<int> out;           // buffer of each element's pixel output (-1: stats element)
     std::vector<char> fuse_next;    // stats element i runs together with element i + 1 from one read
     std::vector<char> used;         // buffers the plan uses (0..2: the slot's dev[], 3..: its device-only extras)
+    std::vector<size_t> bytes;      // the size of each buffer: the frame stride of the largest value it holds
 };
 
 namespace {
 
-bool same_format(const vszip_video_info& a, const vszip_video_info& b) {
-    return a.width == b.width && a.height == b.height && a.color_family == b.color_family && a.sample_type == b.sample_type &&
-           a.bits_per_sample == b.bits_per_sample && a.sub_sampling_w == b.sub_sampling_w && a.sub_sampling_h == b.sub_sampling_h &&
-           a.num_planes == b.num_planes;
+const FrameLayout& value_layout(const vszip_filter* const* filters, int v) { return v == 0 ? filters[0]->layout : filters[v - 1]->out_layout; }
+
+// Element i reads value v: it must have been created for that value's format.  The message names filter 0 when the value has its
+// format (every value of a chain without a format-changing element does).
+bool reads_ok(const vszip_filter* const* filters, int i, int v) {
+    const vszip_video_info& fmt = v == 0 ? filters[0]->vi : filters[v - 1]->out_vi;
+    if (same_format(filters[i]->vi, fmt)) return true;
+    if (same_format(fmt, filters[0]->vi)) set_error("chain: filter %d was created for a different video format than filter 0", i);
+    else set_error("chain: filter %d was created for a different video format than the value it reads", i);
+    return false;
 }
 
 // input / second / third use the value numbering above; input == nullptr: every element reads the latest pixel output (or the source).
@@ -1114,7 +1194,8 @@ vszip_chain* chain_build(const vszip_filter* const* filters, int count, const in
     const int result = is_pixel(fl) ? count : vin[count - 1];
     vszip_chain* c = new vszip_chain();
     c->fl.assign(filters, filters + count);
-    c->layout = filters[0]->layout;
+    c->in_layout = filters[0]->layout;
+    c->out_layout = value_layout(filters, result);
     c->npixel = 0;
     for (int i = 0; i < count; ++i) {
         for (int v : {vin[i], v2[i], v3[i]}) if (v >= 0) last_use[v] = std::max(last_use[v], i);
@@ -1123,8 +1204,11 @@ vszip_chain* chain_build(const vszip_filter* const* filters, int count, const in
     // planes in which each value differs from the source
     std::vector<std::array<bool, 3>> diff(nv, std::array<bool, 3>{false, false, false});
     for (int i = 0; i < count; ++i)
-        if (is_pixel(filters[i]))
-            for (int p = 0; p < 3; ++p) diff[i + 1][p] = diff[vin[i]][p] || filters[i]->process[p];
+        if (is_pixel(filters[i])) {
+            bool w[3];
+            written_planes(filters[i], w);
+            for (int p = 0; p < 3; ++p) diff[i + 1][p] = (!converts(filters[i]) && diff[vin[i]][p]) || w[p];
+        }
     for (int p = 0; p < 3; ++p) c->written[p] = diff[result][p];
     // buffer plan: a value occupies its buffer from the element that writes it to the last element that reads it (both inclusive,
     // so an element never writes the buffer it reads).  The result goes to buffer 2 and lives to the end; the other pixel outputs,
@@ -1149,7 +1233,13 @@ vszip_chain* chain_build(const vszip_filter* const* filters, int count, const in
     }
     c->used.assign(busy.size(), 0);
     c->used[0] = c->used[2] = 1;
-    for (int v = 1; v < nv; ++v) if (buf[v] >= 0) c->used[buf[v]] = 1;
+    c->bytes.assign(busy.size(), 0);
+    c->bytes[0] = c->in_layout.frame_stride;
+    for (int v = 1; v < nv; ++v)
+        if (buf[v] >= 0) {
+            c->used[buf[v]] = 1;
+            c->bytes[buf[v]] = std::max(c->bytes[buf[v]], value_layout(filters, v).frame_stride);
+        }
     for (int i = 0; i < count; ++i) {
         c->in.push_back(buf[vin[i]]);
         c->in2.push_back(v2[i] >= 0 ? buf[v2[i]] : -1);
@@ -1170,19 +1260,17 @@ vszip_chain* chain_build(const vszip_filter* const* filters, int count, const in
 
 vszip_chain* vszip_chain_create(const vszip_filter* const* filters, int32_t count) {
     if (!filters || count < 1 || count > 16) { set_error("chain: between 1 and 16 filters are required"); return nullptr; }
-    const vszip_filter* f0 = filters[0];
     int32_t second[16];
+    int cur = 0;  // the value element i filters: the latest pixel output, or the source
     for (int i = 0; i < count; ++i) {
         const vszip_filter* f = filters[i];
         if (!f) { set_error("chain: filter %d is NULL", i); return nullptr; }
         // LimitFilter (without ref) and AdaptiveBinarize take the chain's SOURCE frame as their second clip ("diamond" elements)
         const bool diamond = (f->kind == F_LIMITFILTER && !f->has_input[1]) || f->kind == F_ADAPTIVEBINARIZE;
         if (f->has_input[0] && !diamond) { set_error("chain: filter %d takes a second clip (ref/clipb); only single-input filters can be fused", i); return nullptr; }
-        if (!same_format(f0->vi, f->vi)) {
-            set_error("chain: filter %d was created for a different video format than filter 0", i);
-            return nullptr;
-        }
+        if (!reads_ok(filters, i, cur) || (diamond && !reads_ok(filters, i, 0))) return nullptr;
         second[i] = diamond ? 0 : -1;
+        if (is_pixel(f)) cur = i + 1;
     }
     return chain_build(filters, count, nullptr, second, nullptr);
 }
@@ -1191,10 +1279,12 @@ vszip_chain* vszip_chain_create2(const vszip_filter* const* filters, int32_t cou
                                  const int32_t* third) {
     if (!filters || count < 1 || count > 16) { set_error("chain: between 1 and 16 filters are required"); return nullptr; }
     const vszip_filter* f0 = filters[0];
+    bool converted = false;  // an earlier element changed the format: the values no longer all have filter 0's
+    int cur = 0;             // the value element i filters when input == NULL
     for (int i = 0; i < count; ++i) {
         const vszip_filter* f = filters[i];
         if (!f) { set_error("chain: filter %d is NULL", i); return nullptr; }
-        if (!same_format(f0->vi, f->vi)) {
+        if (!converted && !same_format(f0->vi, f->vi)) {
             set_error("chain: filter %d was created for a different video format than filter 0", i);
             return nullptr;
         }
@@ -1214,6 +1304,10 @@ vszip_chain* vszip_chain_create2(const vszip_filter* const* filters, int32_t cou
             if (v >= 1 && v - 1 >= i) { set_error("chain: %s[%d] names filter %d, which does not come before filter %d", arr[k], i, v - 1, i); return nullptr; }
             if (v >= 1 && !is_pixel(filters[v - 1])) { set_error("chain: %s[%d] names filter %d (%s), which has no pixel output", arr[k], i, v - 1, kind_info(filters[v - 1]->kind).name); return nullptr; }
         }
+        for (int k = 0; k < 3; ++k)
+            if (refs[k] >= 0 && !reads_ok(filters, i, k == 0 && !input ? cur : refs[k])) return nullptr;
+        converted = converted || (is_pixel(f) && converts(f));
+        if (is_pixel(f)) cur = i + 1;
     }
     return chain_build(filters, count, input, second, third);
 }
@@ -1234,11 +1328,10 @@ int vszip_chain_get_frame(const vszip_chain* c, int32_t n, const vszip_frame* sr
     SlotGuard g(d);
     Slot* s = g.s;
     VSZ_CUDA(cudaSetDevice(d->ordinal));
-    const FrameLayout& l = c->layout;
-    const size_t bytes = l.frame_stride;
-    if (slot_reserve(d, s, 0, bytes) || slot_reserve(d, s, 2, bytes) || (c->used[1] && slot_reserve(d, s, 1, bytes))) return -1;
+    const FrameLayout& l = c->in_layout;
+    if (slot_reserve(d, s, 0, c->bytes[0]) || slot_reserve(d, s, 2, c->bytes[2]) || (c->used[1] && slot_reserve(d, s, 1, c->bytes[1]))) return -1;
     for (int b = 3; b < (int)c->used.size(); ++b)
-        if (slot_reserve_extra(d, s, b - 3, bytes)) return -1;
+        if (slot_reserve_extra(d, s, b - 3, c->bytes[b])) return -1;
     auto B = [&](int b) -> char* { return b < 0 ? nullptr : (b < 3 ? s->dev[b] : s->xdev[b - 3]); };
     bool all[3] = {l.nplanes > 0, l.nplanes > 1, l.nplanes > 2};
     if (stage_in(s, 0, l, src, all)) return -1;  // later filters may read planes that earlier ones do not process
@@ -1249,12 +1342,13 @@ int vszip_chain_get_frame(const vszip_chain* c, int32_t n, const vszip_frame* sr
         const char* in[3] = {B(c->in[i]), B(c->in2[i]), B(c->in3[i])};
         if (is_pixel(f)) {
             char* nxt = B(c->out[i]);
-            for (int p = 0; p < l.nplanes; ++p) {  // planes this filter passes through
+            const FrameLayout& fl = f->layout;
+            for (int p = 0; p < fl.nplanes && !converts(f); ++p) {  // planes this filter passes through (none when it changes the format)
                 if (f->process[p]) continue;
-                VSZ_CUDA(cudaMemcpyAsync(nxt + l.pl[p].offset, in[0] + l.pl[p].offset, (size_t)l.pl[p].pitch * l.pl[p].h,
+                VSZ_CUDA(cudaMemcpyAsync(nxt + fl.pl[p].offset, in[0] + fl.pl[p].offset, (size_t)fl.pl[p].pitch * fl.pl[p].h,
                                          cudaMemcpyDeviceToDevice, s->stream));
             }
-            const int rc = run_pixels(f, dev_index, in, nxt, 0, 1, s->stream);
+            const int rc = run_pixels(f, dev_index, in, 0, nxt, 0, 1, s->stream);
             if (rc) return rc;
             continue;
         }
@@ -1278,9 +1372,9 @@ int vszip_chain_get_frame(const vszip_chain* c, int32_t n, const vszip_frame* sr
         i += ne - 1;
     }
     bool direct[3] = {false, false, false};
-    if (c->npixel > 0 && stage_out_begin(s, l, dst, c->written, direct)) return -1;
+    if (c->npixel > 0 && stage_out_begin(s, c->out_layout, dst, c->written, direct)) return -1;
     VSZ_CUDA(cudaStreamSynchronize(s->stream));
-    if (c->npixel > 0) stage_out_finish(s, l, dst, c->written, direct);
+    if (c->npixel > 0) stage_out_finish(s, c->out_layout, dst, c->written, direct);
     stats_seen = 0;
     for (size_t i = 0; i < c->fl.size(); ++i) {
         const vszip_filter* f = c->fl[i];

@@ -385,4 +385,125 @@ int run_adaptivebinarize(const FrameLayout& l, const char* a, size_t a_fs, const
     return 0;
 }
 
+// =========================================================================== ColorMap
+// DESIGN.md §4.8: plane 0 of an 8..16-bit integer clip through one of OpenCV's colormaps into the three planes of RGB24,
+// i = min(x >> (bits - 8), 255), (R, G, B) = table[i].  One 16-byte load (two for 9..16 bits) per 16 samples, 16 gathers, and
+// three 16-byte stores: 1 + 3 bytes per sample at 8 bits, 2 + 3 above, HBM-bound by construction.  Every CTA copies the 1 KB
+// table into shared memory once per bank, word [i][lane] (32 KB), so that each lane gathers from its own bank: a gather is
+// conflict-free whatever the indices.  Work items (row, 16 samples) of a CTA's rows are spread over all threads, so rows
+// narrower than 256 vectors keep every thread busy.
+static constexpr int CMT = 256, CM_UNROLL = 4, CM_ITEMS = 8;  // CM_ITEMS: work items per thread a CTA's rows are sized for
+
+struct ColorMapJob {
+    const char* src;
+    char* dst;
+    size_t src_fs, dst_fs;
+    size_t dst_off[3];     // R, G, B planes
+    int src_pitch, dst_pitch;
+    int w, h, rows;        // rows: per CTA
+    int shift;             // bits - 8
+    uint32_t lut[256];
+};
+
+// four table words -> the R, G and B bytes of four samples, one word per plane (7 PRMT)
+__device__ __forceinline__ void cm_pack4(uint32_t a, uint32_t b, uint32_t c, uint32_t d, uint32_t& r, uint32_t& g, uint32_t& bl) {
+    const uint32_t ab = __byte_perm(a, b, 0x5140), cd = __byte_perm(c, d, 0x5140);  // R0 R1 G0 G1 / R2 R3 G2 G3
+    r = __byte_perm(ab, cd, 0x5410);
+    g = __byte_perm(ab, cd, 0x7632);
+    bl = __byte_perm(__byte_perm(a, b, 0x0062), __byte_perm(c, d, 0x0062), 0x5410);
+}
+
+template <typename T>
+__device__ __forceinline__ uint32_t cm_index(uint32_t word, int e, int shift) {
+    if (sizeof(T) == 1) return __byte_perm(word, 0u, 0x4440 | e);
+    return min((e ? word >> 16 : word & 0xffffu) >> shift, 255u);
+}
+
+template <typename T>
+__global__ void __launch_bounds__(CMT) colormap_kernel(const __grid_constant__ ColorMapJob job) {
+    __shared__ uint32_t tab[256 * 32];
+    for (int i = threadIdx.x; i < 256 * 32; i += CMT) tab[i] = job.lut[i >> 5];
+    __syncthreads();
+    const uint32_t* my = tab + (threadIdx.x & 31);
+    constexpr int LOADS = (int)sizeof(T);  // 16-byte loads per 16 samples
+    const int y0 = (int)blockIdx.x * job.rows, nrows = min(job.rows, job.h - y0);
+    const char* src = job.src + (size_t)blockIdx.y * job.src_fs + (size_t)y0 * job.src_pitch;
+    char* dst = job.dst + (size_t)blockIdx.y * job.dst_fs + (size_t)y0 * job.dst_pitch;
+    char* const r_pl = dst + job.dst_off[0];
+    char* const g_pl = dst + job.dst_off[1];
+    char* const b_pl = dst + job.dst_off[2];
+    const int nvec = job.w / 16, items = nrows * nvec;
+    for (int it0 = threadIdx.x; it0 < items; it0 += CMT * CM_UNROLL) {
+        uint4 x[CM_UNROLL][LOADS];
+#pragma unroll
+        for (int u = 0; u < CM_UNROLL; ++u) {
+            const int it = min(it0 + u * CMT, items - 1);
+            const int y = it / nvec, v = it - y * nvec;
+            const uint4* p = reinterpret_cast<const uint4*>(src + (size_t)y * job.src_pitch) + v * LOADS;
+#pragma unroll
+            for (int l = 0; l < LOADS; ++l) x[u][l] = __ldg(p + l);
+        }
+#pragma unroll
+        for (int u = 0; u < CM_UNROLL; ++u) {
+            const int it = it0 + u * CMT;
+            if (it < items) {
+                const uint32_t* w = reinterpret_cast<const uint32_t*>(x[u]);
+                constexpr int SPW = 4 / (int)sizeof(T);  // samples per input word
+                uint32_t o[3][4];
+#pragma unroll
+                for (int q = 0; q < 4; ++q) {  // output word q: samples 4q .. 4q + 3
+                    uint32_t t[4];
+#pragma unroll
+                    for (int e = 0; e < 4; ++e) {
+                        const int s = 4 * q + e;
+                        t[e] = my[cm_index<T>(w[s / SPW], s % SPW, job.shift) << 5];
+                    }
+                    cm_pack4(t[0], t[1], t[2], t[3], o[0][q], o[1][q], o[2][q]);
+                }
+                const int y = it / nvec, v = it - y * nvec;
+                const size_t off = (size_t)y * job.dst_pitch + (size_t)v * 16;
+                *reinterpret_cast<uint4*>(r_pl + off) = make_uint4(o[0][0], o[0][1], o[0][2], o[0][3]);
+                *reinterpret_cast<uint4*>(g_pl + off) = make_uint4(o[1][0], o[1][1], o[1][2], o[1][3]);
+                *reinterpret_cast<uint4*>(b_pl + off) = make_uint4(o[2][0], o[2][1], o[2][2], o[2][3]);
+            }
+        }
+    }
+    // row tails (< 16 samples): one sample per thread
+    const int tail = job.w - nvec * 16;
+    for (int it = threadIdx.x; it < nrows * tail; it += CMT) {
+        const int y = it / tail, x0 = nvec * 16 + (it - y * tail);
+        const uint32_t s = reinterpret_cast<const T*>(src + (size_t)y * job.src_pitch)[x0];
+        const uint32_t t = my[cm_index<T>(s, 0, job.shift) << 5];
+        const size_t off = (size_t)y * job.dst_pitch + x0;
+        r_pl[off] = (char)(t & 0xffu);
+        g_pl[off] = (char)((t >> 8) & 0xffu);
+        b_pl[off] = (char)((t >> 16) & 0xffu);
+    }
+}
+
+int run_colormap(const FrameLayout& in, const char* src, size_t src_fs, const FrameLayout& out, char* dst, size_t dst_fs, int count,
+                 const uint32_t lut[256], cudaStream_t st) {
+    if (count <= 0) return 0;
+    if ((in.kind != K_U8 && in.kind != K_U16) || out.kind != K_U8 || out.nplanes != 3) return -1;
+    ColorMapJob job{};
+    job.src = src; job.dst = dst; job.src_fs = src_fs; job.dst_fs = dst_fs;
+    for (int p = 0; p < 3; ++p) job.dst_off[p] = out.pl[p].offset;
+    job.src_pitch = in.pl[0].pitch; job.dst_pitch = out.pl[0].pitch;
+    job.w = in.pl[0].w; job.h = in.pl[0].h;
+    job.shift = in.bits - 8;
+    job.rows = std::max(1, std::min(job.h, CMT * CM_ITEMS / std::max(1, job.w / 16)));
+    for (int i = 0; i < 256; ++i) job.lut[i] = lut[i];
+    const int ctas = (job.h + job.rows - 1) / job.rows;
+    for (int f0 = 0; f0 < count; f0 += 65535) {
+        const int nf = std::min(65535, count - f0);
+        ColorMapJob j = job;
+        j.src += (size_t)f0 * src_fs; j.dst += (size_t)f0 * dst_fs;
+        if (in.kind == K_U8) colormap_kernel<uint8_t><<<dim3(ctas, nf), CMT, 0, st>>>(j);
+        else colormap_kernel<uint16_t><<<dim3(ctas, nf), CMT, 0, st>>>(j);
+        count_launch();
+    }
+    VSZ_CUDA(cudaGetLastError());
+    return 0;
+}
+
 }  // namespace vsz
