@@ -271,6 +271,37 @@ def test_device_batch():
         props_close(got_av[i], oa.planeaverage(ca, [7, 9], clipb=cb))
 
 
+def test_device_batch_frame_limit():
+    """One call takes at most 32768 frames: above that the pair is not fused, and the separate PlaneMinMax call reports the limit."""
+    a = vz.DeviceClip("GRAY8", 16, 16, 32769)
+    mmf = vz.PlaneMinMaxFilter(a.info(), None, minthr=0.1, maxthr=0.1)
+    avf = vz.PlaneAverageFilter(a.info(), None, exclude=[3])
+    with pytest.raises(vz.Error, match="^PlaneMinMax: batches above 32768 frames are not supported$"):
+        mmf.run_device(a)
+    with pytest.raises(vz.Error, match="^PlaneAverage: batches above 32768 frames are not supported$"):
+        avf.run_device(a)
+    with pytest.raises(vz.Error, match="^PlaneMinMax: batches above 32768 frames are not supported$"):
+        vz.plane_stats_device(mmf, avf, a)
+
+
+def test_minmax_exact_env_and_the_pair(monkeypatch):
+    """VSZIP_MINMAX_EXACT=1, read on every call, turns off the sampled threshold path that the fused pair needs; PlaneMinMax without
+    thresholds is still fused.  Either way the props equal the separate calls."""
+    fmt, w, h, n = "GRAY16", 640, 360, 3
+    a = vz.DeviceClip(fmt, w, h, n)
+    a.fill_noise(seed=5)
+    avf = vz.PlaneAverageFilter(a.info(), None, exclude=[7])
+    for exact, mm_args, want_fused in (("1", dict(minthr=0.1, maxthr=0.2), False), ("1", dict(), True), ("0", dict(minthr=0.1, maxthr=0.2), True)):
+        monkeypatch.setenv("VSZIP_MINMAX_EXACT", exact)
+        mmf = vz.PlaneMinMaxFilter(a.info(), None, **mm_args)
+        got, fused = vz.plane_stats_device(mmf, avf, a)
+        assert fused == want_fused, (exact, mm_args)
+        sep_mm, sep_av = mmf.run_device(a), avf.run_device(a)
+        for i in range(n):
+            want = dict(sep_mm[i]); want.update(sep_av[i])
+            assert got[i] == want, (exact, mm_args, i)
+
+
 
 @pytest.mark.parametrize(("fmt", "w", "h", "n"), [("GRAY16", 1920, 1080, 5), ("YUV420P16", 640, 360, 4), ("GRAY10", 517, 243, 3), ("GRAYS", 640, 360, 2), ("GRAYS", 3840, 2160, 2), ("GRAY8", 517, 243, 2)])
 def test_minmax_and_average_from_one_read(fmt, w, h, n):

@@ -136,14 +136,15 @@ struct StatsRaw {  // one per (frame, processed plane), written by the kernels
     unsigned int pad;
 };
 size_t stats_scratch_bytes(int count, int nplanes);
-int run_planeminmax(const FrameLayout& l, const bool mask[3], const char* a, size_t a_fs, const char* b, size_t b_fs, int count,
-                    bool no_thr, float minthr, float maxthr, uint32_t hist_size, void* scratch, StatsRaw* out_dev, cudaStream_t st);
+// a and the clipb b (nullptr when there is none) share the frame stride fs
+int run_planeminmax(const FrameLayout& l, const bool mask[3], const char* a, const char* b, size_t fs, int count, bool no_thr,
+                    float minthr, float maxthr, uint32_t hist_size, void* scratch, StatsRaw* out_dev, cudaStream_t st);
 // PlaneMinMax + PlaneAverage of the same planes (and the same clipb b, or none) from one read: 0 done, 1 not eligible, < 0 error
-int run_planestats_fused(const FrameLayout& l, const bool mask[3], const char* a, size_t a_fs, const char* b, size_t b_fs, int count,
-                         bool no_thr, float minthr, float maxthr, uint32_t hist_size, const int32_t* excl, const float* excl_f, int nex,
+int run_planestats_fused(const FrameLayout& l, const bool mask[3], const char* a, const char* b, size_t fs, int count, bool no_thr,
+                         float minthr, float maxthr, uint32_t hist_size, const int32_t* excl, const float* excl_f, int nex,
                          bool same_float_sums, void* scratch, StatsRaw* out_mm, StatsRaw* out_avg, cudaStream_t st);
-int run_planeaverage(const FrameLayout& l, const bool mask[3], const char* a, size_t a_fs, const char* b, size_t b_fs, int count,
-                     const int32_t* excl_i, const float* excl_f, int nex, const int32_t* excl_i_dev, const float* excl_f_dev, void* scratch,
-                     StatsRaw* out_dev, cudaStream_t st);
+int run_planeaverage(const FrameLayout& l, const bool mask[3], const char* a, const char* b, size_t fs, int count, const int32_t* excl_i,
+                     const float* excl_f, int nex, const int32_t* excl_i_dev, const float* excl_f_dev, void* scratch, StatsRaw* out_dev,
+                     cudaStream_t st);
 
 }  // namespace vsz

@@ -796,10 +796,10 @@ static int run_pixels(const vszip_filter* f, int dev_index, const char* const in
 static int run_stats(const vszip_filter* f, int dev_index, const char* a, const char* b, size_t fs, int count, void* scratch,
                      StatsRaw* raw, cudaStream_t st) {
     if (f->kind == F_PLANEMINMAX)
-        return run_planeminmax(f->layout, f->process, a, fs, b, fs, count, f->no_thr, f->minthr, f->maxthr, f->hist_size, scratch, raw, st);
+        return run_planeminmax(f->layout, f->process, a, b, fs, count, f->no_thr, f->minthr, f->maxthr, f->hist_size, scratch, raw, st);
     const int32_t* xi; const float* xf;
     if (average_upload(f, dev_index, &xi, &xf)) return -1;
-    return run_planeaverage(f->layout, f->process, a, fs, b, fs, count, f->exclude_i.data(), f->exclude_f.data(), (int)f->exclude_i.size(),
+    return run_planeaverage(f->layout, f->process, a, b, fs, count, f->exclude_i.data(), f->exclude_f.data(), (int)f->exclude_i.size(),
                             xi, xf, scratch, raw, st);
 }
 
@@ -829,7 +829,7 @@ static int run_stats_pair(const vszip_filter* f, const vszip_filter* g, int dev_
     if (stats_pair(f, g) && bf == bg) {
         const vszip_filter* fm = f->kind == F_PLANEMINMAX ? f : g;
         const vszip_filter* fa = f->kind == F_PLANEMINMAX ? g : f;
-        const int rc = run_planestats_fused(fm->layout, fm->process, a, fs, bf, fs, count, fm->no_thr, fm->minthr, fm->maxthr, fm->hist_size,
+        const int rc = run_planestats_fused(fm->layout, fm->process, a, bf, fs, count, fm->no_thr, fm->minthr, fm->maxthr, fm->hist_size,
                                             fa->exclude_i.data(), fa->exclude_f.data(), (int)fa->exclude_i.size(), same_float_sums, scratch_f,
                                             fm == f ? raw_f : raw_g, fm == f ? raw_g : raw_f, st);
         if (rc == 0 && fused) *fused = true;

@@ -1085,19 +1085,38 @@ __global__ void __launch_bounds__(NT) minmax_bracket_kernel(const StatsJob j) {
 }
 
 // =========================================================================== host launchers
-// scratch layout (all zeroed before each call):
-//   counters  [2][count][np] u32 | coarse [count][np][256] u32 | fine [count][np][512] u32 | partials
+static constexpr int MAX_BATCH = 32768;  // frames per call
+
 static size_t align256(size_t v) { return (v + 255) / 256 * 256; }
+// The scratch regions, laid out from base (n = frames * planes): stats_scratch_bytes walks them from 0, make_job from the scratch
+// buffer.  Everything before `partials` is zeroed before each call.  Returns the bytes they take.
+static size_t lay_out_scratch(StatsJob& j, uintptr_t base, size_t n) {
+    uintptr_t p = base;
+    auto take = [&](size_t bytes) { const uintptr_t r = p; p += align256(bytes); return r; };
+    const uintptr_t c = take(3 * n * 4);  // counters, counters2, counters3
+    j.counters = (unsigned int*)c; j.counters2 = (unsigned int*)(c + n * 4); j.counters3 = (unsigned int*)(c + 2 * n * 4);
+    j.coarse = (unsigned int*)take(n * 256 * 4);
+    j.ssample = (unsigned int*)take(n * SBINS * 4);
+    j.fine = (unsigned int*)take(n * 512 * 4);
+    j.bfine = (unsigned int*)take(n * 2 * FINE_W * 4);
+    j.brackets = (Bracket*)take(n * sizeof(Bracket));
+    j.partials = (Partial*)take(n * MAX_CTAS_PER_PLANE * sizeof(Partial));
+    return p - base;
+}
 size_t stats_scratch_bytes(int count, int np) {
-    const size_t n = (size_t)count * np;
-    return align256(3 * n * 4) + align256(n * 256 * 4) + align256(n * SBINS * 4) + align256(n * 512 * 4) + align256(n * 2 * FINE_W * 4) + align256(n * sizeof(Bracket)) +
-           align256(n * MAX_CTAS_PER_PLANE * sizeof(Partial));
+    StatsJob j;
+    return lay_out_scratch(j, 0, (size_t)count * np);
+}
+// zeroes the scratch regions before `partials`
+static cudaError_t clear_scratch(const StatsJob& j, void* scratch, cudaStream_t st) {
+    return cudaMemsetAsync(scratch, 0, (const char*)j.partials - (const char*)scratch, st);
 }
 
-static StatsJob make_job(const FrameLayout& l, const bool mask[3], const char* a, size_t a_fs, const char* b, size_t b_fs, int count,
-                         void* scratch, StatsRaw* out, size_t* zero_bytes) {
+// a and b (clipb, nullptr when there is none) share the frame stride fs
+static StatsJob make_job(const FrameLayout& l, const bool mask[3], const char* a, const char* b, size_t fs, int count, void* scratch,
+                         StatsRaw* out) {
     StatsJob j{};
-    j.a = a; j.b = b; j.a_fs = a_fs; j.b_fs = b_fs;
+    j.a = a; j.b = b; j.a_fs = j.b_fs = fs;
     int cta = 0, scta = 0, bcta = 0, k = 0;
     for (int p = 0; p < l.nplanes; ++p) {
         if (!mask[p]) continue;
@@ -1130,79 +1149,13 @@ static StatsJob make_job(const FrameLayout& l, const bool mask[3], const char* a
         bcta += s.b_nctas;
     }
     j.nplanes = k; j.ctas_per_frame = cta; j.sample_ctas_per_frame = scta; j.bracket_ctas_per_frame = bcta;
-    const size_t n = (size_t)count * k;
-    char* sp = (char*)scratch;
-    j.counters = (unsigned int*)sp; j.counters2 = j.counters + n; j.counters3 = j.counters2 + n; sp += align256(3 * n * 4);
-    j.coarse = (unsigned int*)sp; sp += align256(n * 256 * 4);
-    j.ssample = (unsigned int*)sp; sp += align256(n * SBINS * 4);
-    j.fine = (unsigned int*)sp; sp += align256(n * 512 * 4);
-    j.bfine = (unsigned int*)sp; sp += align256(n * 2 * FINE_W * 4);
-    j.brackets = (Bracket*)sp; sp += align256(n * sizeof(Bracket));
-    *zero_bytes = (size_t)(sp - (char*)scratch);
-    j.partials = (Partial*)sp;
+    lay_out_scratch(j, (uintptr_t)scratch, (size_t)count * k);
     j.out = out;
     return j;
 }
 
-template <typename T>
-static int launch_minmax_t(StatsJob j, int count, bool no_thr, bool has_b, size_t bytes_per_frame, cudaStream_t st) {
-    if (count > 32768) { set_error("PlaneMinMax: batches above 32768 frames are not supported"); return -2; }
-    if (no_thr) {
-        const dim3 grid(j.ctas_per_frame, count);
-        if (has_b) stats_kernel<T, true, false><<<grid, NT, 0, st>>>(j);
-        else stats_kernel<T, false, false><<<grid, NT, 0, st>>>(j);
-        count_launch();
-    } else {
-        // Pass 2 re-reads what pass 1 read.  Running the pair on L2-sized chunks (<= 64 MB) was measured SLOWER on
-        // B200 (3-frame launches leave the GPU under-filled and add launch gaps: 42 k vs 77 k fps on 4K GRAY16), so the
-        // whole batch goes through each pass; single frames (<= 64 MB) still hit L2 on the second read.
-        (void)bytes_per_frame;
-        const int chunk = count;
-        const int np = j.nplanes;
-        for (int f0 = 0; f0 < count; f0 += chunk) {
-            const int nf = std::min(chunk, count - f0);
-            StatsJob c = j;
-            c.a += (size_t)f0 * j.a_fs;
-            if (has_b) c.b += (size_t)f0 * j.b_fs;
-            c.partials += (size_t)f0 * np * MAX_CTAS_PER_PLANE;
-            c.counters += (size_t)f0 * np; c.counters2 += (size_t)f0 * np;
-            c.coarse += (size_t)f0 * np * 256; c.fine += (size_t)f0 * np * 512;
-            c.out += (size_t)f0 * np;
-            c.counters3 += (size_t)f0 * np; c.ssample += (size_t)f0 * np * SBINS; c.bfine += (size_t)f0 * np * 2 * FINE_W;
-            c.brackets += (size_t)f0 * np;
-            const dim3 grid(j.ctas_per_frame, nf);
-            // VSZIP_MINMAX_EXACT=1 skips the sampled fast path (used by the tests to exercise the exact kernels)
-            const char* ev = getenv("VSZIP_MINMAX_EXACT");
-            const bool fast = !(ev && ev[0] == '1') && (long long)j.pl[0].w * j.pl[0].h < (1ll << 31);
-            if (fast) {
-                hist_sample_kernel<T><<<dim3(j.sample_ctas_per_frame, nf), NT, 0, st>>>(c);  // 1/16 of the lines
-                // one full read (also Diff); the lean variant needs every bin valid and both ranks > 0 on every plane
-                bool lean = (j.hist_size == 65536u) || (sizeof(T) == 1 && j.hist_size == 256u);
-                for (int k = 0; k < np; ++k) lean = lean && j.pl[k].tmin > 0u && j.pl[k].tmax > 0u;
-                const dim3 bgrid(j.bracket_ctas_per_frame, nf);
-                if (has_b) { if (lean) minmax_bracket_kernel<T, true, false><<<bgrid, NT, 0, st>>>(c); else minmax_bracket_kernel<T, true, true><<<bgrid, NT, 0, st>>>(c); }
-                else { if (lean) minmax_bracket_kernel<T, false, false><<<bgrid, NT, 0, st>>>(c); else minmax_bracket_kernel<T, false, true><<<bgrid, NT, 0, st>>>(c); }
-                count_launch(2);
-            }
-            // exact two-pass select: only for planes the fast path could not resolve (else immediate exit)
-            const dim3 xgrid(j.ctas_per_frame, fast ? std::min(nf, 8) : nf);
-            if (has_b && !fast) hist_coarse_kernel<T, true><<<xgrid, NT, 0, st>>>(c, nf);
-            else hist_coarse_kernel<T, false><<<xgrid, NT, 0, st>>>(c, nf);
-            hist_fine_kernel<T><<<xgrid, NT, 0, st>>>(c, nf);
-            count_launch(2);
-        }
-    }
-    VSZ_CUDA(cudaGetLastError());
-    return 0;
-}
-
-int run_planeminmax(const FrameLayout& l, const bool mask[3], const char* a, size_t a_fs, const char* b, size_t b_fs, int count,
-                    bool no_thr, float minthr, float maxthr, uint32_t hist_size, void* scratch, StatsRaw* out_dev, cudaStream_t st) {
-    size_t zero = 0;
-    StatsJob j = make_job(l, mask, a, a_fs, b, b_fs, count, scratch, out_dev, &zero);
-    if (j.ctas_per_frame == 0) return 0;
-    VSZ_CUDA(cudaMemsetAsync(scratch, 0, zero, st));
-    VSZ_CUDA(cudaMemsetAsync(out_dev, 0, sizeof(StatsRaw) * (size_t)count * j.nplanes, st));
+// hist_size and the thresholds of PlaneMinMax as the threshold kernels read them
+static void set_thresholds(StatsJob& j, uint32_t hist_size, float minthr, float maxthr) {
     j.hist_size = hist_size;
     int bits = 0;
     while ((1u << bits) < hist_size) ++bits;
@@ -1213,97 +1166,25 @@ int run_planeminmax(const FrameLayout& l, const bool mask[3], const char* a, siz
         j.pl[k].tmin = (unsigned int)(total * (double)minthr);  // trunc (src/filters/planeminmax.zig:40-41)
         j.pl[k].tmax = (unsigned int)(total * (double)maxthr);
     }
-    const bool has_b = b != nullptr;
-    size_t fb = 0;
-    for (int k = 0; k < j.nplanes; ++k) fb += (size_t)j.pl[k].w * j.pl[k].h * l.bps * (has_b ? 2 : 1);
-    switch (l.kind) {
-        case K_U8: return launch_minmax_t<uint8_t>(j, count, no_thr, has_b, fb, st);
-        case K_U16: return launch_minmax_t<uint16_t>(j, count, no_thr, has_b, fb, st);
-        case K_F16: return launch_minmax_t<__half>(j, count, no_thr, has_b, fb, st);
-        case K_F32: return launch_minmax_t<float>(j, count, no_thr, has_b, fb, st);
-    }
-    return -1;
 }
 
-// PlaneMinMax + PlaneAverage of the same planes from ONE read (SURVEY 8f rank 4).  run_planestats_fused returns 1 when the
-// combination is not eligible (the caller then runs the two reductions separately), 0 on success, < 0 on error.
-template <typename T, bool HAS_B>
-static int launch_fused_t(const StatsJob& j, int count, int m, cudaStream_t st) {
-    bool lean = (j.hist_size == 65536u) || (sizeof(T) == 1 && j.hist_size == 256u);
-    for (int k = 0; k < j.nplanes; ++k) lean = lean && j.pl[k].tmin > 0u && j.pl[k].tmax > 0u;
-    hist_sample_kernel<T><<<dim3(j.sample_ctas_per_frame, count), NT, 0, st>>>(j);
-    const dim3 bgrid(j.bracket_ctas_per_frame, count);
-#define VSZ_FUSED(M) (lean ? (void)(minmax_bracket_kernel<T, HAS_B, false, M><<<bgrid, NT, 0, st>>>(j)) \
-                           : (void)(minmax_bracket_kernel<T, HAS_B, true, M><<<bgrid, NT, 0, st>>>(j)))
-    switch (m) {
-        case 0: VSZ_FUSED(0); break;
-        case 1: VSZ_FUSED(1); break;
-        case 2: VSZ_FUSED(2); break;
-        case 3: VSZ_FUSED(3); break;
-        default: VSZ_FUSED(4); break;
-    }
-#undef VSZ_FUSED
-    // exact two-pass select for the planes the sampled path could not resolve (immediate exit otherwise)
-    const dim3 xgrid(j.ctas_per_frame, std::min(count, 8));
-    hist_coarse_kernel<T, false><<<xgrid, NT, 0, st>>>(j, count);
-    hist_fine_kernel<T><<<xgrid, NT, 0, st>>>(j, count);
-    count_launch(4);
-    VSZ_CUDA(cudaGetLastError());
-    return 0;
-}
-
-template <typename T, bool HAS_B>
-static int launch_both_nothr_t(const StatsJob& j, int count, cudaStream_t st) {
-    const dim3 grid(j.ctas_per_frame, count);
-    if (j.nex > 4) stats_kernel<T, HAS_B, true, true, true><<<grid, NT, 0, st>>>(j);
-    else stats_kernel<T, HAS_B, true, false, true><<<grid, NT, 0, st>>>(j);
-    count_launch();
-    VSZ_CUDA(cudaGetLastError());
-    return 0;
-}
-
-template <typename T>
-static int launch_both_nothr(const StatsJob& j, int count, cudaStream_t st) {
-    return j.b ? launch_both_nothr_t<T, true>(j, count, st) : launch_both_nothr_t<T, false>(j, count, st);
-}
-template <typename T>
-static int launch_fused(const StatsJob& j, int count, int m, cudaStream_t st) {
-    return j.b ? launch_fused_t<T, true>(j, count, m, st) : launch_fused_t<T, false>(j, count, m, st);
-}
-
-// Eligible: at most 32768 frames; without thresholds any sample type and up to 16 exclude values; with thresholds (sampled fast
-// path enabled) at most 4 distinct exclude values that can match a sample.  b (clipb, may be nullptr): both filters read it; Diff
-// is accumulated once, in the order of the separate kernels.  same_float_sums: fuse a float clip with thresholds only when its float
-// sums come out bit-identical to the separate calls - the bracket kernel walks a plane whose rows are back to back (no row padding)
-// as one run of vectors, which the separate PlaneAverage kernel does not, so such planes are not fused.  Always on with clipb, so
-// that a float Diff is the same whichever route ran.
-int run_planestats_fused(const FrameLayout& l, const bool mask[3], const char* a, size_t a_fs, const char* b, size_t b_fs, int count,
-                         bool no_thr, float minthr, float maxthr, uint32_t hist_size, const int32_t* excl, const float* excl_f, int nex,
-                         bool same_float_sums, void* scratch, StatsRaw* out_mm, StatsRaw* out_avg, cudaStream_t st) {
-    if (count <= 0 || count > 32768) return 1;
-    if (no_thr) {
-        if (nex > 16) return 1;
-        size_t zero = 0;
-        StatsJob j = make_job(l, mask, a, a_fs, b, b_fs, count, scratch, out_mm, &zero);
-        if (j.ctas_per_frame == 0) return 1;
-        VSZ_CUDA(cudaMemsetAsync(scratch, 0, zero, st));
-        j.out_avg = out_avg;
-        j.nex = nex;
-        for (int i = 0; i < nex; ++i) { j.excl_i[i] = excl[i]; j.excl_f[i] = excl_f[i]; }
-        switch (l.kind) {
-            case K_U8: return launch_both_nothr<uint8_t>(j, count, st);
-            case K_U16: return launch_both_nothr<uint16_t>(j, count, st);
-            case K_F16: return launch_both_nothr<__half>(j, count, st);
-            case K_F32: return launch_both_nothr<float>(j, count, st);
-        }
-        return -1;
-    }
+// Whether the threshold path may start with the line sample: every plane under 2^31 samples, and VSZIP_MINMAX_EXACT is not 1 (read on
+// every call; the tests set it to exercise the exact kernels).
+static bool sampled_path_allowed(const StatsJob& j) {
     const char* ev = getenv("VSZIP_MINMAX_EXACT");
-    if (ev && ev[0] == '1') return 1;
-    const bool flt = l.kind == K_F16 || l.kind == K_F32;
-    const int32_t top = l.kind == K_U8 ? 255 : 65535;
-    int32_t ex[4];
-    float exf[4];
+    if (ev && ev[0] == '1') return false;
+    for (int k = 0; k < j.nplanes; ++k)
+        if ((long long)j.pl[k].w * j.pl[k].h >= (1ll << 31)) return false;
+    return true;
+}
+
+// The exclude values that can match a sample of this kind, each once: integers outside the sample range are dropped, float lists are
+// deduplicated as floats.  Writes them to ex / exf and returns how many; -1 when there are more than 4 or the list has more than 16
+// entries.
+static int distinct_exclude(SampleKind kind, const int32_t* excl, const float* excl_f, int nex, int32_t* ex, float* exf) {
+    if (nex > 16) return -1;
+    const bool flt = kind == K_F16 || kind == K_F32;
+    const int32_t top = kind == K_U8 ? 255 : 65535;
     int m = 0;
     for (int i = 0; i < nex; ++i) {
         const int32_t v = excl[i];
@@ -1311,106 +1192,156 @@ int run_planestats_fused(const FrameLayout& l, const bool mask[3], const char* a
         bool dup = false;
         for (int t = 0; t < m; ++t) dup = dup || (flt ? exf[t] == excl_f[i] : ex[t] == v);
         if (dup) continue;
-        if (m == 4) return 1;
+        if (m == 4) return -1;
         ex[m] = v; exf[m] = excl_f[i];
         ++m;
     }
-    size_t zero = 0;
-    StatsJob j = make_job(l, mask, a, a_fs, b, b_fs, count, scratch, out_mm, &zero);
-    if (j.ctas_per_frame == 0) return 1;
-    for (int k = 0; k < j.nplanes; ++k) {
-        if ((long long)j.pl[k].w * j.pl[k].h >= (1ll << 31)) return 1;
-        const int nvec = j.pl[k].w / (16 / l.bps);  // minmax_bracket_kernel's `contiguous` test
-        if (flt && (same_float_sums || b) && nvec > 0 && j.pl[k].a_pitch == nvec * 16) return 1;
-    }
-    VSZ_CUDA(cudaMemsetAsync(scratch, 0, zero, st));
-    VSZ_CUDA(cudaMemsetAsync(out_mm, 0, sizeof(StatsRaw) * (size_t)count * j.nplanes, st));
-    j.out_avg = out_avg;
-    j.hist_size = hist_size;
-    int bits = 0;
-    while ((1u << bits) < hist_size) ++bits;
-    j.shift = bits > 8 ? bits - 8 : 0;
-    j.sshift = bits > SBITS ? bits - SBITS : 0;
-    for (int k = 0; k < j.nplanes; ++k) {
-        const double total = (double)((uint32_t)j.pl[k].w * (uint32_t)j.pl[k].h);
-        j.pl[k].tmin = (unsigned int)(total * (double)minthr);
-        j.pl[k].tmax = (unsigned int)(total * (double)maxthr);
-    }
-    j.nex = m;
-    for (int i = 0; i < m; ++i) { j.excl_i[i] = ex[i]; j.excl_f[i] = exf[i]; }
-    switch (l.kind) {
-        case K_U8: return launch_fused<uint8_t>(j, count, m, st);
-        case K_U16: return launch_fused<uint16_t>(j, count, m, st);
-        case K_F16: return launch_fused<__half>(j, count, m, st);
-        case K_F32: return launch_fused<float>(j, count, m, st);
-    }
-    return -1;
+    return m;
 }
 
-template <typename T>
-static int launch_avg_t(const StatsJob& j, int count, bool has_b, cudaStream_t st) {
-    if (count > 32768) { set_error("PlaneAverage: batches above 32768 frames are not supported"); return -2; }
-    const dim3 grid(j.ctas_per_frame, count);
-    if constexpr (std::is_same<T, uint16_t>::value) {
-        if (!has_b) {  // packed path: needs at most 4 distinct exclude values inside the sample range
-            StatsJob q = j;
-            int m = 0;
-            bool fits = true;
-            for (int i = 0; i < j.nex && fits; ++i) {
-                const int32_t v = i < 16 ? j.excl_i[i] : 0;
-                if (i >= 16) { fits = false; break; }
-                if (v < 0 || v > 65535) continue;  // can never match a sample
-                bool dup = false;
-                for (int t = 0; t < m; ++t) dup = dup || q.excl_i[t] == v;
-                if (dup) continue;
-                if (m == 4) { fits = false; break; }
-                q.excl_i[m++] = v;
-            }
-            if (fits) {
-                switch (m) {
-                    case 0: average_u16_kernel<0><<<grid, NT, 0, st>>>(q); break;
-                    case 1: average_u16_kernel<1><<<grid, NT, 0, st>>>(q); break;
-                    case 2: average_u16_kernel<2><<<grid, NT, 0, st>>>(q); break;
-                    case 3: average_u16_kernel<3><<<grid, NT, 0, st>>>(q); break;
-                    default: average_u16_kernel<4><<<grid, NT, 0, st>>>(q); break;
-                }
-                count_launch();
-                VSZ_CUDA(cudaGetLastError());
-                return 0;
-            }
-        }
+// Calls launch(Type<T>{}, std::bool_constant<HAS_B>{}) for the clip's sample type and whether a clipb is read, then checks the launches.
+template <typename T> struct Type { using type = T; };
+template <class F> static int dispatch(SampleKind kind, bool has_b, F&& launch) {
+    auto with_b = [&](auto t) { if (has_b) launch(t, std::true_type{}); else launch(t, std::false_type{}); };
+    switch (kind) {
+        case K_U8: with_b(Type<uint8_t>{}); break;
+        case K_U16: with_b(Type<uint16_t>{}); break;
+        case K_F16: with_b(Type<__half>{}); break;
+        case K_F32: with_b(Type<float>{}); break;
+        default: return -1;
     }
-    if (j.nex > 4) {
-        if (has_b) stats_kernel<T, true, true, true><<<grid, NT, 0, st>>>(j);
-        else stats_kernel<T, false, true, true><<<grid, NT, 0, st>>>(j);
-    } else {
-        if (has_b) stats_kernel<T, true, true><<<grid, NT, 0, st>>>(j);
-        else stats_kernel<T, false, true><<<grid, NT, 0, st>>>(j);
-    }
-    count_launch();
     VSZ_CUDA(cudaGetLastError());
     return 0;
 }
 
-int run_planeaverage(const FrameLayout& l, const bool mask[3], const char* a, size_t a_fs, const char* b, size_t b_fs, int count,
-                     const int32_t* excl_i, const float* excl_f, int nex, const int32_t* excl_i_dev, const float* excl_f_dev, void* scratch,
-                     StatsRaw* out_dev, cudaStream_t st) {
-    size_t zero = 0;
-    StatsJob j = make_job(l, mask, a, a_fs, b, b_fs, count, scratch, out_dev, &zero);
+// The single-read kernel: raw min/max (PlaneMinMax without thresholds), PlaneAverage, or both (BOTH).
+template <typename T, bool HAS_B, bool AVERAGE, bool BOTH = false>
+static void launch_stats(const StatsJob& j, int count, cudaStream_t st) {
+    const dim3 grid(j.ctas_per_frame, count);
+    if constexpr (!AVERAGE) stats_kernel<T, HAS_B, false><<<grid, NT, 0, st>>>(j);
+    else if (j.nex > 4) stats_kernel<T, HAS_B, true, true, BOTH><<<grid, NT, 0, st>>>(j);
+    else stats_kernel<T, HAS_B, true, false, BOTH><<<grid, NT, 0, st>>>(j);
+    count_launch();
+}
+
+// The threshold path of PlaneMinMax, with PlaneAverage's exclude compares unrolled AVG times in the bracket kernel (-1: PlaneMinMax
+// alone).  Sampled: the line sample brackets both ranks, one full read resolves most planes, and the exact two-pass select takes the
+// rest.  Otherwise (PlaneMinMax alone): the exact two-pass select on every plane.
+template <typename T, bool HAS_B, int AVG>
+static void launch_threshold(const StatsJob& j, int count, bool sampled, cudaStream_t st) {
+    // Pass 2 re-reads what pass 1 read.  Running the pair on L2-sized chunks (<= 64 MB) was measured SLOWER on
+    // B200 (3-frame launches leave the GPU under-filled and add launch gaps: 42 k vs 77 k fps on 4K GRAY16), so the
+    // whole batch goes through each pass; single frames (<= 64 MB) still hit L2 on the second read.
+    if (sampled) {
+        hist_sample_kernel<T><<<dim3(j.sample_ctas_per_frame, count), NT, 0, st>>>(j);  // 1/16 of the lines
+        // one full read (also Diff); the lean variant needs every bin valid and both ranks > 0 on every plane
+        bool lean = (j.hist_size == 65536u) || (sizeof(T) == 1 && j.hist_size == 256u);
+        for (int k = 0; k < j.nplanes; ++k) lean = lean && j.pl[k].tmin > 0u && j.pl[k].tmax > 0u;
+        const dim3 bgrid(j.bracket_ctas_per_frame, count);
+        if (lean) minmax_bracket_kernel<T, HAS_B, false, AVG><<<bgrid, NT, 0, st>>>(j);
+        else minmax_bracket_kernel<T, HAS_B, true, AVG><<<bgrid, NT, 0, st>>>(j);
+        count_launch(2);
+    }
+    // exact two-pass select: after the sampled path only for the planes it could not resolve (else immediate exit)
+    const dim3 xgrid(j.ctas_per_frame, sampled ? std::min(count, 8) : count);
+    if (sampled) hist_coarse_kernel<T, false><<<xgrid, NT, 0, st>>>(j, count);  // Diff came from the bracket kernel
+    else hist_coarse_kernel<T, HAS_B><<<xgrid, NT, 0, st>>>(j, count);
+    hist_fine_kernel<T><<<xgrid, NT, 0, st>>>(j, count);
+    count_launch(2);
+}
+
+int run_planeminmax(const FrameLayout& l, const bool mask[3], const char* a, const char* b, size_t fs, int count, bool no_thr,
+                    float minthr, float maxthr, uint32_t hist_size, void* scratch, StatsRaw* out_dev, cudaStream_t st) {
+    StatsJob j = make_job(l, mask, a, b, fs, count, scratch, out_dev);
+    if (j.ctas_per_frame == 0) return 0;
+    VSZ_CUDA(clear_scratch(j, scratch, st));
+    VSZ_CUDA(cudaMemsetAsync(out_dev, 0, sizeof(StatsRaw) * (size_t)count * j.nplanes, st));
+    if (count > MAX_BATCH) { set_error("PlaneMinMax: batches above %d frames are not supported", MAX_BATCH); return -2; }
+    set_thresholds(j, hist_size, minthr, maxthr);
+    return dispatch(l.kind, b != nullptr, [&](auto t, auto hb) {
+        using T = typename decltype(t)::type;
+        if (no_thr) launch_stats<T, decltype(hb)::value, false>(j, count, st);
+        else launch_threshold<T, decltype(hb)::value, -1>(j, count, sampled_path_allowed(j), st);
+    });
+}
+
+// PlaneMinMax + PlaneAverage of the same planes from ONE read (SURVEY 8f rank 4).  run_planestats_fused returns 1 when the
+// combination is not eligible (the caller then runs the two reductions separately), 0 on success, < 0 on error.
+// Eligible: at most 32768 frames; without thresholds any sample type and up to 16 exclude values; with thresholds (sampled fast
+// path enabled) at most 4 distinct exclude values that can match a sample.  b (clipb, may be nullptr): both filters read it; Diff
+// is accumulated once, in the order of the separate kernels.  same_float_sums: fuse a float clip with thresholds only when its float
+// sums come out bit-identical to the separate calls - the bracket kernel walks a plane whose rows are back to back (no row padding)
+// as one run of vectors, which the separate PlaneAverage kernel does not, so such planes are not fused.  Always on with clipb, so
+// that a float Diff is the same whichever route ran.
+int run_planestats_fused(const FrameLayout& l, const bool mask[3], const char* a, const char* b, size_t fs, int count, bool no_thr,
+                         float minthr, float maxthr, uint32_t hist_size, const int32_t* excl, const float* excl_f, int nex,
+                         bool same_float_sums, void* scratch, StatsRaw* out_mm, StatsRaw* out_avg, cudaStream_t st) {
+    if (count <= 0 || count > MAX_BATCH) return 1;
+    StatsJob j = make_job(l, mask, a, b, fs, count, scratch, out_mm);
+    if (j.ctas_per_frame == 0) return 1;
+    j.out_avg = out_avg;
+    if (no_thr) {
+        if (nex > 16) return 1;
+        VSZ_CUDA(clear_scratch(j, scratch, st));
+        j.nex = nex;
+        for (int i = 0; i < nex; ++i) { j.excl_i[i] = excl[i]; j.excl_f[i] = excl_f[i]; }
+        return dispatch(l.kind, b != nullptr, [&](auto t, auto hb) {
+            launch_stats<typename decltype(t)::type, decltype(hb)::value, true, true>(j, count, st);
+        });
+    }
+    j.nex = distinct_exclude(l.kind, excl, excl_f, nex, j.excl_i, j.excl_f);
+    if (j.nex < 0 || !sampled_path_allowed(j)) return 1;
+    const bool flt = l.kind == K_F16 || l.kind == K_F32;
+    for (int k = 0; k < j.nplanes; ++k) {
+        const int nvec = j.pl[k].w / (16 / l.bps);  // minmax_bracket_kernel's `contiguous` test
+        if (flt && (same_float_sums || b) && nvec > 0 && j.pl[k].a_pitch == nvec * 16) return 1;
+    }
+    VSZ_CUDA(clear_scratch(j, scratch, st));
+    VSZ_CUDA(cudaMemsetAsync(out_mm, 0, sizeof(StatsRaw) * (size_t)count * j.nplanes, st));
+    set_thresholds(j, hist_size, minthr, maxthr);
+    return dispatch(l.kind, b != nullptr, [&](auto t, auto hb) {
+        using T = typename decltype(t)::type;
+        constexpr bool HAS_B = decltype(hb)::value;
+        switch (j.nex) {
+            case 0: launch_threshold<T, HAS_B, 0>(j, count, true, st); break;
+            case 1: launch_threshold<T, HAS_B, 1>(j, count, true, st); break;
+            case 2: launch_threshold<T, HAS_B, 2>(j, count, true, st); break;
+            case 3: launch_threshold<T, HAS_B, 3>(j, count, true, st); break;
+            default: launch_threshold<T, HAS_B, 4>(j, count, true, st); break;
+        }
+    });
+}
+
+int run_planeaverage(const FrameLayout& l, const bool mask[3], const char* a, const char* b, size_t fs, int count, const int32_t* excl_i,
+                     const float* excl_f, int nex, const int32_t* excl_i_dev, const float* excl_f_dev, void* scratch, StatsRaw* out_dev,
+                     cudaStream_t st) {
+    StatsJob j = make_job(l, mask, a, b, fs, count, scratch, out_dev);
     if (j.ctas_per_frame == 0) return 0;
     if (nex > 16 && (!excl_i_dev || !excl_f_dev)) { set_error("PlaneAverage: internal error, long exclude list not uploaded"); return -2; }
-    VSZ_CUDA(cudaMemsetAsync(scratch, 0, zero, st));
+    VSZ_CUDA(clear_scratch(j, scratch, st));
+    if (count > MAX_BATCH) { set_error("PlaneAverage: batches above %d frames are not supported", MAX_BATCH); return -2; }
     j.nex = nex;
     for (int i = 0; i < std::min(nex, 16); ++i) { j.excl_i[i] = excl_i[i]; j.excl_f[i] = excl_f[i]; }
     j.excl_i_more = excl_i_dev; j.excl_f_more = excl_f_dev;  // the whole list (entries >= 16 are read from here)
-    const bool has_b = b != nullptr;
-    switch (l.kind) {
-        case K_U8: return launch_avg_t<uint8_t>(j, count, has_b, st);
-        case K_U16: return launch_avg_t<uint16_t>(j, count, has_b, st);
-        case K_F16: return launch_avg_t<__half>(j, count, has_b, st);
-        case K_F32: return launch_avg_t<float>(j, count, has_b, st);
-    }
-    return -1;
+    return dispatch(l.kind, b != nullptr, [&](auto t, auto hb) {
+        using T = typename decltype(t)::type;
+        constexpr bool HAS_B = decltype(hb)::value;
+        // packed path for 16-bit integer clips: at most 4 distinct exclude values inside the sample range
+        if constexpr (std::is_same<T, uint16_t>::value && !HAS_B) {
+            StatsJob q = j;
+            const int m = distinct_exclude(l.kind, excl_i, excl_f, nex, q.excl_i, q.excl_f);
+            const dim3 grid(j.ctas_per_frame, count);
+            switch (m) {
+                case 0: average_u16_kernel<0><<<grid, NT, 0, st>>>(q); break;
+                case 1: average_u16_kernel<1><<<grid, NT, 0, st>>>(q); break;
+                case 2: average_u16_kernel<2><<<grid, NT, 0, st>>>(q); break;
+                case 3: average_u16_kernel<3><<<grid, NT, 0, st>>>(q); break;
+                case 4: average_u16_kernel<4><<<grid, NT, 0, st>>>(q); break;
+            }
+            if (m >= 0) { count_launch(); return; }
+        }
+        launch_stats<T, HAS_B, true>(j, count, st);
+    });
 }
 
 }  // namespace vsz
