@@ -28,7 +28,7 @@
 extern "C" {
 #endif
 
-#define VSZIP_CUDA_ABI_VERSION 5  /* 2: + vszip_chain_*, vszip_limiter_*; 3: + vszip_limitfilter_*, vszip_adaptivebinarize_*, vszip_planestats_device; 4: + vszip_cuda_host_forget, vszip_cuda_host_registered_bytes, vszip_cuda_host_register_limit; 5: + vszip_cuda_reserve, and additions that leave every earlier entry point unchanged: vszip_chain_create2, vszip_planestats_device_b, vszip_cuda_transfer_bytes, vszip_clahe_create, vszip_clahe_get_frame, vszip_clahe_device, vszip_colormap_create, vszip_colormap_get_frame, vszip_colormap_device, vszip_colormap_get_lut, vszip_filter_output_info (a caller that needs them resolves them by name) */
+#define VSZIP_CUDA_ABI_VERSION 5  /* 2: + vszip_chain_*, vszip_limiter_*; 3: + vszip_limitfilter_*, vszip_adaptivebinarize_*, vszip_planestats_device; 4: + vszip_cuda_host_forget, vszip_cuda_host_registered_bytes, vszip_cuda_host_register_limit; 5: + vszip_cuda_reserve, and additions that leave every earlier entry point unchanged: vszip_chain_create2, vszip_planestats_device_b, vszip_cuda_transfer_bytes, vszip_clahe_create, vszip_clahe_get_frame, vszip_clahe_device, vszip_colormap_create, vszip_colormap_get_frame, vszip_colormap_device, vszip_colormap_get_lut, vszip_filter_output_info, vszip_packrgb_create, vszip_packrgb_get_frame, vszip_packrgb_device (a caller that needs them resolves them by name) */
 
 /* VapourSynth4.h values (VSColorFamily / VSSampleType) so the Zig glue can pass vi.format as is. */
 enum { VSZIP_CF_GRAY = 1, VSZIP_CF_RGB = 2, VSZIP_CF_YUV = 3 };
@@ -264,12 +264,25 @@ int vszip_colormap_get_frame(const vszip_filter* f, int32_t n, const vszip_frame
 /* The selected table, rgb[3 * i + c] = channel c (R, G, B) of index i (for inspection and tests). */
 int vszip_colormap_get_lut(const vszip_filter* f, uint8_t rgb[768]);
 
+/* ------------------------------------------------------------------ PackRGB
+ * The three planes of an RGB24 or RGB30 clip packed into one 32-bit plane in the layout of Qt's QImage, so that a previewer can hand
+ * the frame to Qt without a packing pass of its own.  The output is GRAY32 (integer, 32 bits, one plane) of the same size and length
+ * (vszip_filter_output_info); per pixel
+ *   RGB24: 0xFF000000 | R << 16 | G << 8 | B                                  (QImage::Format_RGB32: bytes B, G, R, 0xFF in memory)
+ *   RGB30: 0xC0000000 | min(R, 1023) << 20 | min(G, 1023) << 10 | min(B, 1023) (QImage::Format_RGB30 with the two top bits set)
+ * Samples above 1023 in an RGB30 clip's u16 containers are clamped, so they never spill into a neighbouring field.  Every other
+ * format fails with "PackRGB: only RGB24 and RGB30 clips are supported."  Argument string: "clip:vnode;".  The props are the source
+ * frame's, unchanged.  The name, argument string and message are this library's. */
+vszip_filter* vszip_packrgb_create(const vszip_video_info* vi);
+/* src: the three RGB planes; dst: the one plane of a GRAY32 frame, written. */
+int vszip_packrgb_get_frame(const vszip_filter* f, int32_t n, const vszip_frame* src, vszip_frame* dst);
+
 /* ------------------------------------------------------------------ common filter calls */
 void vszip_filter_free(vszip_filter* f);                         /* replaces xxxFree */
 int vszip_filter_planes(const vszip_filter* f, int32_t process[3]); /* d.planes after create: the planes the filter reads */
-/* The format of the clip the filter's node returns (the output node's vi): the input format for every filter except ColorMap,
- * whose output is RGB24.  A filter that changes the format writes every plane of its output; any other pixel filter writes the
- * planes vszip_filter_planes reports and leaves the others to the input frame. */
+/* The format of the clip the filter's node returns (the output node's vi): the input format for every filter except ColorMap and
+ * PackRGB, whose outputs are RGB24 and GRAY32.  A filter that changes the format writes every plane of its output; any other pixel
+ * filter writes the planes vszip_filter_planes reports and leaves the others to the input frame. */
 int vszip_filter_output_info(const vszip_filter* f, vszip_video_info* out);
 
 /* ------------------------------------------------------------------ device-resident clips
@@ -293,8 +306,8 @@ void* vszip_dev_clip_plane_ptr(const vszip_dev_clip* c, int32_t frame, int32_t p
 /* Batched, asynchronous, device-resident execution on frames [first, first+count) of the clips.
  * `stream` is a cudaStream_t (as void*) on the clips' device, or NULL for the library's own stream
  * of that device; work is enqueued and NOT synchronised (use vszip_cuda_stream_sync or your own
- * event).  src and dst must have the same format/size and live on the same device; for ColorMap dst has the filter's output format
- * (vszip_filter_output_info). */
+ * event).  src and dst must have the same format/size and live on the same device; for ColorMap and PackRGB dst has the filter's
+ * output format (vszip_filter_output_info). */
 int vszip_boxblur_device(const vszip_filter* f, const vszip_dev_clip* src, vszip_dev_clip* dst,
                          int32_t first, int32_t count, void* stream);
 int vszip_bilateral_device(const vszip_filter* f, const vszip_dev_clip* src, const vszip_dev_clip* ref,
@@ -331,6 +344,8 @@ int vszip_clahe_device(const vszip_filter* f, const vszip_dev_clip* src, vszip_d
                        int32_t first, int32_t count, void* stream);
 int vszip_colormap_device(const vszip_filter* f, const vszip_dev_clip* src, vszip_dev_clip* dst,
                           int32_t first, int32_t count, void* stream);
+int vszip_packrgb_device(const vszip_filter* f, const vszip_dev_clip* src, vszip_dev_clip* dst,
+                         int32_t first, int32_t count, void* stream);
 int vszip_cuda_stream_sync(int32_t device, void* stream);
 
 /* ------------------------------------------------------------------ fused chains of vszip filters (SURVEY 8f rank 1)
@@ -340,7 +355,7 @@ int vszip_cuda_stream_sync(int32_t device, void* stream);
  * chain's SOURCE frame instead of its immediate input and calls this.  Results are identical to calling the
  * per-filter get_frame functions one after the other.
  *  - filters: 1..16 handles in evaluation order, each created for the format of the values it reads (the source's, or, after a
- *    ColorMap, RGB24) and without ref/clipb;
+ *    ColorMap, RGB24, or, after a PackRGB, GRAY32) and without ref/clipb;
  *    the chain borrows them (they must outlive it).  Two "diamond" elements are accepted as well, with the chain's
  *    SOURCE frame as their second clip: a LimitFilter created without ref (flt = the chain's current value, src = the
  *    source frame: `flt = src.vszip.X(); flt.vszip.LimitFilter(src)`) and an AdaptiveBinarize (clip = the source frame,
@@ -366,7 +381,7 @@ vszip_chain* vszip_chain_create(const vszip_filter* const* filters, int32_t coun
  * diamond elements.  An adjacent PlaneMinMax + PlaneAverage that read the same value with the same planes and clipb (or none) share
  * one read when vszip_planestats_device_b would fuse them, with bit-identical results.  Value 0 has filter 0's format and value k
  * the output format of filter k - 1 (vszip_filter_output_info); every element must have been created for the format of each value
- * it reads.  After a ColorMap every plane of the result is written, and dst has the result's format. */
+ * it reads.  After a ColorMap or a PackRGB every plane of the result is written, and dst has the result's format. */
 vszip_chain* vszip_chain_create2(const vszip_filter* const* filters, int32_t count, const int32_t* input, const int32_t* second,
                                  const int32_t* third);
 void vszip_chain_free(vszip_chain* c);

@@ -2,7 +2,7 @@
 Not the contract line (bench.py prints that); results go to stdout as JSON and, with --out, to a file.
 usage: python scripts/bench_extras.py [--frames N] [--reps R] [--only REGEX] [--out profiles/bench_extras_rXX.json]
 --only clahe: the CLAHE group (device batches, get_frame on pinned frames, and OpenCV on every host core for comparison);
---only colormap: the same for ColorMap."""
+--only colormap: the same for ColorMap; --only packrgb: the same for PackRGB, next to a numpy pack on every host core."""
 import argparse
 import json
 import sys
@@ -307,6 +307,72 @@ def colormap_cfgs():
 
 
 colormap_cfgs()
+
+
+def _np_packrgb(job):
+    r, g, b, bits = job
+    u = lambda p: np.minimum(p.astype(np.uint32), 1023) if bits == 10 else p.astype(np.uint32)
+    top, sh = (0xC0000000, 10) if bits == 10 else (0xFF000000, 8)
+    return np.uint32(top) | u(r) << np.uint32(2 * sh) | u(g) << np.uint32(sh) | u(b)
+
+
+def packrgb_cfgs():
+    """PackRGB: device-resident batches (frames/s; algorithmic bytes = the three planes read + 4 * w * h written), get_frame on pinned
+    host frames from 8 threads, and the same pack in numpy over every host core (one frame per worker) for comparison.  Each batch
+    (1.8 GB and more) is larger than the L2."""
+    import ctypes as C
+    import multiprocessing
+    import os
+    import time
+    from concurrent.futures import ProcessPoolExecutor, ThreadPoolExecutor
+
+    lib = vz.load_library()
+    for fmt, w, h in (("RGB24", 1920, 1080), ("RGB30", 3840, 2160)):
+        tag = f"packrgb {fmt} {w}x{h} noise"
+        if skip(tag):
+            continue
+        frames = N if fmt == "RGB24" else max(8, N // 4)
+        src, dst = vz.DeviceClip(fmt, w, h, frames), vz.DeviceClip("GRAY32", w, h, frames)
+        src.fill_noise(1234)
+        algo = src.frame_bytes + 4 * w * h
+        f = vz.PackRGBFilter(src.info())
+        ms = timed(lambda: f.run_device(src, dst, first=0, count=frames, stream=st.cuda_stream), args.reps)
+        record(f"{tag} device batch", fmt, w, h, frames, algo, ms)
+        host = [src.download(i) for i in range(4)]
+
+        def pinned(shape, dtype):
+            t = torch.empty(int(np.prod(shape)) * np.dtype(dtype).itemsize, dtype=torch.uint8, pin_memory=True)
+            return t.numpy().view(dtype).reshape(shape), t
+        ins = [[pinned(p.shape, p.dtype) for p in fr] for fr in host]
+        for fr, pf in zip(host, ins):
+            for p, (q, _) in zip(fr, pf):
+                q[...] = p
+        outs = [pinned((h, w), np.uint32) for _ in range(8)]
+
+        def one(i):
+            s = vz._cframe([q for q, _ in ins[i % 4]])
+            d = vz._cframe([outs[i % 8][0]])
+            vz._check(lib.vszip_packrgb_get_frame(f.handle, i, C.byref(s), C.byref(d)))
+        n_e2e = 4 * frames
+        with ThreadPoolExecutor(8) as ex:
+            list(ex.map(one, range(16)))
+            t0 = time.perf_counter()
+            list(ex.map(one, range(n_e2e)))
+            e2e = time.perf_counter() - t0
+        record(f"{tag} get_frame, pinned frames, 8 threads (end to end)", fmt, w, h, n_e2e, algo, e2e * 1e3)
+        workers = os.cpu_count() or 1
+        n_cpu = 2 * workers
+        bits = vz.FORMATS[fmt].bits_per_sample
+        with ProcessPoolExecutor(workers, mp_context=multiprocessing.get_context("fork")) as ex:
+            list(ex.map(_np_packrgb, [(*host[0], bits)] * workers))
+            t0 = time.perf_counter()
+            list(ex.map(_np_packrgb, [(*host[i % 4], bits) for i in range(n_cpu)]))
+            cpu = time.perf_counter() - t0
+        record(f"{tag} numpy pack on {workers} host cores", fmt, w, h, n_cpu, algo, cpu * 1e3)
+        src.free(); dst.free()
+
+
+packrgb_cfgs()
 
 
 def _gpu():

@@ -2,7 +2,7 @@
 
 The product is the C-ABI library (include/vszip_cuda.h, built into lib/libvszip_cuda.so from
 csrc/*.cu).  This module is the thin host side used where the reference would be driven through
-VapourSynth: it mirrors the `clip.vszip.BoxBlur / Bilateral / PlaneMinMax / PlaneAverage / ... / CLAHE / ColorMap` call
+VapourSynth: it mirrors the `clip.vszip.BoxBlur / Bilateral / PlaneMinMax / PlaneAverage / ... / CLAHE / ColorMap / PackRGB` call
 surface (same names, arguments, defaults, frame props and error messages; src/vszip.zig:46-69,
 :184-199) on top of a minimal clip/frame model, so the parity tests read like the reference's own
 tests (tests/test_boxblur.py etc. of the reference).  All arithmetic happens in the CUDA library;
@@ -159,6 +159,9 @@ ABI = {
     "vszip_colormap_device": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int32, _P]),
     "vszip_colormap_get_lut": (C.c_int, [_P, C.POINTER(C.c_uint8 * 768)]),
     "vszip_filter_output_info": (C.c_int, [_P, C.POINTER(_VideoInfo)]),
+    "vszip_packrgb_create": (_P, [C.POINTER(_VideoInfo)]),
+    "vszip_packrgb_get_frame": (C.c_int, [_P, C.c_int32, C.POINTER(_Frame), C.POINTER(_Frame)]),
+    "vszip_packrgb_device": (C.c_int, [_P, _P, _P, C.c_int32, C.c_int32, _P]),
     "vszip_chain_create": (_P, [C.POINTER(_P), C.c_int32]),
     "vszip_chain_create2": (_P, [C.POINTER(_P), C.c_int32, C.POINTER(C.c_int32), C.POINTER(C.c_int32), C.POINTER(C.c_int32)]),
     "vszip_chain_free": (None, [_P]),
@@ -589,6 +592,19 @@ class ColorMapFilter(_Filter):
         self._device(load_library().vszip_colormap_device, (src, dst), first, count, stream)
 
 
+class PackRGBFilter(_Filter):
+    """RGB24 / RGB30 packed into one GRAY32 plane in Qt's QImage layouts: 0xFFRRGGBB, or 0xC0000000 | R << 20 | G << 10 | B with
+    10-bit samples clamped to 1023 (DESIGN.md §4.9)."""
+
+    GET_FRAME = "vszip_packrgb_get_frame"
+
+    def __init__(self, vi: _VideoInfo):
+        super().__init__(load_library().vszip_packrgb_create(C.byref(vi)))
+
+    def run_device(self, src: "DeviceClip", dst: "DeviceClip", first=0, count=None, stream=None):
+        self._device(load_library().vszip_packrgb_device, (src, dst), first, count, stream)
+
+
 class _Namespace:
     """`clip.vszip` / `core.vszip`: the plugin functions with the reference's argument names."""
 
@@ -620,6 +636,12 @@ class _Namespace:
         if clip is None:
             raise Error("clip argument is required")
         return _node(ColorMapFilter(clip._info(), color), clip, set_props={"_ColorRange": 0, "_Matrix": 0})
+
+    def PackRGB(self, *pos, **kw) -> VideoNode:
+        clip, = self._bind(("clip",), pos, kw)
+        if clip is None:
+            raise Error("clip argument is required")
+        return _node(PackRGBFilter(clip._info()), clip)
 
     def _bind(self, names, pos, kw):
         """VapourSynth binding rule: `clip.vszip.F(a, b)` puts the bound clip first and shifts the positional arguments."""
@@ -722,7 +744,7 @@ def _node(flt: _Filter, main: VideoNode, second: VideoNode | None = None, third:
           prefix="") -> VideoNode:
     """A vszip node on `main`, `second` and `third` (the chain's numbering)."""
     base = (main, second, third)[flt.ARGS[0]]
-    o, b = flt.out_info, base.format  # the library's output format (vszip_filter_output_info): the base clip's but for ColorMap
+    o, b = flt.out_info, base.format  # the library's output format (vszip_filter_output_info): the base clip's but for ColorMap / PackRGB
     same = (o.color_family, o.sample_type, o.bits_per_sample, o.sub_sampling_w, o.sub_sampling_h, o.num_planes) == (
         b.color_family, b.sample_type, b.bits_per_sample, b.subsampling_w, b.subsampling_h, b.num_planes)
     fmt = b if same else _format_of(o)
@@ -813,7 +835,7 @@ def _fused_get(chain_and_source, n: int) -> "VideoFrame":
     chain, source = chain_and_source
     core._ensure_init()
     src = source.get_frame(n)
-    last = chain.nodes[-1]  # the result has the last node's format: the source's, or RGB24 after a ColorMap
+    last = chain.nodes[-1]  # the result has the last node's format: the source's, RGB24 after a ColorMap, GRAY32 after a PackRGB
     fmt = last.format
     out_planes = [np.empty(fmt.plane_shape(src.width, src.height, i), fmt.dtype) if chain.written[i] else src.planes[i]
                   for i in range(fmt.num_planes)]

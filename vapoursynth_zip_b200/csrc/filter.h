@@ -1,4 +1,4 @@
-// filter.h — the immutable per-instance data of the nine filters (the CUDA-side twin of the
+// filter.h — the immutable per-instance data of the ten filters (the CUDA-side twin of the
 // reference's `Data` structs) and the kernel launchers each filter uses.
 #pragma once
 
@@ -7,7 +7,7 @@
 namespace vsz {
 
 enum FilterKind { F_BOXBLUR = 1, F_BILATERAL = 2, F_PLANEMINMAX = 3, F_PLANEAVERAGE = 4, F_LIMITER = 5, F_LIMITFILTER = 6, F_ADAPTIVEBINARIZE = 7,
-                  F_CLAHE = 8, F_COLORMAP = 9 };
+                  F_CLAHE = 8, F_COLORMAP = 9, F_PACKRGB = 10 };
 
 struct BilateralPlane {
     double sigmaS = 0, sigmaR = 0;
@@ -24,7 +24,8 @@ struct vszip_filter {
     vszip_video_info vi;
     vsz::SampleKind sample;
     vsz::FrameLayout layout;
-    // the format of the frames the filter returns, and their layout: vi / layout for every filter except ColorMap (RGB24)
+    // the format of the frames the filter returns, and their layout: vi / layout for every filter except ColorMap (RGB24) and
+    // PackRGB (GRAY32)
     vszip_video_info out_vi;
     vsz::FrameLayout out_layout;
     bool process[3];    // the planes the filter reads (and, unless it changes the format, writes)
@@ -124,6 +125,10 @@ int run_clahe(const FrameLayout& l, const bool mask[3], const char* src, size_t 
 // pointwise_kernels.cu: ColorMap, plane 0 of an 8..16-bit integer clip (layout in) into the three planes of RGB24 (layout out)
 int run_colormap(const FrameLayout& in, const char* src, size_t src_fs, const FrameLayout& out, char* dst, size_t dst_fs, int count,
                  const uint32_t lut[256], cudaStream_t st);
+
+// pointwise_kernels.cu: PackRGB, the three planes of an RGB24 / RGB30 clip (layout in) into the one plane of GRAY32 (layout out)
+int run_packrgb(const FrameLayout& in, const char* src, size_t src_fs, const FrameLayout& out, char* dst, size_t dst_fs, int count,
+                cudaStream_t st);
 
 // planestats_kernels.cu
 struct StatsRaw {  // one per (frame, processed plane), written by the kernels

@@ -185,7 +185,8 @@ bool same_format(const vszip_video_info& a, const vszip_video_info& b) {
            a.num_planes == b.num_planes;
 }
 
-// The format every create function gives its instance: it reads and returns frames of vi (ColorMap then sets its output format).
+// The format every create function gives its instance: it reads and returns frames of vi (ColorMap and PackRGB then set their
+// output format).
 void set_format(vszip_filter* f, const vszip_video_info& vi, SampleKind kind) {
     f->vi = f->out_vi = vi;
     f->sample = kind;
@@ -223,8 +224,9 @@ constexpr KindInfo kKinds[] = {
     {"AdaptiveBinarize", true, {"clip", nullptr}, {false, false}},
     {"CLAHE", true, {nullptr, nullptr}, {false, false}},
     {"ColorMap", true, {nullptr, nullptr}, {false, false}},
+    {"PackRGB", true, {nullptr, nullptr}, {false, false}},
 };
-static_assert(sizeof kKinds / sizeof kKinds[0] == F_COLORMAP, "one row per FilterKind");
+static_assert(sizeof kKinds / sizeof kKinds[0] == F_PACKRGB, "one row per FilterKind");
 
 const KindInfo& kind_info(int kind) { return kKinds[kind - 1]; }
 bool is_pixel(const vszip_filter* f) { return kind_info(f->kind).pixel; }
@@ -773,7 +775,7 @@ int vszip_planeaverage_device(const vszip_filter* f, const vszip_dev_clip* a, co
 static int run_pixels(const vszip_filter* f, int dev_index, const char* const in[3], size_t in_fs, char* out, size_t out_fs, int count,
                       cudaStream_t st) {
     const FrameLayout& l = f->layout;
-    const size_t fs = in_fs;  // every filter but ColorMap: out_fs == in_fs
+    const size_t fs = in_fs;  // every filter but ColorMap and PackRGB: out_fs == in_fs
     switch (f->kind) {
         case F_BOXBLUR:
             return run_boxblur(l, f->process, in[0], fs, out, fs, count, (int)f->hradius, f->hpasses, (int)f->vradius, f->vpasses, st);
@@ -788,6 +790,8 @@ static int run_pixels(const vszip_filter* f, int dev_index, const char* const in
             return run_clahe(l, f->process, in[0], fs, out, fs, count, f->clahe_hs, f->clahe_limit, f->clahe_tiles[0], f->clahe_tiles[1], st);
         case F_COLORMAP:
             return run_colormap(l, in[0], in_fs, f->out_layout, out, out_fs, count, f->cmap_lut, st);
+        case F_PACKRGB:
+            return run_packrgb(l, in[0], in_fs, f->out_layout, out, out_fs, count, st);
         default:  // AdaptiveBinarize: clip = the second input, clip2 = the main one
             return run_adaptivebinarize(l, in[1], fs, in[0], fs, out, fs, count, f->ab_c, st);
     }
@@ -1145,12 +1149,46 @@ int vszip_colormap_device(const vszip_filter* f, const vszip_dev_clip* src, vszi
     return pixel_device(f, F_COLORMAP, {src, nullptr, nullptr}, dst, first, count, stream);
 }
 
+// =========================================================================== PackRGB
+// RGB24 / RGB30 packed into one 32-bit plane in Qt's QImage layouts (DESIGN.md §4.9): RGB in, GRAY32 out.  The argument string and
+// the message are this library's.
+vszip_filter* vszip_packrgb_create(const vszip_video_info* vi) {
+    static const char* name = "PackRGB";
+    if (!basic_vi_ok(vi, name)) return nullptr;
+    const bool rgb = vi->color_family == VSZIP_CF_RGB && vi->sample_type == VSZIP_ST_INTEGER && vi->num_planes == 3 &&
+                     vi->sub_sampling_w == 0 && vi->sub_sampling_h == 0;
+    const bool rgb24 = rgb && vi->bits_per_sample == 8 && vi->bytes_per_sample == 1;
+    const bool rgb30 = rgb && vi->bits_per_sample == 10 && vi->bytes_per_sample == 2;
+    if (!rgb24 && !rgb30) { set_error("PackRGB: only RGB24 and RGB30 clips are supported."); return nullptr; }
+    vszip_filter* f = new vszip_filter();
+    f->kind = F_PACKRGB;
+    set_format(f, *vi, rgb24 ? K_U8 : K_U16);
+    vszip_video_info o = *vi;  // GRAY32 of the same size and length
+    o.color_family = VSZIP_CF_GRAY;
+    o.sample_type = VSZIP_ST_INTEGER;
+    o.bits_per_sample = 32;
+    o.bytes_per_sample = 4;
+    o.num_planes = 1;
+    f->out_vi = o;
+    f->out_layout = make_layout(o, K_U32);
+    for (int i = 0; i < 3; ++i) f->process[i] = true;  // the planes it reads
+    return f;
+}
+
+int vszip_packrgb_get_frame(const vszip_filter* f, int32_t n, const vszip_frame* src, vszip_frame* dst) {
+    return pixel_get_frame(f, F_PACKRGB, n, {src, nullptr, nullptr}, dst);
+}
+
+int vszip_packrgb_device(const vszip_filter* f, const vszip_dev_clip* src, vszip_dev_clip* dst, int32_t first, int32_t count, void* stream) {
+    return pixel_device(f, F_PACKRGB, {src, nullptr, nullptr}, dst, first, count, stream);
+}
+
 // =========================================================================== fused chains
 // Values of a chain: 0 = the source frame, k >= 1 = the pixel output of element k - 1.  Every element reads its main input (the
 // value it filters) and up to two extra inputs; the buffer plan gives every pixel output a frame buffer for as long as a later
 // element reads it (DESIGN.md §5.1).  Buffers 0..2 are the slot's dev[0..2] (0 = the source, never written; 2 = the value the
 // chain returns, the D2H source), buffers 3.. are the slot's device-only extras.  Every value has a format: value 0 filter 0's,
-// value k the output format of element k - 1, which differs from its input's for ColorMap.
+// value k the output format of element k - 1, which differs from its input's for ColorMap and PackRGB.
 struct vszip_chain {
     std::vector<const vszip_filter*> fl;
     vsz::FrameLayout in_layout, out_layout;  // the source's and the returned value's

@@ -506,4 +506,125 @@ int run_colormap(const FrameLayout& in, const char* src, size_t src_fs, const Fr
     return 0;
 }
 
+// =========================================================================== PackRGB
+// DESIGN.md §4.9: the three planes of RGB24 / RGB30 into one GRAY32 plane in Qt's QImage layouts, per pixel
+// RGB24: 0xFF000000 | R << 16 | G << 8 | B (Format_RGB32), RGB30: 0xC0000000 | min(R, 1023) << 20 | min(G, 1023) << 10 |
+// min(B, 1023) (Format_RGB30, top bits set).  3 + 4 bytes per pixel at 8 bits, 6 + 4 at 10: HBM-bound by construction.  The
+// streaming shape of colormap_kernel: work items of 16 pixels of one row, spread over all threads of a CTA, 12 16-byte loads in
+// flight per thread (four 8-bit items or two 10-bit ones) and four 16-byte stores per item.
+static constexpr int PKT = 256, PK_ITEMS = 8;  // PK_ITEMS: work items per thread a CTA's rows are sized for
+
+struct PackRGBJob {
+    const char* src;
+    char* dst;
+    size_t src_fs, dst_fs;
+    size_t src_off[3];  // R, G, B planes
+    size_t dst_off;
+    int src_pitch, dst_pitch;
+    int w, h, rows;     // rows: per CTA
+};
+
+// one word of each plane (four 8-bit pixels) -> four output words, bytes B, G, R, 0xFF (8 PRMT)
+__device__ __forceinline__ void pack_rgb32x4(uint32_t r, uint32_t g, uint32_t b, uint32_t o[4]) {
+    const uint32_t bg01 = __byte_perm(b, g, 0x5140), bg23 = __byte_perm(b, g, 0x7362);                    // B0 G0 B1 G1 / B2 G2 B3 G3
+    const uint32_t r01 = __byte_perm(r, 0xffffffffu, 0x4140), r23 = __byte_perm(r, 0xffffffffu, 0x4342);  // R0 FF R1 FF / R2 FF R3 FF
+    o[0] = __byte_perm(bg01, r01, 0x5410);
+    o[1] = __byte_perm(bg01, r01, 0x7632);
+    o[2] = __byte_perm(bg23, r23, 0x5410);
+    o[3] = __byte_perm(bg23, r23, 0x7632);
+}
+
+// one word of each plane (two 10-bit pixels in u16 containers) -> two output words.  The clamp keeps a sample above 1023 out of the
+// neighbouring field; 0b11 above each clamped R lands in the two top bits after its shift.
+__device__ __forceinline__ void pack_rgb30x2(uint32_t r, uint32_t g, uint32_t b, uint32_t o[2]) {
+    r = __vminu2(r, 0x03ff03ffu) | 0x0c000c00u;
+    g = __vminu2(g, 0x03ff03ffu);
+    b = __vminu2(b, 0x03ff03ffu);
+    o[0] = (r << 20) | ((g & 0xffffu) << 10) | (b & 0xffffu);
+    o[1] = ((r >> 16) << 20) | ((g >> 16) << 10) | (b >> 16);
+}
+
+template <typename T>
+__device__ __forceinline__ uint32_t pack_rgb_pixel(uint32_t r, uint32_t g, uint32_t b) {
+    if (sizeof(T) == 1) return 0xff000000u | r << 16 | g << 8 | b;
+    return 0xc0000000u | min(r, 1023u) << 20 | min(g, 1023u) << 10 | min(b, 1023u);
+}
+
+template <typename T>
+__global__ void __launch_bounds__(PKT) packrgb_kernel(const __grid_constant__ PackRGBJob job) {
+    constexpr int LOADS = (int)sizeof(T);      // 16-byte loads per plane and item
+    constexpr int UNROLL = 4 / (int)sizeof(T);  // items in flight per thread
+    const int y0 = (int)blockIdx.x * job.rows, nrows = min(job.rows, job.h - y0);
+    const char* src = job.src + (size_t)blockIdx.y * job.src_fs + (size_t)y0 * job.src_pitch;
+    char* dst = job.dst + (size_t)blockIdx.y * job.dst_fs + job.dst_off + (size_t)y0 * job.dst_pitch;
+    const int nvec = job.w / 16, items = nrows * nvec;
+    for (int it0 = threadIdx.x; it0 < items; it0 += PKT * UNROLL) {
+        uint4 x[UNROLL][3][LOADS];
+#pragma unroll
+        for (int u = 0; u < UNROLL; ++u) {
+            const int it = min(it0 + u * PKT, items - 1);
+            const int y = it / nvec, v = it - y * nvec;
+#pragma unroll
+            for (int c = 0; c < 3; ++c) {
+                const uint4* p = reinterpret_cast<const uint4*>(src + job.src_off[c] + (size_t)y * job.src_pitch) + v * LOADS;
+#pragma unroll
+                for (int l = 0; l < LOADS; ++l) x[u][c][l] = __ldg(p + l);
+            }
+        }
+#pragma unroll
+        for (int u = 0; u < UNROLL; ++u) {
+            const int it = it0 + u * PKT;
+            if (it < items) {
+                const uint32_t* r = reinterpret_cast<const uint32_t*>(x[u][0]);
+                const uint32_t* g = reinterpret_cast<const uint32_t*>(x[u][1]);
+                const uint32_t* b = reinterpret_cast<const uint32_t*>(x[u][2]);
+                uint32_t o[16];
+#pragma unroll
+                for (int k = 0; k < 4 * LOADS; ++k) {  // input word k of each plane
+                    if (sizeof(T) == 1) pack_rgb32x4(r[k], g[k], b[k], o + 4 * k);
+                    else pack_rgb30x2(r[k], g[k], b[k], o + 2 * k);
+                }
+                const int y = it / nvec, v = it - y * nvec;
+                uint4* q = reinterpret_cast<uint4*>(dst + (size_t)y * job.dst_pitch) + 4 * v;
+#pragma unroll
+                for (int s = 0; s < 4; ++s) q[s] = make_uint4(o[4 * s], o[4 * s + 1], o[4 * s + 2], o[4 * s + 3]);
+            }
+        }
+    }
+    // row tails (< 16 pixels): one pixel per thread
+    const int tail = job.w - nvec * 16;
+    for (int it = threadIdx.x; it < nrows * tail; it += PKT) {
+        const int y = it / tail, x0 = nvec * 16 + (it - y * tail);
+        const size_t off = (size_t)y * job.src_pitch + (size_t)x0 * sizeof(T);
+        const uint32_t r = *reinterpret_cast<const T*>(src + job.src_off[0] + off);
+        const uint32_t g = *reinterpret_cast<const T*>(src + job.src_off[1] + off);
+        const uint32_t b = *reinterpret_cast<const T*>(src + job.src_off[2] + off);
+        reinterpret_cast<uint32_t*>(dst + (size_t)y * job.dst_pitch)[x0] = pack_rgb_pixel<T>(r, g, b);
+    }
+}
+
+int run_packrgb(const FrameLayout& in, const char* src, size_t src_fs, const FrameLayout& out, char* dst, size_t dst_fs, int count,
+                cudaStream_t st) {
+    if (count <= 0) return 0;
+    if ((in.kind != K_U8 && in.kind != K_U16) || in.nplanes != 3 || out.kind != K_U32 || out.nplanes != 1) return -1;
+    PackRGBJob job{};
+    job.src = src; job.dst = dst; job.src_fs = src_fs; job.dst_fs = dst_fs;
+    for (int p = 0; p < 3; ++p) job.src_off[p] = in.pl[p].offset;
+    job.dst_off = out.pl[0].offset;
+    job.src_pitch = in.pl[0].pitch; job.dst_pitch = out.pl[0].pitch;  // the three RGB planes share their geometry
+    job.w = in.pl[0].w; job.h = in.pl[0].h;
+    job.rows = std::max(1, std::min(job.h, PKT * PK_ITEMS / std::max(1, job.w / 16)));
+    const int ctas = (job.h + job.rows - 1) / job.rows;
+    for (int f0 = 0; f0 < count; f0 += 65535) {
+        const int nf = std::min(65535, count - f0);
+        PackRGBJob j = job;
+        j.src += (size_t)f0 * src_fs; j.dst += (size_t)f0 * dst_fs;
+        if (in.kind == K_U8) packrgb_kernel<uint8_t><<<dim3(ctas, nf), PKT, 0, st>>>(j);
+        else packrgb_kernel<uint16_t><<<dim3(ctas, nf), PKT, 0, st>>>(j);
+        count_launch();
+    }
+    VSZ_CUDA(cudaGetLastError());
+    return 0;
+}
+
 }  // namespace vsz

@@ -355,7 +355,7 @@ __global__ void noise_kernel(char* base, size_t frame_stride, size_t plane_off, 
                          ((uint64_t)plane << 36) ^ ((uint64_t)y << 18) ^ (uint64_t)x;
     const uint32_t u = mix64to32(key);
     T* row = reinterpret_cast<T*>(base + (size_t)f * frame_stride + plane_off + (size_t)y * pitch);
-    if constexpr (std::is_same<T, uint8_t>::value || std::is_same<T, uint16_t>::value) {
+    if constexpr (std::is_same<T, uint8_t>::value || std::is_same<T, uint16_t>::value || std::is_same<T, uint32_t>::value) {
         row[x] = (T)(u >> (32 - bits));
     } else {
         float v = (float)(u >> 8) * (1.0f / 16777216.0f);  // [0,1)
@@ -512,7 +512,7 @@ vszip_dev_clip* vszip_dev_clip_alloc(const vszip_video_info* vi, int32_t num_fra
     DeviceCtx* d = device_ctx(device);
     if (!d) { set_error("vszip_dev_clip_alloc: library not initialised or bad device index %d", device); return nullptr; }
     SampleKind kind;
-    if (!select_kind(*vi, "vszip_dev_clip_alloc", false, &kind)) return nullptr;
+    if (!select_kind(*vi, "vszip_dev_clip_alloc", true, &kind)) return nullptr;  // 32-bit integer: Limiter, PackRGB's output
     if (num_frames <= 0 || vi->width <= 0 || vi->height <= 0 || vi->num_planes < 1 || vi->num_planes > 3) {
         set_error("vszip_dev_clip_alloc: bad geometry");
         return nullptr;
@@ -593,6 +593,7 @@ int vszip_dev_clip_fill_noise(vszip_dev_clip* c, uint64_t seed, int32_t first_fr
                 case K_U16: noise_kernel<uint16_t><<<gz, 256, 0, d->batch_stream>>>(base, l.frame_stride, g.offset, g.pitch, g.w, g.h, p, seed, first_frame_no + f0 * frame_no_stride, frame_no_stride, l.kind, l.bits, centered); break;
                 case K_F16: noise_kernel<__half><<<gz, 256, 0, d->batch_stream>>>(base, l.frame_stride, g.offset, g.pitch, g.w, g.h, p, seed, first_frame_no + f0 * frame_no_stride, frame_no_stride, l.kind, l.bits, centered); break;
                 case K_F32: noise_kernel<float><<<gz, 256, 0, d->batch_stream>>>(base, l.frame_stride, g.offset, g.pitch, g.w, g.h, p, seed, first_frame_no + f0 * frame_no_stride, frame_no_stride, l.kind, l.bits, centered); break;
+                case K_U32: noise_kernel<uint32_t><<<gz, 256, 0, d->batch_stream>>>(base, l.frame_stride, g.offset, g.pitch, g.w, g.h, p, seed, first_frame_no + f0 * frame_no_stride, frame_no_stride, l.kind, l.bits, centered); break;
             }
             count_launch();
         }
