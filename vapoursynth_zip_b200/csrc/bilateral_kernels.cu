@@ -364,7 +364,7 @@ static int run_bilateral_t(const FrameLayout& l, const bool mask[3], const char*
         BatchJob j = make_batch(l, one, src, sfs, ref, rfs, dst, dfs, [&](int, int) { return strips_x * tiles_y; });
         const size_t tile = (size_t)(TILE + 2 * r) * (TILE + 2 * r);
         const size_t smem = (tile * (ref ? 2 : 1) + (size_t)(r + 1) * (r + 1) + (size_t)pp.smem_lut) * sizeof(float);
-        if (smem > 227 * 1024) { set_error("Bilateral: spatial radius %d does not fit the shared-memory tile", r); return -2; }
+        if (smem > (size_t)kMaxSmemPerCta) { set_error("Bilateral: spatial radius %d does not fit the shared-memory tile", r); return -2; }
         for (int f0 = 0; f0 < count; f0 += 65535) {
             const int nf = std::min(65535, count - f0);
             BatchJob jj = j;

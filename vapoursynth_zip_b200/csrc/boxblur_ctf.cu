@@ -23,13 +23,14 @@
 //   tap indices.  Long lines are cut into segments (each pays 2r warm-up samples) so that single-frame calls fill the GPU too.
 //
 // Planes with fewer than 2r+1 rows or columns keep the tiled kernel of boxblur_kernels.cu.
-#include <cuda.h>  // CUtensorMap types only: the encoder comes from cudaGetDriverEntryPoint, libcuda is not linked
 #include <cuda_fp16.h>
 
 #include <algorithm>
 #include <type_traits>
 #include <utility>
 
+#include "boxblur_host.h"
+#include "boxblur_tma.h"
 #include "common.h"
 #include "filter.h"
 
@@ -521,22 +522,6 @@ __global__ void __launch_bounds__(kHThreads) ctf_h_kernel(const CtfJob job, cons
 }
 
 // --------------------------------------------------------------------------- host side
-using TensorMapEncodeFn = CUresult (*)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                       const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                       CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-TensorMapEncodeFn tensor_map_encoder() {
-    static const TensorMapEncodeFn fn = [] {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess) {
-            cudaGetLastError();
-            p = nullptr;
-        }
-        return reinterpret_cast<TensorMapEncodeFn>(p);
-    }();
-    return fn;
-}
-
 // pieces along the blurred axis: as many as it takes to give the GPU ~3 waves of CTAs, each a multiple of `quantum` long
 // and at least 8 blocks of 2r+1 samples (a piece pays 2r warm-up samples)
 void cut_line(int interior, int quantum, int ctas_without_cut, int sms, int& segs, int& seg_len) {
@@ -552,11 +537,9 @@ int launch_ctf(const FrameLayout& l, const bool mask[3], const char* src, size_t
                cudaStream_t st) {
     constexpr int K = 2 * R + 1, NC = Smp<T>::NC;
     using G = HTile<T, R>;
-    const TensorMapEncodeFn encode = tensor_map_encoder();
-    if (!encode) return 1;
-    int dev = 0, sms = 148;
-    VSZ_CUDA(cudaGetDevice(&dev));
-    VSZ_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    if (!tensor_map_encoder()) return 1;
+    const int sms = current_sm_count();
+    if (sms < 0) return sms;
     CtfJob jv{}, jh{};
     jv.src = src; jv.src_fs = sfs; jv.dst = tmp; jv.dst_fs = tfs;
     jh.src = tmp; jh.src_fs = tfs; jh.dst = dst; jh.dst_fs = dfs;
@@ -594,13 +577,9 @@ int launch_ctf(const FrameLayout& l, const bool mask[3], const char* src, size_t
         CtfMaps maps;
         for (int q = 0; q < k; ++q) {
             const CtfPlane& pl = b.pl[q];
-            const cuuint64_t dims[3] = {(cuuint64_t)pl.w, (cuuint64_t)pl.h, (cuuint64_t)nf};
-            const cuuint64_t strides[2] = {(cuuint64_t)pl.src_pitch, (cuuint64_t)b.src_fs};
-            const cuuint32_t box[3] = {(cuuint32_t)G::TW, (cuuint32_t)kHRows, 1}, estr[3] = {1, 1, 1};
-            const CUresult rc = encode(&maps.in[q], sizeof(T) == 4 ? CU_TENSOR_MAP_DATA_TYPE_UINT32 : CU_TENSOR_MAP_DATA_TYPE_UINT16, 3,
-                                       const_cast<char*>(b.src) + pl.src_off, dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                                       CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-            if (rc != CUDA_SUCCESS) { set_error("BoxBlur: cuTensorMapEncodeTiled failed (%d)", (int)rc); return -1; }
+            const int rc = encode_plane_map(&maps.in[q], sizeof(T) == 4 ? CU_TENSOR_MAP_DATA_TYPE_UINT32 : CU_TENSOR_MAP_DATA_TYPE_UINT16,
+                                            b.src + pl.src_off, pl.w, pl.h, pl.src_pitch, b.src_fs, nf, G::TW, kHRows);
+            if (rc) return rc;
         }
         ctf_v_kernel<T, R><<<dim3(nf, a.ctas_per_frame), kThreads, 0, st>>>(a);
         ctf_h_kernel<T, R><<<dim3(nf, b.ctas_per_frame), kHThreads, G::SMEM, st>>>(b, maps);
@@ -610,29 +589,16 @@ int launch_ctf(const FrameLayout& l, const bool mask[3], const char* src, size_t
     return 0;
 }
 
-template <typename T>
-int dispatch_ctf(const FrameLayout& l, const bool mask[3], const char* src, size_t sfs, char* tmp, size_t tfs, char* dst, size_t dfs, int count,
-                 int r, cudaStream_t st) {
-    switch (r) {
-#define X(R) case R: return launch_ctf<T, R>(l, mask, src, sfs, tmp, tfs, dst, dfs, count, st);
-#ifdef VSZ_SEG_DEV13  // A/B builds (scripts/build_variant.sh): a few radii, seconds to compile
-        X(4) X(13) X(22)
-#else
-        X(1) X(2) X(3) X(4) X(5) X(6) X(7) X(8) X(9) X(10) X(11) X(12) X(13) X(14) X(15) X(16) X(17) X(18) X(19) X(20) X(21) X(22)
-#endif
-#undef X
-    }
-    return 1;
-}
-
 }  // namespace
 
-// 0 = done, 1 = not applicable (a plane has fewer than 2r+1 rows or columns: the tiled kernel handles it), < 0 = error
 int run_ctf_stream(const FrameLayout& l, const bool mask[3], const char* src, size_t sfs, char* tmp, size_t tfs, char* dst, size_t dfs,
                    int count, int r, cudaStream_t st) {
-    if (l.kind == K_F32) return dispatch_ctf<float>(l, mask, src, sfs, tmp, tfs, dst, dfs, count, r, st);
-    if (l.kind == K_F16) return dispatch_ctf<__half>(l, mask, src, sfs, tmp, tfs, dst, dfs, count, r, st);
-    return 1;
+    return with_radius(r, [&](auto radius) {
+        constexpr int R = decltype(radius)::value;
+        if (l.kind == K_F32) return launch_ctf<float, R>(l, mask, src, sfs, tmp, tfs, dst, dfs, count, st);
+        if (l.kind == K_F16) return launch_ctf<__half, R>(l, mask, src, sfs, tmp, tfs, dst, dfs, count, st);
+        return 1;
+    });
 }
 
 }  // namespace vsz

@@ -22,8 +22,7 @@
 //   ctf_*_kernel  : comptime float path (direct sums, R101q).
 #include <cuda_fp16.h>
 
-#include <cstdlib>
-
+#include "boxblur_host.h"
 #include "common.h"
 #include "filter.h"
 
@@ -952,14 +951,11 @@ static AxisParams axis_params(int r) {
     AxisParams a{};
     a.r = r;
     a.ring = 2 * r + 1;
-    const uint64_t inv = ((1ull << 32) + (uint64_t)r) / (uint64_t)(2 * r + 1);
-    a.inv = (uint32_t)inv;
-    a.inv2 = (uint32_t)(inv >> 16);
+    axis_consts(r, a.inv, a.inv2);
     a.div = 1.0f / (float)(2 * r + 1);
     return a;
 }
 
-static constexpr int kMaxSmem = 227 * 1024;
 #ifndef VSZ_NT_V
 #define VSZ_NT_V 64
 #endif
@@ -972,74 +968,48 @@ static constexpr int NT_H = VSZ_NT_H;
 #ifndef VSZ_V_WORDS
 #define VSZ_V_WORDS 2
 #endif
+static constexpr int V_W = VSZ_V_WORDS, V_NT = NT_V / V_W;  // same shared memory per CTA for W = 1 and W = 2
+
+// dynamic shared memory of blur_v_kernel / blur_h_kernel with P fused passes at radius r: one 2r+1-slot delay ring per pass and
+// thread, then the input stage (V) or the input and output tiles (H)
+static size_t v_smem(int r, int P) { return ((size_t)(2 * r + 1) * P * V_NT * V_W + VStage<V_NT, V_W>::WORDS) * 4; }
+template <typename T>
+static size_t h_smem(int r, int P) { return ((size_t)(2 * r + 1) * P * NT_H + HTile<T, NT_H>::IN_WORDS + HTile<T, NT_H>::OUT_WORDS) * 4; }
+
 template <typename T, int P, int MODE>
 static int launch_v(const FrameLayout& l, const bool mask[3], const char* src, size_t src_fs, char* dst, size_t dst_fs,
                     int count, int r, cudaStream_t st) {
     constexpr int NL = Px<T>::NL;
-    constexpr int W = VSZ_V_WORDS, NT = NT_V / W;  // same shared memory per CTA for W = 1 and W = 2
-    const AxisParams ap = axis_params(r);
-    const size_t smem = ((size_t)ap.ring * P * NT * W + VStage<NT, W>::WORDS) * 4;
-    if (smem > (size_t)kMaxSmem) { set_error("BoxBlur: vradius %d with %d fused passes exceeds the shared-memory delay ring", r, P); return -2; }
-    auto kern = blur_v_kernel<T, P, MODE, NT, W>;
-    VSZ_CUDA(allow_max_dynamic_smem(kern));
-    BatchJob job = make_batch(l, mask, src, src_fs, nullptr, 0, dst, dst_fs,
-                              [](int w, int) { return ((w + NL * W - 1) / (NL * W) + NT - 1) / NT; });
-    if (job.ctas_per_frame == 0) return 0;
-    for (int f0 = 0; f0 < count; f0 += 65535) {
-        const int nf = std::min(65535, count - f0);
-        BatchJob j = job;
-        j.src += (size_t)f0 * src_fs; j.dst += (size_t)f0 * dst_fs;
-        // grid.x = frame, grid.y = CTA within the frame: CTAs are scheduled x-fastest, so every frame's (long) luma CTAs
-        // start before any (short) chroma CTA and the tail of the launch is made of short CTAs
-        kern<<<dim3(nf, job.ctas_per_frame), NT, smem, st>>>(j, ap);
-        count_launch();
-    }
-    VSZ_CUDA(cudaGetLastError());
-    return 0;
+    const BatchJob job = make_batch(l, mask, src, src_fs, nullptr, 0, dst, dst_fs,
+                                    [](int w, int) { return ((w + NL * V_W - 1) / (NL * V_W) + V_NT - 1) / V_NT; });
+    return launch_frames(blur_v_kernel<T, P, MODE, V_NT, V_W>, job, count, V_NT, v_smem(r, P), st, axis_params(r));
 }
 
 template <typename T, int P>
 static int launch_h(const FrameLayout& l, const bool mask[3], const char* src, size_t src_fs, char* dst, size_t dst_fs,
                     int count, int r, cudaStream_t st) {
     constexpr int NL = Px<T>::NL;
-    using TL = HTile<T, NT_H>;
-    const AxisParams ap = axis_params(r);
-    const size_t smem = ((size_t)ap.ring * P * NT_H + TL::IN_WORDS + TL::OUT_WORDS) * 4;
-    if (smem > (size_t)kMaxSmem) { set_error("BoxBlur: hradius %d with %d fused passes exceeds the shared-memory delay ring", r, P); return -2; }
-    auto kern = blur_h_kernel<T, P, NT_H>;
-    VSZ_CUDA(allow_max_dynamic_smem(kern));
-    BatchJob job = make_batch(l, mask, src, src_fs, nullptr, 0, dst, dst_fs,
-                              [](int, int h) { return (h + NT_H * NL - 1) / (NT_H * NL); });
-    if (job.ctas_per_frame == 0) return 0;
-    for (int f0 = 0; f0 < count; f0 += 65535) {
-        const int nf = std::min(65535, count - f0);
-        BatchJob j = job;
-        j.src += (size_t)f0 * src_fs; j.dst += (size_t)f0 * dst_fs;
-        kern<<<dim3(nf, job.ctas_per_frame), NT_H, smem, st>>>(j, ap);  // see launch_v for the grid order
-        count_launch();
-    }
-    VSZ_CUDA(cudaGetLastError());
-    return 0;
+    const BatchJob job = make_batch(l, mask, src, src_fs, nullptr, 0, dst, dst_fs,
+                                    [](int, int h) { return (h + NT_H * NL - 1) / (NT_H * NL); });
+    return launch_frames(blur_h_kernel<T, P, NT_H>, job, count, NT_H, h_smem<T>(r, P), st, axis_params(r));
 }
 
 // largest number of passes one launch can fuse for this radius (shared-memory bound), at most 5
-static int max_fused(int r, bool horizontal) {
-    const size_t per_pass = (size_t)(2 * r + 1) * (horizontal ? NT_H : NT_V) * 4;
-    const size_t fixed = horizontal ? (size_t)(HTile<uint16_t, NT_H>::IN_WORDS + HTile<uint16_t, NT_H>::OUT_WORDS) * 4 : (size_t)VStage<NT_V, 1>::WORDS * 4;
-    int p = (int)((kMaxSmem - fixed) / per_pass);
-    return p > 5 ? 5 : p;
+template <typename T, bool H>
+static int max_fused(int r) {
+    int p = 5;
+    while (p > 0 && (H ? h_smem<T>(r, p) : v_smem(r, p)) > (size_t)kMaxSmemPerCta) --p;
+    return p;
 }
 
 template <typename T, bool H>
 static int launch_axis_p(int P, const FrameLayout& l, const bool mask[3], const char* src, size_t sfs, char* dst, size_t dfs,
                          int count, int r, cudaStream_t st) {
-    switch (P) {
-        case 1: return H ? launch_h<T, 1>(l, mask, src, sfs, dst, dfs, count, r, st) : launch_v<T, 1, MODE_RT>(l, mask, src, sfs, dst, dfs, count, r, st);
-        case 2: return H ? launch_h<T, 2>(l, mask, src, sfs, dst, dfs, count, r, st) : launch_v<T, 2, MODE_RT>(l, mask, src, sfs, dst, dfs, count, r, st);
-        case 3: return H ? launch_h<T, 3>(l, mask, src, sfs, dst, dfs, count, r, st) : launch_v<T, 3, MODE_RT>(l, mask, src, sfs, dst, dfs, count, r, st);
-        case 4: return H ? launch_h<T, 4>(l, mask, src, sfs, dst, dfs, count, r, st) : launch_v<T, 4, MODE_RT>(l, mask, src, sfs, dst, dfs, count, r, st);
-        case 5: return H ? launch_h<T, 5>(l, mask, src, sfs, dst, dfs, count, r, st) : launch_v<T, 5, MODE_RT>(l, mask, src, sfs, dst, dfs, count, r, st);
-    }
+    const int rc = with_constant(std::integer_sequence<int, 1, 2, 3, 4, 5>{}, P, [&](auto passes) {
+        if constexpr (H) return launch_h<T, decltype(passes)::value>(l, mask, src, sfs, dst, dfs, count, r, st);
+        else return launch_v<T, decltype(passes)::value, MODE_RT>(l, mask, src, sfs, dst, dfs, count, r, st);
+    });
+    if (rc != 1) return rc;  // launch_h / launch_v return 0 or an error: 1 = P is not in 1..5
     set_error("BoxBlur: internal error, bad fused pass count %d", P);
     return -3;
 }
@@ -1109,7 +1079,7 @@ static int launch_global(const FrameLayout& l, const bool mask[3], const char* s
 template <typename T, bool H>
 static int run_axis(const FrameLayout& l, const bool mask[3], const char* src, size_t sfs, char* dst, size_t dfs, int count,
                     int r, int passes, cudaStream_t st) {
-    const int cap = max_fused(r, H);
+    const int cap = max_fused<T, H>(r);
     if (cap < 1) {
         // out-of-place passes from global memory, ping-ponging two scratch clips so the last pass lands in dst
         AsyncScratch scratch;
@@ -1177,22 +1147,14 @@ static int run_ct_float(const FrameLayout& l, const bool mask[3], const char* sr
     return 0;
 }
 
-// 8- and 16-bit integer clips take the segment kernels (boxblur_seg_{h,v,ct}.cu) where they apply; VSZIP_BOXBLUR_LEGACY=1 keeps
-// every clip on the streaming kernels of this file (A/B timing, and the parity tests run both).
-static bool use_seg_kernels() {
-    static const bool on = [] { const char* e = getenv("VSZIP_BOXBLUR_LEGACY"); return !(e && e[0] == '1'); }();
-    return on;
-}
-
+// 8- and 16-bit integer clips take the segment kernels (boxblur_seg_{h,v,ct}.cu) where they apply
 template <typename T, bool H>
 static int run_axis_any(const FrameLayout& l, const bool mask[3], const char* src, size_t sfs, char* dst, size_t dfs, int count, int r,
                         int passes, cudaStream_t st) {
     if constexpr (std::is_same<T, uint16_t>::value || std::is_same<T, uint8_t>::value) {
-        if (use_seg_kernels()) {
-            const int rc = H ? run_seg_h(l, mask, src, sfs, dst, dfs, count, r, passes, st)
-                             : run_seg_v(l, mask, src, sfs, dst, dfs, count, r, passes, st);
-            if (rc <= 0) return rc;  // done, or a CUDA error; 1 = not applicable
-        }
+        const int rc = H ? run_seg_h(l, mask, src, sfs, dst, dfs, count, r, passes, st)
+                         : run_seg_v(l, mask, src, sfs, dst, dfs, count, r, passes, st);
+        if (rc <= 0) return rc;  // done, or a CUDA error; 1 = nothing launched
     }
     return run_axis<T, H>(l, mask, src, sfs, dst, dfs, count, r, passes, st);
 }
@@ -1212,18 +1174,15 @@ static int run_boxblur_t(const FrameLayout& l, const bool mask[3], const char* s
     if constexpr (Px<T>::flt) {
         AsyncScratch tmp;
         VSZ_CUDA(tmp.alloc(l.frame_stride * (size_t)count, st));
-        if (use_seg_kernels()) {  // streaming accumulators (boxblur_ctf.cu); planes smaller than the window keep the tiled kernel
-            const int rc = run_ctf_stream(l, mask, src, sfs, tmp.p, l.frame_stride, dst, dfs, count, hr, st);
-            if (rc <= 0) return rc;
-        }
+        // streaming accumulators (boxblur_ctf.cu); planes smaller than the window keep the tiled kernel
+        const int rc = run_ctf_stream(l, mask, src, sfs, tmp.p, l.frame_stride, dst, dfs, count, hr, st);
+        if (rc <= 0) return rc;
         return run_ct_float<T>(l, mask, src, sfs, tmp.p, l.frame_stride, dst, dfs, count, hr, st);
     } else {
         // comptime integer path: exact R101q column sums + rounded mean, then the SYM H pass
         if constexpr (std::is_same<T, uint16_t>::value || std::is_same<T, uint8_t>::value) {
-            if (use_seg_kernels()) {  // one read, one write
-                const int rc = run_seg_ct(l, mask, src, sfs, dst, dfs, count, hr, st);
-                if (rc <= 0) return rc;
-            }
+            const int rc = run_seg_ct(l, mask, src, sfs, dst, dfs, count, hr, st);  // one read, one write
+            if (rc <= 0) return rc;
         }
         int rc = launch_v<T, 1, MODE_CTV>(l, mask, src, sfs, dst, dfs, count, hr, st);
         if (rc) return rc;

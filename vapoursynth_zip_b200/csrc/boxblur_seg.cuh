@@ -23,6 +23,7 @@
 
 #include <algorithm>
 
+#include "boxblur_host.h"
 #include "boxblur_seg_core.h"
 #include "common.h"
 #include "filter.h"
@@ -197,14 +198,6 @@ __device__ __forceinline__ uint32_t hseg_window(const uint32_t (&p)[NP], int lan
 }
 
 // --------------------------------------------------------------------------- host side
-constexpr int kMaxSmem = 227 * 1024;
-
-void axis_consts(int r, uint32_t& inv, uint32_t& inv2) {
-    const uint64_t v = ((1ull << 32) + (uint64_t)r) / (uint64_t)(2 * r + 1);
-    inv = (uint32_t)v;
-    inv2 = (uint32_t)(v >> 16);
-}
-
 SegJob base_job(const FrameLayout& l, const bool mask[3], const char* src, size_t sfs, char* dst, size_t dfs, int r, int passes) {
     SegJob j{};
     j.src = src; j.dst = dst; j.src_fs = sfs; j.dst_fs = dfs; j.passes = passes;
@@ -232,42 +225,21 @@ int rowbuf_bytes(int samples, int G) {
     return words * 4;
 }
 
-template <class K>
-int launch_frames(K kern, SegJob job, int count, int threads, size_t smem, cudaStream_t st) {
-    VSZ_CUDA(allow_max_dynamic_smem(kern));
-    for (int f0 = 0; f0 < count; f0 += 65535) {
-        const int nf = std::min(65535, count - f0);
-        SegJob j = job;
-        j.src += (size_t)f0 * job.src_fs; j.dst += (size_t)f0 * job.dst_fs;
-        kern<<<dim3(nf, job.ctas_per_frame), threads, smem, st>>>(j);  // frame index on grid.x (see boxblur_kernels.cu, launch_v)
-        count_launch();
-    }
-    VSZ_CUDA(cudaGetLastError());
-    return 0;
-}
-
 // Planes of different shapes want different CTA shapes (V: warps = segments per column; comptime: columns per thread), so a
-// job is launched once per group of equally shaped planes.
-template <class F>
-int for_each_shape(const SegJob& job, F launch) {
+// job is launched once per group of equally shaped planes.  Returns the number of groups.
+int shape_groups(const SegJob& job, SegJob (&groups)[3]) {
     bool done[3] = {false, false, false};
+    int n = 0;
     for (int k = 0; k < job.nplanes; ++k) {
         if (done[k]) continue;
-        SegJob sub = job;
+        SegJob& sub = groups[n++];
+        sub = job;
         sub.nplanes = 0;
         for (int q = k; q < job.nplanes; ++q)
             if (!done[q] && job.pl[q].w == job.pl[k].w && job.pl[q].h == job.pl[k].h) { sub.pl[sub.nplanes++] = job.pl[q]; done[q] = true; }
-        const int rc = launch(sub);
-        if (rc) return rc;
     }
-    return 0;
+    return n;
 }
-
-#ifdef VSZ_SEG_DEV13  // A/B builds (scripts/build_variant.sh): one radius, seconds to compile
-#define VSZ_SEG_RADII(X) X(13)
-#else
-#define VSZ_SEG_RADII(X) X(1) X(2) X(3) X(4) X(5) X(6) X(7) X(8) X(9) X(10) X(11) X(12) X(13) X(14) X(15) X(16) X(17) X(18) X(19) X(20) X(21) X(22)
-#endif
 
 }  // namespace
 

@@ -164,7 +164,10 @@ int launch_ctfused(const SegJob& whole, int count, cudaStream_t st) {
     using Gm = HGeom<R>;
     for (int k = 0; k < whole.nplanes; ++k)
         if (whole.pl[k].w > CTF_WARPS * 32 * 8 || (whole.pl[k].w + L - 1) / L > 32) return 1;
-    return for_each_shape(whole, [&](SegJob job) {
+    SegJob groups[3];
+    const int ngroups = shape_groups(whole, groups);
+    for (int g = 0; g < ngroups; ++g) {
+        SegJob& job = groups[g];
         const int w = job.pl[0].w, h = job.pl[0].h;
         // planes up to 960 wide (1080p chroma): 4 warps x 8 columns per thread and 4 CTAs per SM instead of 8 warps x 4 columns and 2 -
         // the two CTA-wide barriers per group of rows cost less across 4 warps, and 4 CTAs interleave their V and H phases
@@ -189,24 +192,23 @@ int launch_ctfused(const SegJob& whole, int count, cudaStream_t st) {
             cta += (h + band - 1) / band;
         }
         job.ctas_per_frame = cta;
-        if (narrow) return launch_frames(ctfused_kernel<R, 8, U8, 4>, job, count, 4 * 32, smem, st);
-        return launch_frames(ctfused_kernel<R, 8, U8>, job, count, CTF_WARPS * 32, smem, st);
-    });
+        const int rc = narrow ? launch_frames(ctfused_kernel<R, 8, U8, 4>, job, count, 4 * 32, smem, st)
+                              : launch_frames(ctfused_kernel<R, 8, U8>, job, count, CTF_WARPS * 32, smem, st);
+        if (rc) return rc;
+    }
+    return 0;
 }
 
 }  // namespace
 
-// Entry points.  Return 0 = done, 1 = not applicable (the caller falls back to the streaming kernels), < 0 = error.
 int run_seg_ct(const FrameLayout& l, const bool mask[3], const char* src, size_t sfs, char* dst, size_t dfs, int count, int r, cudaStream_t st) {
     if ((l.kind != K_U16 && l.kind != K_U8) || src == dst) return 1;
     const SegJob job = base_job(l, mask, src, sfs, dst, dfs, r, 1);
     const bool u8 = l.kind == K_U8;
-    switch (r) {
-#define X(R) case R: return u8 ? launch_ctfused<R, true>(job, count, st) : launch_ctfused<R, false>(job, count, st);
-        VSZ_SEG_RADII(X)
-#undef X
-    }
-    return 1;
+    return with_radius(r, [&](auto radius) {
+        constexpr int R = decltype(radius)::value;
+        return u8 ? launch_ctfused<R, true>(job, count, st) : launch_ctfused<R, false>(job, count, st);
+    });
 }
 
 }  // namespace vsz

@@ -137,32 +137,21 @@ int launch_hseg(SegJob job, int count, cudaStream_t st) {
         cta += (groups + s.per_cta - 1) / s.per_cta;
     }
     job.ctas_per_frame = cta;
-    if (cta == 0) return 0;
-    if (smem > (size_t)kMaxSmem) return 1;
+    if (smem > (size_t)kMaxSmemPerCta) return 1;
     return launch_frames(hseg_kernel<R, U8>, job, count, HSEG_WARPS * 32, smem, st);
 }
 
 }  // namespace
 
-// Entry points.  Return 0 = done, 1 = not applicable (the caller falls back to the streaming kernels), < 0 = error.
 int run_seg_h(const FrameLayout& l, const bool mask[3], const char* src, size_t sfs, char* dst, size_t dfs, int count, int r, int passes,
               cudaStream_t st) {
     if ((l.kind != K_U16 && l.kind != K_U8) || passes < 1) return 1;
     const SegJob job = base_job(l, mask, src, sfs, dst, dfs, r, passes);
-    if (l.kind == K_U8) {
-        switch (r) {
-#define X(R) case R: return launch_hseg<R, true>(job, count, st);
-            VSZ_SEG_RADII(X)
-#undef X
-        }
-        return 1;
-    }
-    switch (r) {
-#define X(R) case R: return launch_hseg<R, false>(job, count, st);
-        VSZ_SEG_RADII(X)
-#undef X
-    }
-    return 1;
+    const bool u8 = l.kind == K_U8;
+    return with_radius(r, [&](auto radius) {
+        constexpr int R = decltype(radius)::value;
+        return u8 ? launch_hseg<R, true>(job, count, st) : launch_hseg<R, false>(job, count, st);
+    });
 }
 
 }  // namespace vsz

@@ -1,7 +1,6 @@
 // boxblur_seg_v.cu — vseg_kernel: vertical passes on 64-column strips (see boxblur_seg.cuh for the design of the segment kernels).
-#include <cuda.h>  // CUtensorMap types only: the encoder comes from cudaGetDriverEntryPoint, libcuda is not linked
-
 #include "boxblur_seg.cuh"
+#include "boxblur_tma.h"
 
 namespace vsz {
 
@@ -247,34 +246,30 @@ __global__ void __launch_bounds__(VSegShape<LVT>::MAX_WARPS * 32, 1)
     }
 }
 
-using TensorMapEncodeFn = CUresult (*)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                       const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                       CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-TensorMapEncodeFn tensor_map_encoder() {
-    static const TensorMapEncodeFn fn = [] {
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult q;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess)
-            p = nullptr;
-        return reinterpret_cast<TensorMapEncodeFn>(p);
-    }();
-    return fn;
+template <int R, bool U8> size_t vseg_tile_smem(int S) { return (size_t)S * LVT * (U8 ? 64 : 128) + ((size_t)2 * S * 2 * R * 32 + 128) * 4; }
+
+// Whether the tile kernel can run planes of height h (S = h / 90 warps): 0 = yes, with `resident` CTAs on the GPU at once;
+// 1 = no (no tensor-map encoder in this driver, too much shared memory or no resident CTA); < 0 = error
+template <int R, bool U8>
+int vseg_tile_fit(int h, int& resident) {
+    if (!tensor_map_encoder()) return 1;
+    const int S = h / LVT;
+    const size_t smem = vseg_tile_smem<R, U8>(S);
+    if (smem > (size_t)kMaxSmemPerCta) return 1;
+    auto kern = vseg_tile_kernel<R, U8>;
+    VSZ_CUDA(allow_max_dynamic_smem(kern));
+    const int sms = current_sm_count();
+    if (sms < 0) return sms;
+    int per_sm = 1;
+    VSZ_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, S * 32, smem));
+    if (per_sm < 1) return 1;
+    resident = sms * per_sm;
+    return 0;
 }
 
 template <int R, bool U8>
-int launch_vseg_tile(SegJob job, int count, cudaStream_t st) {
-    const TensorMapEncodeFn encode = tensor_map_encoder();
-    if (!encode) return 1;  // no tensor-map encoder in this driver: the generic kernel below does the job
+int launch_vseg_tile(const SegJob& job, int count, int resident, cudaStream_t st) {
     const int S = job.pl[0].h / LVT, strips = ((job.pl[0].w + 1) / 2 + 31) / 32;
-    const size_t smem = (size_t)S * LVT * (U8 ? 64 : 128) + ((size_t)2 * S * 2 * R * 32 + 128) * 4;
-    if (smem > (size_t)kMaxSmem) return 1;
-    auto kern = vseg_tile_kernel<R, U8>;
-    VSZ_CUDA(allow_max_dynamic_smem(kern));
-    int dev = 0, sms = 148, per_sm = 1;
-    VSZ_CUDA(cudaGetDevice(&dev));
-    VSZ_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-    VSZ_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, S * 32, smem));
-    if (per_sm < 1) return 1;
     for (int f0 = 0; f0 < count; f0 += 32768) {
         const int nf = std::min(32768, count - f0);
         SegJob j = job;
@@ -282,17 +277,12 @@ int launch_vseg_tile(SegJob job, int count, cudaStream_t st) {
         VTiles tiles;
         for (int k = 0; k < j.nplanes; ++k) {
             const SegPlane& pl = j.pl[k];
-            const cuuint64_t dims[3] = {(cuuint64_t)pl.w, (cuuint64_t)pl.h, (cuuint64_t)nf};
-            const cuuint64_t strides[2] = {(cuuint64_t)pl.src_pitch, (cuuint64_t)j.src_fs};
-            const cuuint32_t box[3] = {64, (cuuint32_t)LVT, 1}, estr[3] = {1, 1, 1};
-            const CUresult rc = encode(&tiles.map[k], U8 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : CU_TENSOR_MAP_DATA_TYPE_UINT16, 3, const_cast<char*>(j.src) + pl.src_off, dims, strides, box,
-                                       estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                                       CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-            if (rc != CUDA_SUCCESS) { set_error("BoxBlur: cuTensorMapEncodeTiled failed (%d)", (int)rc); return -1; }
+            const int rc = encode_plane_map(&tiles.map[k], U8 ? CU_TENSOR_MAP_DATA_TYPE_UINT8 : CU_TENSOR_MAP_DATA_TYPE_UINT16, j.src + pl.src_off,
+                                            pl.w, pl.h, pl.src_pitch, j.src_fs, nf, 64, LVT);
+            if (rc) return rc;
         }
         const int nitems = nf * j.nplanes * strips;
-        const int grid = std::min(nitems, sms * per_sm);
-        kern<<<grid, S * 32, smem, st>>>(j, tiles, strips, nitems);
+        vseg_tile_kernel<R, U8><<<std::min(nitems, resident), S * 32, vseg_tile_smem<R, U8>(S), st>>>(j, tiles, strips, nitems);
         count_launch();
     }
     VSZ_CUDA(cudaGetLastError());
@@ -317,37 +307,38 @@ int launch_vseg_shape(SegJob job, int count, cudaStream_t st) {
     return launch_frames(vseg_kernel<R, LV, U8>, job, count, S * 32, smem, st);
 }
 
+// Every shape group's kernel (tile or plain) is settled before the first launch, so that 1 means nothing was launched.
 template <int R, bool U8>
 int launch_vseg(const SegJob& whole, int count, cudaStream_t st) {
     for (int k = 0; k < whole.nplanes; ++k)
         if (!vseg_long(whole.pl[k].w, whole.pl[k].h) && !vseg_fits<60>(whole.pl[k].h)) return 1;
-    return for_each_shape(whole, [&](SegJob job) {
-        if (vseg_long(job.pl[0].w, job.pl[0].h)) return launch_vseg_tile<R, U8>(job, count, st);
-        return launch_vseg_shape<R, 60, U8>(job, count, st);
-    });
+    SegJob groups[3];
+    const int ngroups = shape_groups(whole, groups);
+    int resident[3] = {0, 0, 0};  // tile kernel: resident CTAs; 0 = plain kernel
+    for (int g = 0; g < ngroups; ++g) {
+        const SegPlane& p = groups[g].pl[0];
+        if (!vseg_long(p.w, p.h)) continue;
+        const int rc = vseg_tile_fit<R, U8>(p.h, resident[g]);
+        if (rc) return rc;
+    }
+    for (int g = 0; g < ngroups; ++g) {
+        const int rc = resident[g] ? launch_vseg_tile<R, U8>(groups[g], count, resident[g], st) : launch_vseg_shape<R, 60, U8>(groups[g], count, st);
+        if (rc) return rc;
+    }
+    return 0;
 }
 
 }  // namespace
 
-// Entry points.  Return 0 = done, 1 = not applicable (the caller falls back to the streaming kernels), < 0 = error.
 int run_seg_v(const FrameLayout& l, const bool mask[3], const char* src, size_t sfs, char* dst, size_t dfs, int count, int r, int passes,
               cudaStream_t st) {
     if ((l.kind != K_U16 && l.kind != K_U8) || passes < 1) return 1;
     const SegJob job = base_job(l, mask, src, sfs, dst, dfs, r, passes);
-    if (l.kind == K_U8) {
-        switch (r) {
-#define X(R) case R: return launch_vseg<R, true>(job, count, st);
-            VSZ_SEG_RADII(X)
-#undef X
-        }
-        return 1;
-    }
-    switch (r) {
-#define X(R) case R: return launch_vseg<R, false>(job, count, st);
-        VSZ_SEG_RADII(X)
-#undef X
-    }
-    return 1;
+    const bool u8 = l.kind == K_U8;
+    return with_radius(r, [&](auto radius) {
+        constexpr int R = decltype(radius)::value;
+        return u8 ? launch_vseg<R, true>(job, count, st) : launch_vseg<R, false>(job, count, st);
+    });
 }
 
 }  // namespace vsz

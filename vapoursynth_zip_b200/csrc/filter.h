@@ -77,8 +77,9 @@ namespace vsz {
 int run_boxblur(const FrameLayout& l, const bool mask[3], const char* src, size_t src_fs, char* dst, size_t dst_fs, int count,
                 int hr, int hp, int vr, int vp, cudaStream_t st);
 
+// The BoxBlur fast paths below return 0 = done, 1 = nothing was launched; the caller runs the streaming kernels
+// (boxblur_kernels.cu), < 0 = error.
 // boxblur_seg_{h,v,ct}.cu: 8- and 16-bit integer clips, radius 1..22, planes up to 1920x1080 (comptime path: up to 2048 wide).
-// 0 = done, 1 = not applicable (use the streaming kernels), < 0 = error
 int run_seg_h(const FrameLayout& l, const bool mask[3], const char* src, size_t src_fs, char* dst, size_t dst_fs, int count, int r,
               int passes, cudaStream_t st);
 int run_seg_v(const FrameLayout& l, const bool mask[3], const char* src, size_t src_fs, char* dst, size_t dst_fs, int count, int r,
@@ -86,7 +87,8 @@ int run_seg_v(const FrameLayout& l, const bool mask[3], const char* src, size_t 
 int run_seg_ct(const FrameLayout& l, const bool mask[3], const char* src, size_t src_fs, char* dst, size_t dst_fs, int count, int r,
                cudaStream_t st);
 
-// boxblur_ctf.cu: comptime float path (f16/f32), streaming accumulators; tmp = scratch clip with the layout's frame stride
+// boxblur_ctf.cu: comptime float path (f16/f32), streaming accumulators, planes of at least 2r+1 rows and columns; tmp = scratch clip
+// with the layout's frame stride
 int run_ctf_stream(const FrameLayout& l, const bool mask[3], const char* src, size_t src_fs, char* tmp, size_t tmp_fs, char* dst, size_t dst_fs,
                    int count, int r, cudaStream_t st);
 
